@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path
+    python bench.py ... --dump-outputs DIR      # also write what the last timed step computed (dump_outputs)
 
 Workload (BASELINE.json configs[1], "C2"): cs16 capture of 100 Mi complex samples PER GPU, FFT
 N=4096, Blackman-Harris window, Viridis colormap, dB histogram + colour histogram + min/max/amp
@@ -241,6 +242,34 @@ def oracle_parity_sample(eng, torch, d_img, width, total_samples, w, wt, cm, gro
             "checker": "oracle/ (float64 restatement of lib/worker.js pinned to the reference's own replies)"}
 
 
+DUMP_FRAMES = 512                           # picture columns kept by --dump-outputs: 4096 x 512 x 4 float32 = 32 MiB
+
+
+def dump_outputs(out_dir, torch, d_img, d_g, stats, width, world, ncm):
+    """--dump-outputs: what the last timed C2 step handed its caller, one DIR/<name>.npy per array, so that two builds
+    can be compared output for output.  The RGBA picture (419 MB) is kept at DUMP_FRAMES frames chosen by a fixed seed
+    (all N_FFT rows each, their indices in image_frames.npy); gauges, both histograms and dBfs_min / dBfs_max are whole.
+    At N > 1 rank 0 writes: the picture sample, its frame indices and the gauges are rank 0's own shard (frames counted
+    from its first frame), while the histograms and dBfs_min / dBfs_max are merged over all ranks.  Integers are stored
+    as float32 / float64, exactly."""
+    from spectro_b200 import sharding
+    _, d_hist, d_mm, d_gath = stats
+    if world > 1:
+        hist, mn, mx = sharding.fold_gathered(torch, d_gath, 1000 + ncm)
+    else:
+        hist, (mn, mx) = d_hist, d_mm.tolist()
+    frames = np.sort(np.random.default_rng(SEED).choice(width, min(width, DUMP_FRAMES), replace=False))
+    img = d_img.view(N_FFT, width, 4).index_select(1, torch.from_numpy(frames).to(d_img.device))
+    g = d_g.view(3, width).cpu().numpy().astype(np.float32)
+    hist = hist.cpu().numpy().astype(np.float64)
+    arrays = {"image": img.cpu().numpy().astype(np.float32), "image_frames": frames.astype(np.float64),
+              "gauge_mins": g[0], "gauge_maxs": g[1], "gauge_amps": g[2], "cB_hist": hist[:1000], "c_hist": hist[1000:],
+              "dBfs_min_max": np.array([mn, mx], np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------
 # the other BASELINE.json configs, device resident (N=1): what only builder-run sweeps showed in round 1
 # ----------------------------------------------------------------------------------------------
@@ -470,6 +499,8 @@ def run_ours(args):
     barrier()
     ms_total = e0.elapsed_time(e1)
     kern_ms = eng.profile_read(args.steps)
+    if args.dump_outputs and rank == 0:                     # before the untimed steps below reuse the buffers
+        dump_outputs(args.dump_outputs, torch, d_img, d_g, stats[(state["i"] - 1) & 1], width, world, len(cm))
     # nvidia-smi samples every 100 ms and the timed region is a few ms: keep the SAME step running (untimed)
     # until the sampler has seen >= 0.7 s of this load, so the clock record describes the kernel under load
     t_load = time.perf_counter()
@@ -511,7 +542,7 @@ def run_ours(args):
     eng.d2h(pin_in.array, d_in.data_ptr())
     pin_img = spectro_b200.PinnedBuffer(4 * width * N_FFT)
     pin_img2 = spectro_b200.PinnedBuffer(4 * width * N_FFT)
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     eng.set_stream(None)
     out = None
 
@@ -659,7 +690,14 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` block (N=1) / the `c5_strong` record (N>1)")
     ap.add_argument("--kernel-only", action="store_true",
                     help="development: device-resident leg only (no e2e, no cpu leg, no output check) - A/B runs of experiment builds ($SP_LIB)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of this repo's CUDA path computed as DIR/<name>.npy (float32 / float64, "
+                         "sampled to <= 64 MB; at N > 1 rank 0's shard with the merged histograms)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to this repo's CUDA path only, not to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -1,4 +1,7 @@
 """Shared helpers of the parity tests: the tolerances of BASELINE.json's north_star."""
+import contextlib
+import hashlib
+
 import numpy as np
 
 # north_star: "dB values within 0.01 dB wherever the bin is above -120 dBFS (the fp32 GPU FFT is
@@ -18,6 +21,33 @@ DB_FLOOR_STRICT = -50.0
 DB_FLOOR_REF = -60.0
 DB_TOL_FLOOR_MAX = 0.05
 PIXEL_FRAC = 1e-3        # <= 0.1 % of pixels may differ, by one colour step (quantisation ties)
+
+
+def load_fixture(path):
+    """A tests/golden .npz as a dict (0-d arrays as Python scalars).  A fixture whose capture is a seeded synthetic one
+    may store its recipe (synth_fmt, synth_samples, synth_seed) and the SHA-256 of its bytes instead of the bytes, which
+    keeps the file under 1 MB: `buf` is then regenerated with the oracle's generator and checked against that digest."""
+    g = np.load(path)
+    f = {k: (g[k].item() if g[k].shape == () else g[k]) for k in g.files}
+    if "buf" not in f:
+        from oracle import oracle as O
+        S = int(f["synth_samples"])
+        f["buf"] = O.synth(str(f["synth_fmt"]), 0, S, S, int(f["synth_seed"]))
+        assert hashlib.sha256(f["buf"].tobytes()).hexdigest() == f["buf_sha256"], f"{path}: regenerated capture differs"
+    return f
+
+
+@contextlib.contextmanager
+def restored_cmap_tables():
+    """spectro_b200.Spectroplot overwrites the end points of the shared colormap tables in place, as the reference's
+    lib/spectroplot.js:1129-1130 does: put them back afterwards, so that tests run later see the tables as shipped."""
+    from spectro_b200 import cmaps
+    ends = {k: (t[0], t[-1]) for k, t in cmaps.cmaps.items()}
+    try:
+        yield
+    finally:
+        for k, (first, last) in ends.items():
+            cmaps.cmaps[k][0], cmaps.cmaps[k][-1] = first, last
 
 
 def injective_cmap(n):

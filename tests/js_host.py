@@ -6,11 +6,11 @@ import os
 
 import numpy as np
 
-from oracle.jsmini import Interp, JSObject, JSArray, JSTypedArray, JSArrayBuffer, NativeFunction, UNDEF, JSThrow
+from oracle.jsmini import Interp, JSObject, JSArray, JSTypedArray, JSArrayBuffer, NativeFunction, UNDEF, JSThrow, js_to_string
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 JS = os.path.join(ROOT, "spectroplot-js_b200", "js")
-REFERENCE = "/root/reference/lib"
+REF_HOST = os.path.join(ROOT, "tests", "golden", "ref_js", "ref_host.json")
 FORMATS = ["CU4", "CS4", "CU8", "CS8", "CU12", "CS12", "CU16", "CS16", "CU32", "CS32", "CU64", "CS64", "CF32", "CF64"]
 
 
@@ -70,24 +70,58 @@ class JsHost:
     def __init__(self, render_fn):
         self.I = I = Interp(JS)
         self.log = []
+        self._deps = None
         addon = make_addon(I, render_fn, self.log)
         self.worker_mod = I.require_file(os.path.join(JS, "gpu_worker.js"), lambda spec: addon if spec.endswith("spectro_napi.node") else None)
         self.GpuWorker = I.get_prop(self.worker_mod, "GpuWorker")
         self.formatId = I.get_prop(self.worker_mod, "formatId")
 
-    def reference_deps(self):
-        """The reference's pure modules, loaded from its own files (only where /root/reference exists)."""
+    def mirror_deps(self):
+        """The reference's pure modules that js/spectroplot_headless.js takes injected (windows, cmaps, lookup,
+        parseFreqRate / parseFormat, SampleView), served by the package's Python mirrors of them, which
+        tests/test_reference_js.py pins to the reference's own answers.  Built once per host: the cmap tables are
+        shared objects that the controller overwrites in place, as the reference's are."""
+        if self._deps is not None:
+            return self._deps
+        import json
+        from spectro_b200 import cmaps, parse_freq_rate, utils, windows
+        from spectro_b200.samples import SampleView
         I = self.I
-        deps = JSObject(I.object_proto)
+        native = lambda name, fn: NativeFunction(I, name, fn)
         win = JSObject(I.object_proto)
-        win.props.update(I.load_module("./windows", REFERENCE))
+        for kind in ("rectangular", "bartlett", "hamming", "hann", "blackman", "blackmanHarris"):   # lib/windows.js order
+            fn = getattr(windows, kind + "Window")
+            win.props[kind + "Window"] = native(kind + "Window", lambda t, a, fn=fn: I.from_py(fn(int(a[0]))))
         cm = JSObject(I.object_proto)
-        for m in ("cube1cmap", "matplotlibcmaps", "parabolacmap", "soxcmap", "naivecmap"):   # import order of lib/spectroplot.js
-            cm.props.update(I.load_module("./" + m, REFERENCE))
-        pfr = I.load_module("./parseFreqRate", REFERENCE)
-        deps.props.update(windows=win, cmaps=cm, lookup=I.load_module("./utils", REFERENCE)["lookup"],
-                          parseFreqRate=pfr["parseFreqRate"], parseFormat=pfr["parseFormat"],
-                          SampleView=I.load_module("./samples", REFERENCE)["default"], Worker=self.GpuWorker)
+        with open(REF_HOST) as f:                     # key order of the reference's merged tables (lookup prefix matches)
+            for name in json.load(f)["cmap_key_order"]:
+                cm.props[name] = I.from_py([list(map(int, c)) for c in cmaps.cmaps[name]])
+
+        def lookup(this, a):
+            return utils.lookup(a[0].props, a[1] if len(a) > 1 else UNDEF)
+
+        def sample_view(a):
+            sv = SampleView(js_to_string(a[0]), None, *[None if x is UNDEF else x for x in a[2:4]])
+            obj = JSObject(I.object_proto)
+
+            def sync():
+                obj.props.update(format=sv.format, sampleWidth=sv.sampleWidth, sampleRate=sv.sampleRate, sampleCount=sv.sampleCount)
+
+            def load_buffer(this, b):
+                sv.loadBuffer(bytes(b[0].data))
+                obj.props["buffer"] = b[0]
+                sync()
+                return I.call(I.get_prop(I.globals.vars["Promise"], "resolve"), UNDEF, [obj])
+            obj.props.update(buffer=None, loadBuffer=native("loadBuffer", load_buffer),
+                             slice=native("slice", lambda t, b: JSArrayBuffer(I, bytearray(sv.slice(*[int(x) for x in b[:4]])))))
+            sync()
+            return obj
+        deps = JSObject(I.object_proto)
+        deps.props.update(windows=win, cmaps=cm, lookup=native("lookup", lookup),
+                          parseFreqRate=native("parseFreqRate", lambda t, a: I.from_py(parse_freq_rate.parseFreqRate(js_to_string(a[0])))),
+                          parseFormat=native("parseFormat", lambda t, a: parse_freq_rate.parseFormat(js_to_string(a[0]))),
+                          SampleView=NativeFunction(I, "SampleView", None, sample_view), Worker=self.GpuWorker)
+        self._deps = deps
         return deps
 
     def spectroplot_class(self, deps):

@@ -3,10 +3,16 @@ checked against the oracle's restatement of the reference's caller-side fan-out.
 import numpy as np
 import pytest
 
-from helpers import gray_from_image
+from helpers import gray_from_image, restored_cmap_tables
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
+
+
+@pytest.fixture(autouse=True)
+def _shipped_cmap_tables():
+    with restored_cmap_tables():
+        yield
 
 
 def test_worker_message_protocol(engine):

@@ -8,7 +8,14 @@ import wave
 import numpy as np
 import pytest
 
+from helpers import restored_cmap_tables
 from oracle import oracle as O
+
+
+@pytest.fixture(autouse=True)
+def _shipped_cmap_tables():
+    with restored_cmap_tables():
+        yield
 
 
 def wav_bytes(frames, rate=48000, width=2):

@@ -10,11 +10,11 @@ import os
 import numpy as np
 import pytest
 
-from js_host import JsHost, REFERENCE, typed
+from helpers import load_fixture
+from js_host import JsHost, typed
 from oracle import oracle as O
 from oracle.jsmini import JSObject, JSArray, NativeFunction, UNDEF, JSThrow
 
-HAVE_REF = os.path.isdir(REFERENCE)
 REFJS = os.path.join(os.path.dirname(__file__), "golden", "ref_js")
 
 
@@ -36,8 +36,7 @@ def message(I, f, **over):
 
 
 def load(name):
-    g = np.load(os.path.join(REFJS, name + ".npz"))
-    return {k: (g[k].item() if g[k].shape == () else g[k]) for k in g.files}
+    return load_fixture(os.path.join(REFJS, name + ".npz"))
 
 
 def post(host, worker, msg):
@@ -122,12 +121,11 @@ def test_format_ids_follow_sampleview_aliases():
     assert fid("whatever") == 2 and fid("") == 2               # unknown -> CU8 (lib/samples.js:149-155)
 
 
-# ------------------------------------------------------------------ CPU: js/spectroplot_headless.js over the reference's own modules
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference's pure modules (/root/reference) for injection")
+# ------------------------------------------------------------------ CPU: js/spectroplot_headless.js over the mirrors of the reference's modules
 def test_headless_spectroplot_js_matches_reference_fanout():
     host = JsHost(oracle_render)
     I = host.I
-    Spectroplot = host.spectroplot_class(host.reference_deps())
+    Spectroplot = host.spectroplot_class(host.mirror_deps())
     opts = I.from_py({"fftN": "256", "windowF": "hann", "cmap": "hot", "gain": "6", "range": 30, "clientWidth": 500, "workerCount": 3})
     sp = I.construct(Spectroplot, [opts])
     g = lambda k: I.get_prop(sp, k)
@@ -144,7 +142,7 @@ def test_headless_spectroplot_js_matches_reference_fanout():
     assert g("center_freq") == 433920000.0 and g("sample_rate") == 250000.0 and g("sampleFormat") == "CS16"
     width = 500 - (40 + 60 + 100)
     assert I.get_prop(res, "width") == width == g("width") and I.get_prop(res, "height") == 512
-    hot = I.to_py(host.reference_deps().props["cmaps"].props["hot_cmap"])
+    hot = I.to_py(host.mirror_deps().props["cmaps"].props["hot_cmap"])
     assert hot[0] == [0, 0, 0] and hot[-1] == [255, 255, 255]          # the shared table was overwritten in place (:1129-1130)
     w, wt = O.window("hann", 512)
     ora = O.render(buf, "CS16", 512, width, w, 1 / wt, 6, 30, np.array(hot, np.uint8), workers=3)
@@ -172,14 +170,13 @@ def test_headless_spectroplot_js_matches_reference_fanout():
     assert I.get_prop(r3, "waterfall") is True
     wf_width = int(3200 - 200)                                            # innerHeight stand-in
     w, wt = O.window("blackman", 128)
-    vir = I.to_py(host.reference_deps().props["cmaps"].props["viridis_cmap"])
+    vir = I.to_py(host.mirror_deps().props["cmaps"].props["viridis_cmap"])
     ora = O.render(buf, "CS16", 128, wf_width, w, 1 / wt, 20, 30, np.array(vir, np.uint8), waterfall=True, workers=3)
     assert np.array_equal(I.get_prop(r3, "image").arr, ora.image.reshape(-1))
     call("destroy")
     assert [t[0] for t in host.log[-3:]] == ["destroy"] * 3
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference's pure modules (/root/reference) for injection")
 def test_headless_spectroplot_js_rejects_instead_of_hanging():
     state = {"fail": False}
 
@@ -189,7 +186,7 @@ def test_headless_spectroplot_js_rejects_instead_of_hanging():
         return oracle_render(*a)
     host = JsHost(sometimes)
     I = host.I
-    Spectroplot = host.spectroplot_class(host.reference_deps())
+    Spectroplot = host.spectroplot_class(host.mirror_deps())
     sp = I.construct(Spectroplot, [I.from_py({"fftN": 64, "clientWidth": 300, "workerCount": 2})])
     buf = O.synth("CU8", 0, 4000, 4000, 5).tobytes()
     fd = I.from_py({"name": "x_100M_1000k.cu8"})

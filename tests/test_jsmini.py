@@ -11,7 +11,7 @@ from oracle.jsmini import Interp, UNDEF, JSThrow
 
 
 def run(src):
-    I = Interp("/tmp")
+    I = Interp()
     env = I.run_source(src)
     I.drain()
     return I, env.vars

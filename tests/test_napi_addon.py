@@ -87,8 +87,8 @@ class Addon:
 def load(name):
     from spectro_b200 import _lib
     from spectro_b200.samples import SampleView
-    g = np.load(os.path.join(REFJS, name + ".npz"))
-    f = {k: (g[k].item() if g[k].shape == () else g[k]) for k in g.files}
+    from helpers import load_fixture
+    f = load_fixture(os.path.join(REFJS, name + ".npz"))
     f["format_id"] = _lib.FORMATS.index(SampleView(str(f["fmt"])).canonical)
     return f
 

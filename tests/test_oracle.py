@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O, np_restatement as R
-from helpers import injective_cmap
+from helpers import injective_cmap, load_fixture
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -134,7 +134,7 @@ def test_appendix_b3_end_to_end():
 
 @pytest.mark.parametrize("path", sorted(glob.glob(os.path.join(GOLD, "c*.npz"))))
 def test_oracle_reproduces_golden(path):
-    g = np.load(path)
+    g = load_fixture(path)
     r = O.render(g["buf"].tobytes(), str(g["fmt"]), int(g["n"]), int(g["width"]), g["windowc"], 1.0 / float(g["weight"]),
                  float(g["gain"]), float(g["range"]), g["cmap"], bool(g["channel_mode"]), bool(g["waterfall"]), taps=True)
     assert np.array_equal(r.image, g["image"]) and np.array_equal(r.gray, g["gray"])

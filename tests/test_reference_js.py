@@ -20,17 +20,12 @@ import os
 import numpy as np
 import pytest
 
-from helpers import PIXEL_FRAC, DB_TOL, DB_FLOOR_STRICT, DB_FLOOR_REF, DB_TOL_FLOOR_MAX, cmap_index_image
+from helpers import PIXEL_FRAC, DB_TOL, DB_FLOOR_STRICT, DB_FLOOR_REF, DB_TOL_FLOOR_MAX, cmap_index_image, load_fixture as load
 from oracle import oracle as O
 
 REF = os.path.join(os.path.dirname(__file__), "golden", "ref_js")
 CASES = sorted(glob.glob(os.path.join(REF, "*.npz")))
 IDS = [os.path.basename(p)[:-4] for p in CASES]
-
-
-def load(path):
-    g = np.load(path)
-    return {k: (g[k].item() if g[k].shape == () else g[k]) for k in g.files}
 
 
 def canonical(fmt):

@@ -6,13 +6,14 @@ restatement before being written; SURVEY.md Appendix B's derived known-answers a
 These are restatement-vs-restatement vectors; the pins against the reference's own code are
 tests/golden/ref_js/ (tools/make_ref_golden.py).  Re-run:  python tools/make_golden.py
 """
-import os, sys
+import hashlib, os, sys
 import numpy as np
 ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
 sys.path.insert(0, ROOT)
 from oracle import oracle as O, np_restatement as R
 
 OUT = os.path.join(ROOT, "tests", "golden")
+BUF_INLINE_MAX = 1 << 18                # larger seeded captures are stored as their recipe: every fixture stays under 1 MB
 os.makedirs(OUT, exist_ok=True)
 
 
@@ -31,7 +32,11 @@ def case(name, fmt, n, width, window, gain, rng, cmap, nsamples, seed, channel_m
     assert bad <= max(1, r["gray"].size // 100000), (name, bad)
     fin = np.isfinite(c.db) & np.isfinite(r["db"])
     assert np.abs(r["db"][fin] - c.db[fin]).max() < 1e-9, name
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), buf=np.frombuffer(buf, np.uint8), fmt=fmt, n=n, width=width,
+    if len(buf) > BUF_INLINE_MAX:       # the recipe instead of the bytes (tests/helpers.py load_fixture regenerates them)
+        cap = dict(synth_fmt=fmt, synth_samples=nsamples, synth_seed=seed, buf_sha256=hashlib.sha256(buf).hexdigest())
+    else:
+        cap = dict(buf=np.frombuffer(buf, np.uint8))
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **cap, fmt=fmt, n=n, width=width,
                         window=window, windowc=w, weight=weight, gain=gain, range=rng, cmap=cmap,
                         channel_mode=channel_mode, waterfall=waterfall, image=c.image, gray=c.gray,
                         db=c.db.astype(np.float64), cB_hist=c.cB_hist, c_hist=c.c_hist, gauge_mins=c.gauge_mins,

@@ -9,9 +9,10 @@ oracle/jsmini.py (an ES-subset interpreter written for this purpose, test infras
 
 The only caller-side lines restated here are the ones that build the message from those parts
 (lib/spectroplot.js:1114-1116 block_norm = 1/weight, :1129-1130 cmap end points, :1213-1226 the message fields),
-because lib/spectroplot.js itself needs a DOM.  /root/reference is read at generation time only; the fixtures and
-this script are committed, the tests never touch /root/reference.  Re-run:  python tools/make_ref_golden.py
+because lib/spectroplot.js itself needs a DOM.  The reference's lib/ directory ($SP_REFERENCE) is read at generation time
+only; the fixtures and this script are committed, the tests never need it.  Re-run:  SP_REFERENCE=<reference>/lib python tools/make_ref_golden.py
 """
+import hashlib
 import json
 import math
 import os
@@ -25,7 +26,7 @@ sys.path.insert(0, ROOT)
 from oracle import oracle as O
 from oracle.jsmini import Interp, JSObject, NativeFunction, UNDEF
 
-REF = os.environ.get("SP_REFERENCE", "/root/reference/lib")
+REF = os.environ.get("SP_REFERENCE", "")
 OUT = os.path.join(ROOT, "tests", "golden", "ref_js")
 
 
@@ -84,7 +85,9 @@ def injective_cmap(n):
     return np.stack([i & 255, (i * 7 + 3) & 255, ((i >> 8) * 16 + (i * 37 & 15)) & 255], 1).astype(np.uint8)
 
 
-def run_case(W, name, fmt, n, width, window, cmap, gain, rng, buf, channel_mode=False, waterfall=False):
+def run_case(W, name, fmt, n, width, window, cmap, gain, rng, buf, channel_mode=False, waterfall=False, recipe=None):
+    """recipe = (format, samples, seed) of a capture that is synth()'s output: the fixture stores it and the SHA-256 of the
+    bytes instead of the bytes (tests/helpers.py load_fixture regenerates them), which keeps every file under 1 MB."""
     I = W.I
     t0 = time.time()
     windowc, weight = W.window(window, n)
@@ -98,8 +101,13 @@ def run_case(W, name, fmt, n, width, window, cmap, gain, rng, buf, channel_mode=
     img = I.get_prop(g("imageData"), "data").arr.copy()
     assert img.size == 4 * width * n
     os.makedirs(OUT, exist_ok=True)
+    if recipe is not None:
+        assert bytes(buf) == synth(*recipe), name
+        cap = dict(synth_fmt=recipe[0], synth_samples=recipe[1], synth_seed=recipe[2], buf_sha256=hashlib.sha256(bytes(buf)).hexdigest())
+    else:
+        cap = dict(buf=np.frombuffer(bytes(buf), np.uint8))
     np.savez_compressed(
-        os.path.join(OUT, name + ".npz"), buf=np.frombuffer(bytes(buf), np.uint8), fmt=fmt, n=n, width=width, window=window,
+        os.path.join(OUT, name + ".npz"), **cap, fmt=fmt, n=n, width=width, window=window,
         windowc=np.array(I.to_py(windowc), np.float64), weight=float(weight), gain=gain, range=rng,
         cmap_name=cmap if isinstance(cmap, str) else "custom", cmap=np.array(I.to_py(cm), np.uint8),
         channel_mode=channel_mode, waterfall=waterfall, image=img, cB_hist=cB, cB_extra=json.dumps(cB_x), c_hist=ch,
@@ -120,7 +128,8 @@ def render_cases(W):
     run_case(W, "cs16_n4096_hann_inj_w9", "CS16", 4096, 9, "hann", cm256, 6, 30, synth("CS16", 4096 * 6 + 1234, 0x5EC70103))
     run_case(W, "cf32_n8192_hann_inferno_w4", "CF32", 8192, 4, "hann", "inferno", 6, 30, synth("CF32", 8192 * 4, 0x5EC70104))
     run_case(W, "cf32_n32768_hann_inj_w3", "CF32", 32768, 3, "hann", cm256, 6, 30, synth("CF32", 32768 * 2 + 999, 0x5EC70105))
-    run_case(W, "cf32_n65536_bh_viridis_w2", "CF32", 65536, 2, "blackmanHarris", "viridis", 6, 30, synth("CF32", 65536 * 2, 0x5EC70106))
+    run_case(W, "cf32_n65536_bh_viridis_w2", "CF32", 65536, 2, "blackmanHarris", "viridis", 6, 30, synth("CF32", 65536 * 2, 0x5EC70106),
+             recipe=("CF32", 65536 * 2, 0x5EC70106))
     # ---- every format, every window, every colormap family
     run_case(W, "cu4_n64_rect_naive_w9", "CU4", 64, 9, "rectangular", "naive", 6, 30, synth("CU4", 700, 0x5EC70107))
     run_case(W, "cs4_n128_bartlett_sox_w20", "CS4", 128, 20, "bartlett", "sox", 6, 30, synth("CS4", 128 * 12 + 5, 0x5EC70108))

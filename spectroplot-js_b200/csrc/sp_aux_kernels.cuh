@@ -38,16 +38,23 @@ __global__ void __launch_bounds__(256) jh_table_kernel(JhConst jc, int cmax, int
 // values and scatter jh into acc; the LAST CTA to finish publishes min / max as doubles, copies acc to the reply's histograms and
 // zeroes every counter again, so no launch is needed to reset anything before the next render.
 // `ordered` says fmin/fmax hold f2ord() encodings (sub-frame mode).  mm = {ordered min, ordered max, done counter}.
+// t_end (may be null): the last CTA stores %globaltimer there (the end of the message's device time).
 __global__ void __launch_bounds__(256) finalize_kernel(const float *fmin, const float *fmax, const float2 *fmid,
                                                        long long nframes, double range, double gain, int ordered,
                                                        unsigned char *gmin, unsigned char *gmax, unsigned char *gamp,
                                                        unsigned *mm, double *stats /* [2] min, max */,
                                                        unsigned long long *jh, const int2 *jh_table, int cmap_len,
                                                        unsigned long long *acc_cb, unsigned long long *acc_c,
-                                                       unsigned long long *cb_hist, unsigned long long *c_hist)
+                                                       unsigned long long *cb_hist, unsigned long long *c_hist,
+                                                       unsigned long long *t_end)
 {
     __shared__ float s_mn[8], s_mx[8];
     __shared__ int s_last;
+    // The trigger comes before the wait: the next render may then start on the SMs that the tail of this message's render
+    // leaves idle.  That render only reads the capture and constant tables before its own griddep_wait(), which returns once
+    // this grid - and so, through the wait below, the render before it - has completed.
+    griddep_launch_dependents();
+    griddep_wait();
     // joint histogram of the fused kernels -> the reference's two histograms (lib/worker.js:106,113)
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < JH_SIZE; j += gridDim.x * blockDim.x) {
         const unsigned long long c = jh[j];
@@ -108,6 +115,7 @@ __global__ void __launch_bounds__(256) finalize_kernel(const float *fmin, const 
     for (int i = threadIdx.x; i < CB_BINS; i += blockDim.x) { cb_hist[i] = vcb[i]; vcb[i] = 0; }
     for (int i = threadIdx.x; i < cmap_len; i += blockDim.x) { c_hist[i] = vc[i]; vc[i] = 0; }
     for (int i = threadIdx.x; i < JH_SIZE; i += blockDim.x) jh[i] = 0;
+    if (t_end && threadIdx.x == 0) *t_end = globaltimer_ns();
 }
 
 // decode tap (sp_decode): same device functions as the fused kernel

@@ -27,7 +27,7 @@ using sp::Params;
 #define SP_DECL(tag)                                                                                             \
     extern "C" cudaError_t sp_rl_##tag(int, const Params *, int, size_t, cudaStream_t, int *) __attribute__((weak)); \
     extern "C" cudaError_t sp_pl_##tag(int, const Params *, float2 *, const float2 *, cudaStream_t) __attribute__((weak)); \
-    extern "C" cudaError_t sp_r64_##tag(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int *) __attribute__((weak)); \
+    extern "C" cudaError_t sp_r64_##tag(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int, int *) __attribute__((weak)); \
     extern "C" cudaError_t sp_rc_##tag(int, const Params *, int, cudaStream_t, const float2 *, int *) __attribute__((weak)); \
     extern "C" cudaError_t sp_w_##tag(int, const Params *, int, cudaStream_t, const float2 *, int *) __attribute__((weak)); \
     extern "C" cudaError_t sp_big_##tag(const Params *, const sp::BigArgs *, int, cudaStream_t, const float2 *, int *) __attribute__((weak));
@@ -36,7 +36,7 @@ SP_DECL(cs16) SP_DECL(cu32) SP_DECL(cs32) SP_DECL(cu64) SP_DECL(cs64) SP_DECL(cf
 
 typedef cudaError_t (*render_fn)(int, const Params *, int, size_t, cudaStream_t, int *);
 typedef cudaError_t (*prepass_fn)(int, const Params *, float2 *, const float2 *, cudaStream_t);
-typedef cudaError_t (*r64_fn)(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int *);
+typedef cudaError_t (*r64_fn)(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int, int *);
 typedef cudaError_t (*rc_fn)(int, const Params *, int, cudaStream_t, const float2 *, int *);
 typedef cudaError_t (*big_fn)(const Params *, const sp::BigArgs *, int, cudaStream_t, const float2 *, int *);
 
@@ -204,7 +204,20 @@ struct sp_engine {
     long long pend_width = 0;
     int pend_cmap_len = 0;
     int launches = 0;
+    // render_r64_kernel / finalize_kernel overlap (programmatic dependent launch, see enqueue_end)
+    DevBuf tilectr;                          // two tile counters of render_r64_kernel, used by alternate launches
+    DevBuf tstamp;                           // [2] %globaltimer: start of the message's render_r64_kernel, end of its finalize_kernel
+    unsigned long long r64_count = 0;        // render_r64_kernel launches so far (picks the tile counter)
+    bool after_fin = false;                  // the last thing this engine enqueued is a finalize_kernel (no event behind it)
+    bool stamped = false;                    // the last enqueued render times itself with tstamp instead of ev0 / ev1
 };
+
+// SP_NO_PDL=1: launch render_r64_kernel and finalize_kernel in plain stream order and time messages with events (A/B runs)
+static bool pdl_enabled()
+{
+    static const bool on = getenv("SP_NO_PDL") == nullptr;
+    return on;
+}
 
 static thread_local std::string g_create_err;
 
@@ -331,7 +344,7 @@ extern "C" void sp_destroy(sp_engine *e)
     for (auto &kv : e->twB) cudaFree(kv.second);
     DevBuf *bufs[] = { &e->in, &e->zin, &e->spec, &e->image, &e->fmin, &e->fmax, &e->fmid, &e->gauges, &e->hist, &e->jhist, &e->stats, &e->mm,
                        &e->lut, &e->window, &e->window_t, &e->acc, &e->jhtab, &e->ring, &e->ringctl, &e->scratch, &e->db, &e->synth_lut, &e->pin[0], &e->pin[1],
-                       &e->pimg[0], &e->pimg[1] };
+                       &e->pimg[0], &e->pimg[1], &e->tilectr, &e->tstamp };
     for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
     for (auto ev : e->prof0) cudaEventDestroy(ev);
     for (auto ev : e->prof1) cudaEventDestroy(ev);
@@ -535,6 +548,8 @@ struct Job {
     unsigned long long *d_cb = nullptr, *d_c = nullptr;
     double *d_stats = nullptr;
     bool pipelined = false;    // host buffers streamed chunk by chunk: no whole-message device copies
+    bool pdl = false;          // the render kernel may start early behind the previous message's finalize_kernel
+    bool stamp = false;        // device time from tstamp (the message goes through render_r64_kernel) instead of ev0 / ev1
 };
 
 // bracket a render-kernel launch with the next event pair of the profiling ring.  An event pair between two dependent kernels
@@ -615,6 +630,10 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
     int rc = validate(e, rq, shard, &sample_count, &stride);
     if (rc) return rc;
     CU(cudaSetDevice(e->dev));
+    // a render may overlap the previous message's finalize_kernel only when nothing was enqueued in between: a copy below
+    // (input, window, LUT) or one in enqueue_begin clears j.pdl
+    j.pdl = e->after_fin;
+    e->after_fin = false;
     const int n = rq->n;
     j.log2n = ilog2_exact(n);
     j.plan = make_plan(j.log2n);
@@ -636,6 +655,7 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
         if ((rc = ensure(e, e->in, rq->byte_length + 16))) return rc;
         CU(cudaMemcpyAsync(e->in.p, rq->buffer, rq->byte_length, cudaMemcpyHostToDevice, e->stream));
         p.buf = (const uint8_t *)e->in.p;
+        j.pdl = false;
     }
     p.valid_bytes = rq->byte_length;
     p.sample_base = shard ? (long long)rq->buffer_first_sample : 0;
@@ -662,7 +682,10 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
                                    ((uint32_t)rq->cmap_rgb[3 * i + 2] << 16) | 0xff000000u;
                 if (e->h_lut[i] != v) { same_l = false; break; }
             }
-        if (!same_w || !same_l) CU(cudaStreamSynchronize(e->stream));   // staging vectors may still be in flight
+        if (!same_w || !same_l) {
+            CU(cudaStreamSynchronize(e->stream));                       // staging vectors may still be in flight
+            j.pdl = false;
+        }
         if (!same_w) {
             e->h_window.resize((size_t)n);
             for (int i = 0; i < n; i++) e->h_window[i] = (float)rq->windowc[i] * wscale;
@@ -792,7 +815,9 @@ static bool image_tensor_map(CUtensorMap *tm, uint8_t *image, long long width, i
 
 // Frames [0, *nfast) of the chunk described by q go through render_r64_kernel: every group of 8 frames that lies inside the buffer
 // (the same frames whatever the chunking or sharding, so pipelined / sharded renders stay bit-identical to the single shot).
-static int launch_r64_kernel(sp_engine *e, r64_fn fn, Params &q, long long *nfast)
+// pdl: launch with programmatic stream serialization (the kernel ahead of it cannot write what the kernel reads before its
+// griddep_wait); stamp: CTA 0 records the message's start time in tstamp[0].
+static int launch_r64_kernel(sp_engine *e, r64_fn fn, Params &q, long long *nfast, bool pdl = false, bool stamp = false)
 {
     const bool sub = q.sub_r > 1;
     long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (8 of 16 frames)
@@ -814,15 +839,23 @@ static int launch_r64_kernel(sp_engine *e, r64_fn fn, Params &q, long long *nfas
     if (rc) return rc;
     CUtensorMap tm;
     memset(&tm, 0, sizeof tm);
-    CU(fn(sub ? 1 : 0, &q, 0, e->stream, tw14, &tm, &occ));
+    CU(fn(sub ? 1 : 0, &q, 0, e->stream, tw14, &tm, 0, &occ));
     if (occ < 1) { *nfast = 0; return SP_OK; }             // not built for this format: the caller falls back
+    if (!e->tilectr.p) {                                   // the kernel leaves its counter at zero: set once
+        if ((rc = ensure(e, e->tilectr, 16))) return rc;
+        CU(cudaMemsetAsync(e->tilectr.p, 0, 16, e->stream));
+        pdl = false;
+    }
+    if (stamp && (rc = ensure(e, e->tstamp, 16))) return rc;
     Params r = q;
     r.chunk_frames = nf;
     r.ntiles = ((nf + 15) / 16) * (sub ? q.sub_r : 1);
     r.use_tma = (!sub && !r.waterfall && image_tensor_map(&tm, r.image, r.nframes, r.n_full)) ? 1 : 0;
+    r.tile_ctr = (unsigned long long *)e->tilectr.p + (e->r64_count++ & 1);
+    r.t_stamp = stamp ? (unsigned long long *)e->tstamp.p : nullptr;
     const int grid = (int)(r.ntiles < e->sm_count ? r.ntiles : e->sm_count);
     prof_begin(e);
-    CU(fn(sub ? 1 : 0, &r, grid, e->stream, tw14, &tm, nullptr));
+    CU(fn(sub ? 1 : 0, &r, grid, e->stream, tw14, &tm, pdl ? 1 : 0, nullptr));
     prof_end(e);
     e->launches++;
     return SP_OK;
@@ -993,7 +1026,11 @@ static int launch_rc_kernel(sp_engine *e, rc_fn fn, int log2n, Params &q, long l
 static int enqueue_begin(sp_engine *e, Job &j)
 {
     e->launches = 0;
+    // device time: a message whose frames go through render_r64_kernel is timed by that kernel and finalize_kernel
+    // (%globaltimer), so that no event sits between the finalize_kernel of one message and the render of the next
+    j.stamp = pdl_enabled() && !j.pipelined && j.plan.sub_r == 1 && j.plan.log2k == 12 && fused_eligible(j.p, true, true) && r64_for(j.p.format);
     if (e->acc_dirty) {
+        j.pdl = false;
         // first render, or the previous one was abandoned before finalize_kernel could clean up: zero every accumulator once
         const unsigned mm0[4] = { 0x80000000u /* f2ord(0.0f) */, 0x3cb7ffffu /* f2ord(-200.0f) */, 0u, 0u };
         CU(cudaMemsetAsync(e->acc.p, 0, 8 * (size_t)(SP_CB_HIST_SIZE + SP_MAX_CMAP), e->stream));
@@ -1008,8 +1045,10 @@ static int enqueue_begin(sp_engine *e, Job &j)
         sp::jh_table_kernel<<<(sp::JH_BINS + 255) / 256, 256, 0, e->stream>>>(sp::jh_const(j.p), j.p.cmap_len - 1, (int2 *)e->jhtab.p);
         memcpy(e->jhtab_key, key, sizeof key);
         e->launches++;
+        j.pdl = false;
     }
-    CU(cudaEventRecord(e->ev0, e->stream));
+    if (!j.stamp) CU(cudaEventRecord(e->ev0, e->stream));
+    e->stamped = j.stamp;
     return SP_OK;
 }
 
@@ -1023,10 +1062,14 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         Params q = p;
         if (j.plan.log2k == 12 && fused_eligible(p, /* waterfall rows in the store warps */ true, /* split-real in the FFT warps */ true) && r64_for(fmt)) {
             long long nfast = 0;
-            int rc = launch_r64_kernel(e, r64_for(fmt), q, &nfast);
+            int rc = launch_r64_kernel(e, r64_for(fmt), q, &nfast, j.pdl && pdl_enabled(), j.stamp);
             if (rc) return rc;
             q.chunk_first += nfast;
             q.chunk_frames -= nfast;
+            if (j.stamp && nfast == 0) {                      // no frame went through it: time the message with events
+                j.stamp = e->stamped = false;
+                CU(cudaEventRecord(e->ev0, e->stream));
+            }
         }
         // N = 64 .. 1024, spectrogram layout: the warp-synchronous kernel (SP_W_MAX: largest log2 N it takes, default 10; 0 = off)
         static const int w_max = getenv("SP_W_MAX") ? atoi(getenv("SP_W_MAX")) : 10;
@@ -1140,17 +1183,31 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
     return SP_OK;
 }
 
+// finalize_kernel, launched behind the render kernels with programmatic stream serialization: it starts while the render
+// ends and, as it triggers before its wait, the next message's render_r64_kernel can start as soon as it is resident.  Its
+// grid stays one CTA per 256 frames: capped at 8 or 32 CTAs it hid less of itself than it held back from the next render
+// (C2 on B200: 0.2616 / 0.2483 against 0.2458 ms per step, profiles/r03_overlap_ab.txt).
 static int enqueue_end(sp_engine *e, Job &j)
 {
     Params &p = j.p;
-    sp::finalize_kernel<<<(unsigned)((p.nframes + 255) / 256), 256, 0, e->stream>>>(
-        p.fmin, p.fmax, p.fmid, p.nframes, j.range, j.gain, j.plan.sub_r > 1 ? 1 : 0, j.d_gmin, j.d_gmax, j.d_gamp,
-        (unsigned *)e->mm.p, j.d_stats, (unsigned long long *)e->jhist.p, (const int2 *)e->jhtab.p, p.cmap_len,
-        (unsigned long long *)e->acc.p, (unsigned long long *)e->acc.p + SP_CB_HIST_SIZE, j.d_cb, j.d_c);
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)((p.nframes + 255) / 256));
+    cfg.blockDim = dim3(256);
+    cfg.stream = e->stream;
+    cfg.attrs = &attr;
+    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    CU(cudaLaunchKernelEx(&cfg, sp::finalize_kernel,
+        (const float *)p.fmin, (const float *)p.fmax, (const float2 *)p.fmid, p.nframes, j.range, j.gain, j.plan.sub_r > 1 ? 1 : 0,
+        j.d_gmin, j.d_gmax, j.d_gamp, (unsigned *)e->mm.p, j.d_stats, (unsigned long long *)e->jhist.p, (const int2 *)e->jhtab.p,
+        p.cmap_len, (unsigned long long *)e->acc.p, (unsigned long long *)e->acc.p + SP_CB_HIST_SIZE, j.d_cb, j.d_c,
+        j.stamp ? (unsigned long long *)e->tstamp.p + 1 : (unsigned long long *)nullptr));
     e->launches++;
-    CU(cudaGetLastError());
     e->acc_dirty = false;
-    CU(cudaEventRecord(e->ev1, e->stream));
+    if (j.stamp) e->after_fin = true;
+    else CU(cudaEventRecord(e->ev1, e->stream));
     return SP_OK;
 }
 
@@ -1295,12 +1352,15 @@ static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Jo
 static int finish(sp_engine *e, sp_reply *rp)
 {
     double st[2];
+    unsigned long long ts[2] = { 0, 0 };
     CU(cudaMemcpyAsync(st, e->stats_src ? (void *)e->stats_src : e->stats.p, 16, cudaMemcpyDeviceToHost, e->stream));
+    if (e->stamped) CU(cudaMemcpyAsync(ts, e->tstamp.p, 16, cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     rp->dBfs_min = st[0];
     rp->dBfs_max = st[1];
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
+    if (e->stamped) ms = (float)((double)(long long)(ts[1] - ts[0]) * 1e-6);
+    else CU(cudaEventElapsedTime(&ms, e->ev0, e->ev1));
     rp->device_ms = ms;
     rp->kernel_launches = e->launches;
     return SP_OK;

@@ -77,9 +77,10 @@ static cudaError_t launch_prepass(int r, const Params &p, float2 *out, const flo
     return cudaGetLastError();
 }
 
-// N = 4096 "64 x 64" path: one CTA of 4 x 64 threads per SM, 16 frames per tile (sp_kernel_r64.cuh).
+// N = 4096 "64 x 64" path: one CTA of 4 x 64 threads per SM, 16 frames per tile (sp_kernel_r64.cuh).  pdl: the launch may start
+// before the kernel ahead of it in the stream has completed (programmatic dependent launch; the engine decides when that is safe).
 template <int FMT, bool SUB, bool OPT>
-static cudaError_t launch_r64_k(const Params &p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int *occ_out)
+static cudaError_t launch_r64_k(const Params &p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int pdl, int *occ_out)
 {
     using B = R64Cfg<FMT, SUB>;
     auto kfn = render_r64_kernel<FMT, SUB, OPT>;
@@ -96,22 +97,31 @@ static cudaError_t launch_r64_k(const Params &p, int grid, cudaStream_t st, cons
         *occ_out = nb;
         return e;
     }
-    kfn<<<grid, B::THREADS, B::SMEM_BYTES, st>>>(p, tw14, *tm);
-    return cudaGetLastError();
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3(B::THREADS);
+    cfg.dynamicSmemBytes = B::SMEM_BYTES;
+    cfg.stream = st;
+    cfg.attrs = &attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kfn, p, tw14, *tm);
 }
 template <int FMT, bool SUB>
-static cudaError_t launch_r64_v(const Params &p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int *occ_out)
+static cudaError_t launch_r64_v(const Params &p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int pdl, int *occ_out)
 {
     using B = R64Cfg<FMT, SUB>;
     if constexpr (!B::OK) {
         if (occ_out) *occ_out = 0;
         return occ_out ? cudaSuccess : cudaErrorInvalidValue;
     } else if constexpr (SUB) {
-        return launch_r64_k<FMT, true, false>(p, grid, st, tw14, tm, occ_out);
+        return launch_r64_k<FMT, true, false>(p, grid, st, tw14, tm, pdl, occ_out);
     } else {
         // messages that ask for the waterfall layout or the split-real post-process take the kernel compiled with them
-        if (p.waterfall || p.channel_mode) return launch_r64_k<FMT, false, true>(p, grid, st, tw14, tm, occ_out);
-        return launch_r64_k<FMT, false, false>(p, grid, st, tw14, tm, occ_out);
+        if (p.waterfall || p.channel_mode) return launch_r64_k<FMT, false, true>(p, grid, st, tw14, tm, pdl, occ_out);
+        return launch_r64_k<FMT, false, false>(p, grid, st, tw14, tm, pdl, occ_out);
     }
 }
 
@@ -205,12 +215,13 @@ extern "C" cudaError_t SP_CAT(sp_rl_, SP_INST_TAG)(int log2n, const sp::Params *
 {
     return sp::launch_render<SP_INST_FMT>(log2n, *p, grid, smem, st, occ_out);
 }
-extern "C" cudaError_t SP_CAT(sp_r64_, SP_INST_TAG)(int sub, const sp::Params *p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int *occ_out)
+extern "C" cudaError_t SP_CAT(sp_r64_, SP_INST_TAG)(int sub, const sp::Params *p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm,
+                                                     int pdl, int *occ_out)
 {
     if constexpr (SP_INST_FMT == sp::CF32 || SP_INST_FMT == sp::FMT_RUNTIME) {
-        if (sub) return sp::launch_r64_v<SP_INST_FMT, true>(*p, grid, st, tw14, tm, occ_out);
+        if (sub) return sp::launch_r64_v<SP_INST_FMT, true>(*p, grid, st, tw14, tm, pdl, occ_out);
     } else if (sub) return cudaErrorInvalidValue;
-    return sp::launch_r64_v<SP_INST_FMT, false>(*p, grid, st, tw14, tm, occ_out);
+    return sp::launch_r64_v<SP_INST_FMT, false>(*p, grid, st, tw14, tm, pdl, occ_out);
 }
 extern "C" cudaError_t SP_CAT(sp_rc_, SP_INST_TAG)(int log2n, const sp::Params *p, int grid, cudaStream_t st, const float2 *tw14, int *occ_out)
 {

@@ -46,6 +46,7 @@ template <int FMT, bool SUB> struct R64Cfg {
     static constexpr int WIN_PITCH = 64;                                         // floats per thread row, rotated by 4*t (conflict-free LDS.128)
     static constexpr int TW_PITCH = 14;                                          // float2 per thread row: w^1..w^7, w^8, w^16 .. w^56
     static constexpr int ST_PITCH = 1026;                                        // staging words per frame (1024 used)
+    static constexpr int RING = 4;                                               // tile indices handed from the store warps' ticket thread to the CTA
     // SP_R64_TMA: the 16 KB the window table took hold the store warps' RGBA tiles (one 4 KB tile per warp: four boxes of
     // 32 rows x 8 frames), and the window comes from global memory (p.window_t, 16 KB: it stays in the 28 KB of L1 that the
     // shared-memory carve-out leaves, because nothing else of this kernel goes through L1 any more)
@@ -53,7 +54,8 @@ template <int FMT, bool SUB> struct R64Cfg {
     static constexpr int TILE_BYTES = TMA ? (STORE_THREADS / 32) * 4096 : 0;
     static constexpr size_t SMEM_BYTES = (size_t)STREAMS * X_BYTES + (size_t)F * ST_PITCH * 4 + (size_t)JH_SIZE * 4
                                        + ((SUB || TMA) ? 0 : (size_t)T * WIN_PITCH * 4) + TILE_BYTES + (size_t)T * TW_PITCH * 8 + 1024 /* LUT */
-                                       + (size_t)F * 2 * 8 + 128 + 1024 /* LUT alignment */;
+                                       + (size_t)F * 2 * 8 /* s_mm */ + (size_t)2 * F * 8 /* s_fmid */ + 192 + 1024 /* LUT alignment */;
+    static_assert(SMEM_BYTES <= 232448, "render_r64_kernel: dynamic shared memory above the 227 KB an sm_100 CTA may have");
 };
 
 // RGBA of byte j of a staged word: table base on a 1 KB boundary of the shared window
@@ -102,10 +104,14 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     float *s_win = reinterpret_cast<float *>(s_jh + JH_SIZE);                         // [64][64] (row t: window[64 a + t] at (a + 4t) mod 64)
     float2 *s_tw = reinterpret_cast<float2 *>(s_win + ((SUB || B::TMA) ? 0 : T * B::WIN_PITCH));  // [64][14]
     uint2 *s_mm = reinterpret_cast<uint2 *>(s_tw + T * B::TW_PITCH);                  // [16][2] per-warp min/max bit patterns of |X|^2
-    uint64_t *s_mbar = reinterpret_cast<uint64_t *>(s_mm + F * 2);                    // [4]
+    float2 *s_fmid = reinterpret_cast<float2 *>(s_mm + F * 2);                       // [2 tile parities][16] raw mid sample of each frame
+    uint64_t *s_mbar = reinterpret_cast<uint64_t *>(s_fmid + 2 * F);                  // [4]
     int *s_off = reinterpret_cast<int *>(s_mbar + B::STREAMS);                        // [4][2] misalignment of the staged frame
     uint64_t *s_full = reinterpret_cast<uint64_t *>(s_off + B::STREAMS * 2);          // [2] staging half h holds 8 finished frames
     uint64_t *s_empty = s_full + 2;                                                   // [2] staging half h has been stored
+    uint64_t *s_tready = s_empty + 2;                                                 // [RING] ring slot holds its next tile index
+    long long *s_ring = reinterpret_cast<long long *>(s_tready + B::RING);            // [RING] tile j >= 1 of this CTA in slot (j - 1) % RING
+    long long *s_tile0 = s_ring + B::RING;                                            // this CTA's first tile
 
     const int tid = threadIdx.x;
     const int s = tid >> 6;                 // stream
@@ -146,22 +152,52 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     // tile -> first chunk-relative frame, sub-sequence
     auto tile_xr0 = [&](long long tile) -> long long { return (SUB ? tile / sub_r : tile) * F; };
 
-    // tiles are dealt round-robin: every stream of the CTA walks the same list without a barrier
+    // Tiles are taken from the launch's counter in the order CTAs ask for them, so that a CTA which starts early (programmatic
+    // dependent launch: on an SM the previous render has left) or runs fast takes more of them.  Tickets ntiles .. ntiles + grid - 1
+    // mean "no more tiles", one per CTA; the CTA that draws the last of them resets the counter.  The engine alternates two
+    // counters by launch: the launch after next reuses this one, and it starts only once this launch has completed (see
+    // griddep_launch_dependents below).  One thread of the store warps draws the tickets, one tile ahead, and publishes them
+    // through the ring.  A slot is rewritten RING tiles later; by then the full / empty hand-off has taken every warp at least
+    // two tiles past reading it (RING >= 3).
+    auto ticket = [&]() -> long long {
+        const unsigned long long k = atomicAdd(p.tile_ctr, 1ull);
+        if (k == (unsigned long long)p.ntiles + gridDim.x - 1) atomicExch(p.tile_ctr, 0ull);
+        return (long long)k;
+    };
+    auto ring_put = [&](unsigned j, long long tl) {
+        s_ring[(j - 1) % B::RING] = tl;
+        mbar_arrive(s_tready + (j - 1) % B::RING);
+    };
+    auto ring_get = [&](unsigned j) -> long long {
+        mbar_wait(s_tready + (j - 1) % B::RING, ((j - 1) / B::RING) & 1);
+        return s_ring[(j - 1) % B::RING];
+    };
+
+    if (p.t_stamp && blockIdx.x == 0 && tid == 0) p.t_stamp[0] = globaltimer_ns();   // engine-owned: read only after the stream has drained
     if (t == 0 && tid < B::FFT_THREADS) mbar_init(mbar, 1);
     if (tid == 0) {
         for (int h = 0; h < 2; h++) { mbar_init(s_full + h, B::FFT_THREADS / 32); mbar_init(s_empty + h, B::STORE_THREADS / 32); }
+        for (int r = 0; r < B::RING; r++) mbar_init(s_tready + r, 1);
     }
+    if (tid == B::FFT_THREADS) *s_tile0 = ticket();
     if (t == 0) asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
-    long long tile = blockIdx.x;
-    unsigned kk = 0;                        // tiles done by this CTA (phase of the full / empty barriers)
+    long long tile = *s_tile0;
+    unsigned kk = 0;                        // tiles done by this CTA (phase of the full / empty barriers, ring position)
 
     if (tid >= B::FFT_THREADS) {
         // ================= store warps: staged colour bytes -> LUT -> image rows (lib/worker.js:115-121) =================
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(B::STORE_REGS));
         const int ht = tid - B::FFT_THREADS;
         const bool rows_aligned = (p.nframes % 8 == 0) && ((reinterpret_cast<uintptr_t>(p.image) & 31) == 0);
-        for (; tile < p.ntiles; tile += gridDim.x, kk++) {
+        if (ht == 0 && tile < p.ntiles) ring_put(1, ticket());
+        // Everything before this point reads only the capture and constant tables and writes only shared memory (the FFT warps
+        // never write global memory before the joint-histogram flush): every global write of the CTA comes after the wait.  The
+        // trigger comes after it on every path, tiles or none, so "render i + 2 has started" implies that render i and the
+        // finalize_kernel behind it have completed - which the tile counters and the engine's accumulators rely on.
+        griddep_wait();
+        griddep_launch_dependents();
+        while (tile < p.ntiles) {
             const int k0sub = SUB ? (int)(tile % sub_r) : 0;
             const long long xr0 = tile_xr0(tile);
 #pragma unroll 1
@@ -265,11 +301,13 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     if constexpr (SUB) {
                         atomicMin(reinterpret_cast<unsigned *>(p.fmin) + xl, f2ord(mn));
                         atomicMax(reinterpret_cast<unsigned *>(p.fmax) + xl, f2ord(mx));
-                    } else { p.fmin[xl] = mn; p.fmax[xl] = mx; }
+                    } else { p.fmin[xl] = mn; p.fmax[xl] = mx; p.fmid[xl] = s_fmid[(kk & 1) * F + fl]; }
                 }
                 __syncwarp();                                   // this warp is done reading the half (and s_mm)
                 if ((ht & 31) == 0) mbar_arrive(s_empty + h);
             }
+            tile = ring_get(++kk);
+            if (ht == 0 && tile < p.ntiles) ring_put(kk + 1, ticket());
         }
         if constexpr (B::TMA && !SUB) bulk_wait_read0();        // the tiles must outlive the last tensor stores
     } else {
@@ -281,7 +319,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     while (tile < p.ntiles) {
         const int k0sub = SUB ? (int)(tile % sub_r) : 0;
         const long long xr0 = tile_xr0(tile);
-        const long long next_tile = tile + gridDim.x;
+        long long next_tile = 0;
 
 #pragma unroll 1
         for (int step = 0; step < B::STEPS; step++) {
@@ -294,6 +332,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
             // (opaque to the optimiser: with `step & 1` known, nvcc 12.9 folded 8*(step >> 1) into 4*step and
             // produced a misaligned mbarrier address)
             asm volatile("" : "+r"(half));
+            if (step == B::STEPS - 1) next_tile = ring_get(kk + 1);      // published when the store warps began this tile
             cf v[64];
             const bool split = OPT && !SUB && p.channel_mode;           // split-real needs the buffer once more, see below
             auto prefetch = [&]() {
@@ -319,8 +358,9 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     cf d[4];
 #pragma unroll
                     for (int c = 0; c < 4; c++) d[c] = decode_raw_cf<FMT>(rp, T * (4 * q + c) + t, p.format);
-                    // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact
-                    if (q == 8 && t == 0 && valid) p.fmid[p.chunk_first + xr0 + fl] = make_float2(cre(d[0]) * raw_scale<FMT>(), cim(d[0]) * raw_scale<FMT>());
+                    // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact.  The store warps write it out
+                    // (no global writes here, see griddep_wait); by parity of the tile, as this runs before the wait for the half
+                    if (q == 8 && t == 0 && valid) s_fmid[(kk & 1) * F + fl] = make_float2(cre(d[0]) * raw_scale<FMT>(), cim(d[0]) * raw_scale<FMT>());
                     v[4 * q] = cscale(d[0], w.x);     v[4 * q + 1] = cscale(d[1], w.y);
                     v[4 * q + 2] = cscale(d[2], w.z); v[4 * q + 3] = cscale(d[3], w.w);
                 }
@@ -507,6 +547,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     } // FFT warps
 
     __syncthreads();
+    griddep_wait();                         // (the FFT warps' first global write)
     for (int i = tid; i < JH_SIZE; i += B::THREADS)
         if (s_jh[i]) atomicAdd(&p.j_hist[i], (unsigned long long)s_jh[i]);
 }

@@ -59,7 +59,21 @@ struct Params {
     int use_tma;                   // render_r64_kernel: image rows leave through tensor-TMA stores (width % 4 == 0, 16-byte aligned image)
     int dbg;                       // SP_DEBUG_SKIP bit mask (performance experiments only): 1 image stores, 4 LUT lookups (store warps of render_r64_kernel),
                                    // 16 no span staging in render_w_kernel (every frame copied on its own)
+    unsigned long long *tile_ctr;  // render_r64_kernel: the launch's tile counter, zero at launch and left at zero by the launch
+    unsigned long long *t_stamp;   // render_r64_kernel: %globaltimer at the start of CTA 0 goes to t_stamp[0] (null: not recorded)
 };
+
+// Programmatic dependent launch (render_r64_kernel, finalize_kernel).  wait: the grid this one was launched behind has completed
+// and its memory operations are visible (returns at once without such a grid).  launch_dependents: the next grid of the stream,
+// launched with cudaLaunchAttributeProgrammaticStreamSerialization, may start once every CTA of this grid has executed it or exited.
+__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ unsigned long long globaltimer_ns()
+{
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
 
 template <int LOG2N> struct Cfg {
     static constexpr int N = 1 << LOG2N;

@@ -5,9 +5,7 @@
 // No CPU fallback exists: without an sm_100 device sp_create fails with SP_E_NO_DEVICE.
 #include "../../include/spectro_b200.h"
 #include "sp_aux_kernels.cuh"
-#include "sp_kernel_r64.cuh"
-#include "sp_kernel_big.cuh"
-#include "sp_kernel_w.cuh"
+#include "sp_inst.cuh"
 
 #include <cmath>
 #include <dlfcn.h>
@@ -23,64 +21,28 @@
 
 using sp::Params;
 
-// ---- per-format kernel entry points (weak: a build may carry any subset, "rt" is mandatory) ----
-#define SP_DECL(tag)                                                                                             \
-    extern "C" cudaError_t sp_rl_##tag(int, const Params *, int, size_t, cudaStream_t, int *) __attribute__((weak)); \
-    extern "C" cudaError_t sp_pl_##tag(int, const Params *, float2 *, const float2 *, cudaStream_t) __attribute__((weak)); \
-    extern "C" cudaError_t sp_r64_##tag(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int, int *) __attribute__((weak)); \
-    extern "C" cudaError_t sp_rc_##tag(int, const Params *, int, cudaStream_t, const float2 *, int *) __attribute__((weak)); \
-    extern "C" cudaError_t sp_w_##tag(int, const Params *, int, cudaStream_t, const float2 *, int *) __attribute__((weak)); \
-    extern "C" cudaError_t sp_big_##tag(const Params *, const sp::BigArgs *, int, cudaStream_t, const float2 *, int *) __attribute__((weak));
+// ---- per-format kernels: sp_inst_<tag>.cu exports sp_kernels_<tag> (weak: a build may carry any subset, "rt" is mandatory)
+#define SP_DECL(tag) extern "C" const sp::Kernels sp_kernels_##tag __attribute__((weak));
 SP_DECL(rt) SP_DECL(cu4) SP_DECL(cs4) SP_DECL(cu8) SP_DECL(cs8) SP_DECL(cu12) SP_DECL(cs12) SP_DECL(cu16)
 SP_DECL(cs16) SP_DECL(cu32) SP_DECL(cs32) SP_DECL(cu64) SP_DECL(cs64) SP_DECL(cf32) SP_DECL(cf64)
 
-typedef cudaError_t (*render_fn)(int, const Params *, int, size_t, cudaStream_t, int *);
-typedef cudaError_t (*prepass_fn)(int, const Params *, float2 *, const float2 *, cudaStream_t);
-typedef cudaError_t (*r64_fn)(int, const Params *, int, cudaStream_t, const float2 *, const CUtensorMap *, int, int *);
-typedef cudaError_t (*rc_fn)(int, const Params *, int, cudaStream_t, const float2 *, int *);
-typedef cudaError_t (*big_fn)(const Params *, const sp::BigArgs *, int, cudaStream_t, const float2 *, int *);
-
-static render_fn render_for(int fmt)
+// the format's own build, null when the library carries none
+static const sp::Kernels *own_kernels(int fmt)
 {
-    static const render_fn tab[SP_FORMAT_COUNT] = { sp_rl_cu4, sp_rl_cs4, sp_rl_cu8, sp_rl_cs8, sp_rl_cu12, sp_rl_cs12,
-        sp_rl_cu16, sp_rl_cs16, sp_rl_cu32, sp_rl_cs32, sp_rl_cu64, sp_rl_cs64, sp_rl_cf32, sp_rl_cf64 };
-    return tab[fmt] ? tab[fmt] : sp_rl_rt;
-}
-static prepass_fn prepass_for(int fmt)
-{
-    static const prepass_fn tab[SP_FORMAT_COUNT] = { sp_pl_cu4, sp_pl_cs4, sp_pl_cu8, sp_pl_cs8, sp_pl_cu12, sp_pl_cs12,
-        sp_pl_cu16, sp_pl_cs16, sp_pl_cu32, sp_pl_cs32, sp_pl_cu64, sp_pl_cs64, sp_pl_cf32, sp_pl_cf64 };
-    return tab[fmt] ? tab[fmt] : sp_pl_rt;
-}
-static r64_fn r64_for(int fmt)
-{
-    static const r64_fn tab[SP_FORMAT_COUNT] = { sp_r64_cu4, sp_r64_cs4, sp_r64_cu8, sp_r64_cs8, sp_r64_cu12, sp_r64_cs12,
-        sp_r64_cu16, sp_r64_cs16, sp_r64_cu32, sp_r64_cs32, sp_r64_cu64, sp_r64_cs64, sp_r64_cf32, sp_r64_cf64 };
-    return tab[fmt];                                    // specialised formats only (the runtime-switch build has no raw staging)
-}
-static rc_fn rc_for(int fmt)
-{
-    static const rc_fn tab[SP_FORMAT_COUNT] = { sp_rc_cu4, sp_rc_cs4, sp_rc_cu8, sp_rc_cs8, sp_rc_cu12, sp_rc_cs12,
-        sp_rc_cu16, sp_rc_cs16, sp_rc_cu32, sp_rc_cs32, sp_rc_cu64, sp_rc_cs64, sp_rc_cf32, sp_rc_cf64 };
+    static const sp::Kernels *const tab[SP_FORMAT_COUNT] = { &sp_kernels_cu4, &sp_kernels_cs4, &sp_kernels_cu8, &sp_kernels_cs8,
+        &sp_kernels_cu12, &sp_kernels_cs12, &sp_kernels_cu16, &sp_kernels_cs16, &sp_kernels_cu32, &sp_kernels_cs32,
+        &sp_kernels_cu64, &sp_kernels_cs64, &sp_kernels_cf32, &sp_kernels_cf64 };
     return tab[fmt];
 }
-static rc_fn w_for(int fmt)
+static bool specialised(int fmt) { return own_kernels(fmt) != nullptr; }
+// The launchers of format fmt: its own build, else the runtime-switch build's render, prepass and big.  r64, rc and w stage raw
+// frames of one sample format and exist for specialised formats only.
+static const sp::Kernels &kernels_for(int fmt)
 {
-    static const rc_fn tab[SP_FORMAT_COUNT] = { sp_w_cu4, sp_w_cs4, sp_w_cu8, sp_w_cs8, sp_w_cu12, sp_w_cs12,
-        sp_w_cu16, sp_w_cs16, sp_w_cu32, sp_w_cs32, sp_w_cu64, sp_w_cs64, sp_w_cf32, sp_w_cf64 };
-    return tab[fmt];
-}
-static big_fn big_for(int fmt)
-{
-    static const big_fn tab[SP_FORMAT_COUNT] = { sp_big_cu4, sp_big_cs4, sp_big_cu8, sp_big_cs8, sp_big_cu12, sp_big_cs12,
-        sp_big_cu16, sp_big_cs16, sp_big_cu32, sp_big_cs32, sp_big_cu64, sp_big_cs64, sp_big_cf32, sp_big_cf64 };
-    return tab[fmt] ? tab[fmt] : sp_big_rt;
-}
-static bool specialised(int fmt)
-{
-    static const render_fn tab[SP_FORMAT_COUNT] = { sp_rl_cu4, sp_rl_cs4, sp_rl_cu8, sp_rl_cs8, sp_rl_cu12, sp_rl_cs12,
-        sp_rl_cu16, sp_rl_cs16, sp_rl_cu32, sp_rl_cs32, sp_rl_cu64, sp_rl_cs64, sp_rl_cf32, sp_rl_cf64 };
-    return tab[fmt] != nullptr;
+    static const sp::Kernels rt = &sp_kernels_rt ? sp::Kernels{ sp_kernels_rt.render, sp_kernels_rt.prepass, nullptr, nullptr, nullptr, sp_kernels_rt.big }
+                                                  : sp::Kernels{};
+    const sp::Kernels *own = own_kernels(fmt);
+    return own ? *own : rt;
 }
 
 // ------------------------------------------------------------------ formats (lib/samples.js:22-155)
@@ -504,6 +466,25 @@ static Plan make_plan(int log2n)
     return pl;
 }
 
+// The fused kernel that takes the bulk of the frames described by p.  render_kernel (for n > 4096: prepass_kernel and the
+// sub-frame render_kernel) takes whatever it leaves.  Every fused kernel writes a colour image with 4-byte-aligned rows (any width:
+// rows that are not 32-byte aligned are written word by word) and at most 256 colours, and starts on a group of 8 frames, so the
+// same frames take the same kernel whether a message is rendered in one piece, in pipeline chunks or in shards.
+// For n > 4096 the frame count picks one of the two forms of the four-step transform (enqueue_frames).
+enum class Route { none, r64, w, rc, fourstep };
+static Route route(const Plan &pl, int fmt, const Params &p)
+{
+    const sp::Kernels &k = kernels_for(fmt);
+    if (!p.image || p.db_out || p.cmap_len > 256 || p.chunk_first % 8 != 0 || ((uintptr_t)p.image & 3) != 0) return Route::none;
+    if (pl.sub_r > 1) return !p.waterfall && !p.channel_mode && k.big ? Route::fourstep : Route::none;
+    if (sp::sample_width(fmt) > 8) return Route::none;           // a raw frame must fit the exchange buffer
+    // r64 and w: waterfall rows in the store warps, split-real in the FFT warps
+    if (pl.log2k == 12 && k.r64) return Route::r64;
+    if (pl.log2k >= 6 && pl.log2k <= 10 && k.w) return Route::w;
+    if (pl.log2k == 11 && k.rc && !p.channel_mode) return Route::rc;
+    return Route::none;
+}
+
 extern "C" const char *sp_kernel_plan(sp_engine *e, int format, int n, int channel_mode)
 {
     e = dev0(e);
@@ -513,22 +494,33 @@ extern "C" const char *sp_kernel_plan(sp_engine *e, int format, int n, int chann
     if (l < 1 || l > 18 || format < 0 || format >= SP_FORMAT_COUNT) { e->plan = "unsupported"; return e->plan.c_str(); }
     Plan pl = make_plan(l);
     const char *fname = specialised(format) ? k_names[format] : "runtime-format";
-    const bool fast_ok = !getenv("SP_NO_FAST") && sp::sample_width(format) <= 8 && specialised(format);
+    Params p;                                                   // spectrogram layout, 256 colours, an aligned image, no dB tap
+    memset(&p, 0, sizeof p);
+    p.image = (uint8_t *)(uintptr_t)256;
+    p.cmap_len = 256;
+    p.channel_mode = channel_mode ? 1 : 0;
+    const int P = pl.log2k <= 6 ? 8 : (pl.log2k <= 8 ? 16 : 32);
     size_t o = 0;
-    // the kernel the bulk of a spectrogram-layout message takes, then what catches the rest
-    if (pl.sub_r > 1 && !channel_mode && !getenv("SP_NO_FAST") && big_for(format))
+    // the kernel the bulk of the message takes, then what catches the rest
+    switch (route(pl, format, p)) {
+    case Route::fourstep:
         o += snprintf(buf + o, sizeof buf - o, "four-step n = %d x 4096: render_big_kernel<%s> (one persistent launch, pre-pass and 64x64 second stage as queue items over an "
                       "L2-resident ring; long captures at n = 32768 / 65536, SP_FOURSTEP=ring) or prepass_kernel + render_r64_kernel<sub-frame> over an HBM scratch | ",
                       pl.sub_r, fname);
-    else if (pl.log2k == 12 && pl.sub_r == 1 && fast_ok && r64_for(format))
+        break;
+    case Route::r64:
         o += snprintf(buf + o, sizeof buf - o, "render_r64_kernel<%s> (64x64 FFT, one exchange, 4 frame streams + store warpgroup, TMA-staged input, joint histogram, "
                       "RGBA tiles + tensor-TMA row stores%s) | ", fname, channel_mode ? ", split-real in the FFT warps" : "");
-    else if (pl.log2k >= 6 && pl.log2k <= 10 && fast_ok && w_for(format))
+        break;
+    case Route::w:
         o += snprintf(buf + o, sizeof buf - o, "render_w_kernel<%s, N=%dx%d> (warp-synchronous, one exchange, span-staged input, tables in registers, joint histogram, "
-                      "store warpgroup, spectrogram and waterfall layout%s) | ", fname, pl.log2k <= 6 ? 8 : (pl.log2k <= 8 ? 16 : 32),
-                      (1 << pl.log2k) / (pl.log2k <= 6 ? 8 : (pl.log2k <= 8 ? 16 : 32)), channel_mode ? ", split-real in the FFT warps" : "");
-    else if (pl.log2k == 11 && !channel_mode && fast_ok && rc_for(format))
+                      "store warpgroup, spectrogram and waterfall layout%s) | ", fname, P, (1 << pl.log2k) / P, channel_mode ? ", split-real in the FFT warps" : "");
+        break;
+    case Route::rc:
         o += snprintf(buf + o, sizeof buf - o, "render_rc_kernel<%s, N=64x%d> (one exchange, joint histogram, TMA-staged input, store warpgroup) | ", fname, (1 << pl.log2k) / 64);
+        break;
+    case Route::none: break;
+    }
     snprintf(buf + o, sizeof buf - o, "%s%srender_kernel<N=%d,%s> tile=%d frames%s (every option; remainder frames, ragged ends, dB tap, cmap_len > 256)",
              pl.sub_r > 1 ? "prepass_kernel<R=" : "", pl.sub_r > 1 ? (std::to_string(pl.sub_r) + "> + ").c_str() : "", 1 << pl.log2k, fname, pl.tile,
              channel_mode ? " +splitreal" : "");
@@ -777,14 +769,6 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
     return SP_OK;
 }
 
-// render_r64_kernel / render_rc_kernel: any width (rows that are not 32-byte aligned are written word by word), so the
-// same frames take the same kernel whether a message is rendered in one piece, in pipeline chunks or in shards
-static bool fused_eligible(const Params &p, bool waterfall_ok = false, bool split_ok = false)
-{
-    static const bool off = getenv("SP_NO_FAST") != nullptr;
-    return !off && p.image && (!p.waterfall || waterfall_ok) && (!p.channel_mode || split_ok) && !p.db_out && p.cmap_len <= 256 && (p.chunk_first % 8 == 0) &&
-           (((uintptr_t)p.image) & 3) == 0;
-}
 // Tensor map of the [n rows][width] RGBA picture for the store warps of render_r64_kernel: boxes of 32 rows x 8 pixels,
 // 32-byte swizzle.  The encoder is a driver entry point; it is resolved at run time so that the library keeps linking the
 // CUDA runtime only.
@@ -803,9 +787,8 @@ static encode_tiled_fn tensor_map_encoder()
 }
 static bool image_tensor_map(CUtensorMap *tm, uint8_t *image, long long width, int rows)
 {
-    static const bool off = getenv("SP_NO_TMA_STORE") != nullptr;
     encode_tiled_fn enc = tensor_map_encoder();
-    if (off || !enc || !image || width % 8 != 0 || ((uintptr_t)image & 31) != 0 || width > 0x7fffffffLL) return false;
+    if (!enc || !image || width % 8 != 0 || ((uintptr_t)image & 31) != 0 || width > 0x7fffffffLL) return false;
     const cuuint64_t dims[2] = { (cuuint64_t)width, (cuuint64_t)rows };
     const cuuint64_t strides[1] = { (cuuint64_t)width * 4 };
     const cuuint32_t box[2] = { 8, 32 }, estr[2] = { 1, 1 };
@@ -813,140 +796,152 @@ static bool image_tensor_map(CUtensorMap *tm, uint8_t *image, long long width, i
                CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// Frames [0, *nfast) of the chunk described by q go through render_r64_kernel: every group of 8 frames that lies inside the buffer
-// (the same frames whatever the chunking or sharding, so pipelined / sharded renders stay bit-identical to the single shot).
-// pdl: launch with programmatic stream serialization (the kernel ahead of it cannot write what the kernel reads before its
-// griddep_wait); stamp: CTA 0 records the message's start time in tstamp[0].
-static int launch_r64_kernel(sp_engine *e, r64_fn fn, Params &q, long long *nfast, bool pdl = false, bool stamp = false)
+// The leading whole groups of 8 frames of the chunk q whose `len` samples lie inside the buffer: the same frames whatever the
+// chunking or sharding, so pipelined / sharded renders stay bit-identical to the single shot.  The fused kernels stage raw frames
+// in whole 16-byte units, which the buffer's readable slack covers as long as the frame itself lies inside.
+static long long frames_inside(const Params &q, int len)
 {
-    const bool sub = q.sub_r > 1;
-    long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (8 of 16 frames)
-    if (!sub) {
-        const long long sw = sp::sample_width(q.format);
-        auto inside = [&](long long xr) {
-            const long long xgl = q.frame_first + q.chunk_first + xr;
-            const long long p0 = (long long)(0.5 + q.stride * (double)xgl) - q.sample_base;       // lib/worker.js:72
-            // the bulk copy reads whole 16-byte units: keep the rounded-up end inside the buffer's readable slack
-            return p0 >= 0 && (unsigned long long)(p0 + 4096) * (unsigned long long)sw <= q.valid_bytes;
-        };
-        while (nf > 0 && !inside(nf - 1)) nf -= 8;
-        if (nf > 0 && !inside(0)) nf = 0;
-    }
-    *nfast = nf;
-    if (nf == 0) return SP_OK;
-    const float2 *tw14 = nullptr;
-    int rc = get_r64_table(e, &tw14), occ = 0;
-    if (rc) return rc;
-    CUtensorMap tm;
-    memset(&tm, 0, sizeof tm);
-    CU(fn(sub ? 1 : 0, &q, 0, e->stream, tw14, &tm, 0, &occ));
-    if (occ < 1) { *nfast = 0; return SP_OK; }             // not built for this format: the caller falls back
-    if (!e->tilectr.p) {                                   // the kernel leaves its counter at zero: set once
-        if ((rc = ensure(e, e->tilectr, 16))) return rc;
-        CU(cudaMemsetAsync(e->tilectr.p, 0, 16, e->stream));
-        pdl = false;
-    }
-    if (stamp && (rc = ensure(e, e->tstamp, 16))) return rc;
-    Params r = q;
-    r.chunk_frames = nf;
-    r.ntiles = ((nf + 15) / 16) * (sub ? q.sub_r : 1);
-    r.use_tma = (!sub && !r.waterfall && image_tensor_map(&tm, r.image, r.nframes, r.n_full)) ? 1 : 0;
-    r.tile_ctr = (unsigned long long *)e->tilectr.p + (e->r64_count++ & 1);
-    r.t_stamp = stamp ? (unsigned long long *)e->tstamp.p : nullptr;
-    const int grid = (int)(r.ntiles < e->sm_count ? r.ntiles : e->sm_count);
-    prof_begin(e);
-    CU(fn(sub ? 1 : 0, &r, grid, e->stream, tw14, &tm, pdl ? 1 : 0, nullptr));
-    prof_end(e);
-    e->launches++;
-    return SP_OK;
-}
-
-// n = R * 4096: frames [0, *nfast) (whole blocks of 8 frames inside the buffer) go through ONE launch of render_big_kernel, whose
-// pre-pass output lives in an L2-resident ring of S blocks (S * 8 * n * 8 bytes, pinned by a persisting access-policy window).
-static int launch_big_kernel(sp_engine *e, big_fn fn, Params &q, long long *nfast)
-{
-    const int n = q.n_full, R = q.sub_r;
-    long long nf = q.chunk_frames / 8 * 8;
     const long long sw = sp::sample_width(q.format);
     auto inside = [&](long long xr) {
         const long long xgl = q.frame_first + q.chunk_first + xr;
         const long long p0 = (long long)(0.5 + q.stride * (double)xgl) - q.sample_base;       // lib/worker.js:72
-        return p0 >= 0 && (unsigned long long)(p0 + n) * (unsigned long long)sw <= q.valid_bytes;
+        return p0 >= 0 && (unsigned long long)(p0 + len) * (unsigned long long)sw <= q.valid_bytes;
     };
+    long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (a multiple of 8 frames)
     while (nf > 0 && !inside(nf - 1)) nf -= 8;
     if (nf > 0 && !inside(0)) nf = 0;
-    *nfast = nf;
-    if (nf == 0) return SP_OK;
+    return nf;
+}
+
+// The launch every fused kernel shares, of frames [0, nf) of the chunk q.  launch(r, grid, occ_out) calls the format's launcher
+// (occ_out set: occupancy probe only).  A kernel that does not fit an SM, or is not built for the format, takes no frames
+// (*nfast stays 0) and the caller's remaining kernels take them.  Otherwise setup(r) does the family's own work on the launch's
+// parameters, and the kernel runs ntiles tiles on at most one CTA per SM, in one slot of the profiling ring; `kernels` is what
+// the launch adds to kernel_launches.
+static int no_setup(Params &) { return SP_OK; }
+template <typename Launch, typename Setup>
+static int launch_fused(sp_engine *e, const Params &q, long long nf, long long ntiles, int kernels, long long *nfast, Launch launch, Setup setup)
+{
     int occ = 0, rc;
-    sp::BigArgs g;
-    memset(&g, 0, sizeof g);
-    CU(fn(&q, &g, 0, e->stream, nullptr, &occ));
-    if (occ < 1) { *nfast = 0; return SP_OK; }
-    const int env_slots = getenv("SP_BIG_SLOTS") ? atoi(getenv("SP_BIG_SLOTS")) : 0;       // tuning / tests: ring slots and pre-pass lead
-    const int env_lead = getenv("SP_BIG_LEAD") ? atoi(getenv("SP_BIG_LEAD")) : 0;
-    // Ring: 64 MB, half of the L2 (every CTA holds 512 KB of it for the length of a second-stage tile: with less the pre-pass
-    // waits for free slots, with more the ring no longer fits the 79 MB that can be pinned and spills to HBM - ncu: 1.0 x the
-    // algorithmic DRAM traffic at 64 MB, 1.23 x at 80 MB; profiles/r02_big_kernel.txt), at least 8 blocks; the pre-pass runs
-    // L = 3 S / 8 blocks ahead of the second stage.
-    const size_t block_bytes = (size_t)8 * (size_t)n * 8;
-    int S = env_slots > 0 ? env_slots : (int)(((size_t)64 << 20) / block_bytes);
-    if (S < 8 && env_slots <= 0) S = 8;
-    if (S < 2) S = 2;
-    if (S > 64) S = 64;
-    int L = env_lead > 0 ? env_lead : (3 * S / 8 > 2 ? 3 * S / 8 : 2);
-    if (L > S) L = S;
-    if (L < 1) L = 1;
-    const float2 *tw14 = nullptr, *twT = nullptr;
-    if ((rc = get_r64_table(e, &tw14)) || (rc = get_big_twiddles(e, n, &twT))) return rc;
-    if ((rc = ensure(e, e->ring, (size_t)S * block_bytes)) || (rc = ensure(e, e->ringctl, 4 * (size_t)(1 + 2 * 64) + 64 + 64))) return rc;
-    if (e->l2_window != (size_t)S * block_bytes && !getenv("SP_BIG_NO_L2PIN")) {
-        // keep the ring in L2: persisting lines for the ring's address range, everything else streams through the rest
-        cudaDeviceProp prop;
-        CU(cudaGetDeviceProperties(&prop, e->dev));
-        size_t want = (size_t)S * block_bytes;
-        if (prop.persistingL2CacheMaxSize > 0) {
-            const size_t set_aside = want < (size_t)prop.persistingL2CacheMaxSize ? want : (size_t)prop.persistingL2CacheMaxSize;
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, set_aside);
-            cudaStreamAttrValue av;
-            memset(&av, 0, sizeof av);
-            av.accessPolicyWindow.base_ptr = e->ring.p;
-            av.accessPolicyWindow.num_bytes = want < (size_t)prop.accessPolicyMaxWindowSize ? want : (size_t)prop.accessPolicyMaxWindowSize;
-            av.accessPolicyWindow.hitRatio = 1.0f;
-            av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-            cudaStreamSetAttribute(e->stream, cudaStreamAttributeAccessPolicyWindow, &av);
-            cudaGetLastError();                               // best effort: the kernel is correct without the pin
-        }
-        e->l2_window = want;
-    }
-    CU(cudaMemsetAsync(e->ringctl.p, 0, 4 * (size_t)(1 + 2 * 64), e->stream));
-    g.ring = (float2 *)e->ring.p;
-    g.twT = twT;
-    g.ctl = (unsigned *)e->ringctl.p;
-    g.slots = S;
-    g.lead = L;
-    g.nblocks = nf / 8;
-    g.R = R;
-    g.dbg = getenv("SP_BIG_DBG") ? atoi(getenv("SP_BIG_DBG")) : 0;
-    // SP_BIG_STATS=1: per-phase SM cycle sums of the launch (development), printed when the engine is destroyed / next launch
-    static const bool want_stats = getenv("SP_BIG_STATS") != nullptr;
-    if (want_stats) {
-        g.stats = (unsigned long long *)((unsigned char *)e->ringctl.p + ((4 * (size_t)(1 + 2 * 64) + 63) & ~(size_t)63));
-        unsigned long long h[8];
-        CU(cudaMemcpyAsync(h, g.stats, sizeof h, cudaMemcpyDeviceToHost, e->stream));   // the PREVIOUS launch's sums (stream order)
-        CU(cudaStreamSynchronize(e->stream));
-        if (h[4] || h[5])
-            fprintf(stderr, "[big] P: %llu items, wait %.0f work %.0f (first frame landed after %.0f, 8-frame loop %.0f) cycles/item | F: %llu tiles, wait %.0f work %.0f cycles/tile\n", h[4],
-                    h[4] ? (double)h[0] / h[4] : 0.0, h[4] ? (double)h[1] / h[4] : 0.0, h[4] ? (double)h[6] / h[4] : 0.0, h[4] ? (double)h[7] / h[4] : 0.0, h[5], h[5] ? (double)h[2] / h[5] : 0.0, h[5] ? (double)h[3] / h[5] : 0.0);
-        CU(cudaMemsetAsync(g.stats, 0, 64, e->stream));
-    }
+    CU(launch(q, 0, &occ));
+    if (occ < 1) return SP_OK;
     Params r = q;
     r.chunk_frames = nf;
+    r.ntiles = ntiles;
+    if ((rc = setup(r))) return rc;
     prof_begin(e);
-    CU(fn(&r, &g, e->sm_count, e->stream, tw14, nullptr));
+    CU(launch(r, (int)(ntiles < e->sm_count ? ntiles : e->sm_count), nullptr));
     prof_end(e);
-    e->launches += 2;
+    e->launches += kernels;
+    *nfast = nf;
     return SP_OK;
+}
+
+// render_r64_kernel: N = 4096, or in sub-frame mode the second stage of the HBM-scratch form of n > 4096, which reads the
+// pre-pass scratch instead of the buffer and takes every whole group of 8 frames.  pdl: launch with programmatic stream
+// serialization (the kernel ahead of it cannot write what the kernel reads before its griddep_wait); stamp: CTA 0 records the
+// message's start time in tstamp[0].
+static int launch_r64_kernel(sp_engine *e, const sp::Kernels &k, const Params &q, long long *nfast, bool pdl = false, bool stamp = false)
+{
+    const bool sub = q.sub_r > 1;
+    const long long nf = sub ? q.chunk_frames / 8 * 8 : frames_inside(q, 4096);   // the last tile may be partial (8 of 16 frames)
+    if (nf == 0) return SP_OK;
+    const float2 *tw14 = nullptr;
+    int rc = get_r64_table(e, &tw14);
+    if (rc) return rc;
+    CUtensorMap tm;
+    memset(&tm, 0, sizeof tm);
+    auto launch = [&](const Params &r, int grid, int *occ) { return k.r64(sub ? 1 : 0, &r, grid, e->stream, tw14, &tm, pdl ? 1 : 0, occ); };
+    auto setup = [&](Params &r) -> int {
+        if (!e->tilectr.p) {                               // the kernel leaves its counter at zero: set once
+            if ((rc = ensure(e, e->tilectr, 16))) return rc;
+            CU(cudaMemsetAsync(e->tilectr.p, 0, 16, e->stream));
+            pdl = false;
+        }
+        if (stamp && (rc = ensure(e, e->tstamp, 16))) return rc;
+        r.use_tma = (!sub && !r.waterfall && image_tensor_map(&tm, r.image, r.nframes, r.n_full)) ? 1 : 0;
+        r.tile_ctr = (unsigned long long *)e->tilectr.p + (e->r64_count++ & 1);
+        r.t_stamp = stamp ? (unsigned long long *)e->tstamp.p : nullptr;
+        return SP_OK;
+    };
+    return launch_fused(e, q, nf, ((nf + 15) / 16) * (sub ? q.sub_r : 1), 1, nfast, launch, setup);
+}
+
+// n = R * 4096: ONE launch of render_big_kernel (a pre-pass and a second stage, counted as two kernels), whose pre-pass output
+// lives in an L2-resident ring of S blocks (S * 8 * n * 8 bytes, pinned by a persisting access-policy window).  The kernel is
+// persistent and takes its work from a queue: one CTA per SM.
+static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q, long long *nfast)
+{
+    const int n = q.n_full, R = q.sub_r;
+    const long long nf = frames_inside(q, n);
+    if (nf == 0) return SP_OK;
+    sp::BigArgs g;
+    memset(&g, 0, sizeof g);
+    const float2 *tw14 = nullptr;
+    auto launch = [&](const Params &r, int grid, int *occ) { return k.big(&r, &g, grid, e->stream, tw14, occ); };
+    auto setup = [&](Params &) -> int {
+        int rc;
+        const int env_slots = getenv("SP_BIG_SLOTS") ? atoi(getenv("SP_BIG_SLOTS")) : 0;       // tuning / tests: ring slots and pre-pass lead
+        const int env_lead = getenv("SP_BIG_LEAD") ? atoi(getenv("SP_BIG_LEAD")) : 0;
+        // Ring: 64 MB, half of the L2 (every CTA holds 512 KB of it for the length of a second-stage tile: with less the pre-pass
+        // waits for free slots, with more the ring no longer fits the 79 MB that can be pinned and spills to HBM - ncu: 1.0 x the
+        // algorithmic DRAM traffic at 64 MB, 1.23 x at 80 MB; profiles/r02_big_kernel.txt), at least 8 blocks; the pre-pass runs
+        // L = 3 S / 8 blocks ahead of the second stage.
+        const size_t block_bytes = (size_t)8 * (size_t)n * 8;
+        int S = env_slots > 0 ? env_slots : (int)(((size_t)64 << 20) / block_bytes);
+        if (S < 8 && env_slots <= 0) S = 8;
+        if (S < 2) S = 2;
+        if (S > 64) S = 64;
+        int L = env_lead > 0 ? env_lead : (3 * S / 8 > 2 ? 3 * S / 8 : 2);
+        if (L > S) L = S;
+        if (L < 1) L = 1;
+        const float2 *twT = nullptr;
+        if ((rc = get_r64_table(e, &tw14)) || (rc = get_big_twiddles(e, n, &twT))) return rc;
+        if ((rc = ensure(e, e->ring, (size_t)S * block_bytes)) || (rc = ensure(e, e->ringctl, 4 * (size_t)(1 + 2 * 64) + 64 + 64))) return rc;
+        if (e->l2_window != (size_t)S * block_bytes && !getenv("SP_BIG_NO_L2PIN")) {
+            // keep the ring in L2: persisting lines for the ring's address range, everything else streams through the rest
+            cudaDeviceProp prop;
+            CU(cudaGetDeviceProperties(&prop, e->dev));
+            size_t want = (size_t)S * block_bytes;
+            if (prop.persistingL2CacheMaxSize > 0) {
+                const size_t set_aside = want < (size_t)prop.persistingL2CacheMaxSize ? want : (size_t)prop.persistingL2CacheMaxSize;
+                cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, set_aside);
+                cudaStreamAttrValue av;
+                memset(&av, 0, sizeof av);
+                av.accessPolicyWindow.base_ptr = e->ring.p;
+                av.accessPolicyWindow.num_bytes = want < (size_t)prop.accessPolicyMaxWindowSize ? want : (size_t)prop.accessPolicyMaxWindowSize;
+                av.accessPolicyWindow.hitRatio = 1.0f;
+                av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
+                av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
+                cudaStreamSetAttribute(e->stream, cudaStreamAttributeAccessPolicyWindow, &av);
+                cudaGetLastError();                               // best effort: the kernel is correct without the pin
+            }
+            e->l2_window = want;
+        }
+        CU(cudaMemsetAsync(e->ringctl.p, 0, 4 * (size_t)(1 + 2 * 64), e->stream));
+        g.ring = (float2 *)e->ring.p;
+        g.twT = twT;
+        g.ctl = (unsigned *)e->ringctl.p;
+        g.slots = S;
+        g.lead = L;
+        g.nblocks = nf / 8;
+        g.R = R;
+        g.dbg = getenv("SP_BIG_DBG") ? atoi(getenv("SP_BIG_DBG")) : 0;
+        // SP_BIG_STATS=1: per-phase SM cycle sums of the launch (development), printed when the engine is destroyed / next launch
+        static const bool want_stats = getenv("SP_BIG_STATS") != nullptr;
+        if (want_stats) {
+            g.stats = (unsigned long long *)((unsigned char *)e->ringctl.p + ((4 * (size_t)(1 + 2 * 64) + 63) & ~(size_t)63));
+            unsigned long long h[8];
+            CU(cudaMemcpyAsync(h, g.stats, sizeof h, cudaMemcpyDeviceToHost, e->stream));   // the PREVIOUS launch's sums (stream order)
+            CU(cudaStreamSynchronize(e->stream));
+            if (h[4] || h[5])
+                fprintf(stderr, "[big] P: %llu items, wait %.0f work %.0f (first frame landed after %.0f, 8-frame loop %.0f) cycles/item | F: %llu tiles, wait %.0f work %.0f cycles/tile\n", h[4],
+                        h[4] ? (double)h[0] / h[4] : 0.0, h[4] ? (double)h[1] / h[4] : 0.0, h[4] ? (double)h[6] / h[4] : 0.0, h[4] ? (double)h[7] / h[4] : 0.0, h[5], h[5] ? (double)h[2] / h[5] : 0.0, h[5] ? (double)h[3] / h[5] : 0.0);
+            CU(cudaMemsetAsync(g.stats, 0, 64, e->stream));
+        }
+        return SP_OK;
+    };
+    return launch_fused(e, q, nf, e->sm_count, 2, nfast, launch, setup);
 }
 
 // render_w_kernel table: [P][T] = W_N^{t*k}, k = 0 .. P-1 (N = P * T)
@@ -959,67 +954,31 @@ static int get_w_table(sp_engine *e, int n, int P, const float2 **out)
     for (int k = 0; k < P; k++) for (int t = 0; t < T; t++) h[(size_t)k * T + t] = twid((long long)t * k, n);
     return upload_table(e, e->twA, -200000 - n, h, out);
 }
-// Frames [0, *nfast) of the chunk go through render_w_kernel (N = 64 .. 1024): whole groups of 8 frames inside the buffer.
-static int launch_w_kernel(sp_engine *e, rc_fn fn, int log2n, Params &q, long long *nfast)
+// render_w_kernel: N = 64 .. 1024
+static int launch_w_kernel(sp_engine *e, const sp::Kernels &k, int log2n, const Params &q, long long *nfast)
 {
     const int n = 1 << log2n, P = log2n <= 6 ? 8 : (log2n <= 8 ? 16 : 32), T = n / P, FW = 32 / T, NW = P <= 16 ? SP_W_NW16 : SP_W_NW32, WSH = n == 64 ? 4 : 2;
     const int tile = 2 * NW * WSH * FW;
-    long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (a multiple of 8 frames)
-    const long long sw = sp::sample_width(q.format);
-    auto inside = [&](long long xr) {
-        const long long xgl = q.frame_first + q.chunk_first + xr;
-        const long long p0 = (long long)(0.5 + q.stride * (double)xgl) - q.sample_base;       // lib/worker.js:72
-        return p0 >= 0 && (unsigned long long)(p0 + n) * (unsigned long long)sw <= q.valid_bytes;
-    };
-    while (nf > 0 && !inside(nf - 1)) nf -= 8;
-    if (nf > 0 && !inside(0)) nf = 0;
-    *nfast = nf;
+    const long long nf = frames_inside(q, n);
     if (nf == 0) return SP_OK;
     const float2 *twW = nullptr;
-    int rc = get_w_table(e, n, P, &twW), occ = 0;
+    const int rc = get_w_table(e, n, P, &twW);
     if (rc) return rc;
-    CU(fn(log2n, &q, 0, e->stream, twW, &occ));
-    if (occ < 1) { *nfast = 0; return SP_OK; }
-    Params r = q;
-    r.chunk_frames = nf;
-    r.ntiles = (nf + tile - 1) / tile;
-    const int grid = (int)(r.ntiles < e->sm_count ? r.ntiles : e->sm_count);
-    prof_begin(e);
-    CU(fn(log2n, &r, grid, e->stream, twW, nullptr));
-    prof_end(e);
-    e->launches++;
-    return SP_OK;
+    return launch_fused(e, q, nf, (nf + tile - 1) / tile, 1, nfast,
+                        [&](const Params &r, int grid, int *occ) { return k.w(log2n, &r, grid, e->stream, twW, occ); }, no_setup);
 }
 
-// Frames [0, *nfast) of the chunk go through render_rc_kernel (N = 256 .. 2048): whole tiles of 65536 / N frames inside the buffer.
-static int launch_rc_kernel(sp_engine *e, rc_fn fn, int log2n, Params &q, long long *nfast)
+// render_rc_kernel: N = 2048, tiles of 65536 / N frames
+static int launch_rc_kernel(sp_engine *e, const sp::Kernels &k, int log2n, const Params &q, long long *nfast)
 {
     const int n = 1 << log2n, tile = 65536 / n;
-    long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (a multiple of 8 frames)
-    const long long sw = sp::sample_width(q.format);
-    auto inside = [&](long long xr) {
-        const long long xgl = q.frame_first + q.chunk_first + xr;
-        const long long p0 = (long long)(0.5 + q.stride * (double)xgl) - q.sample_base;       // lib/worker.js:72
-        return p0 >= 0 && (unsigned long long)(p0 + n) * (unsigned long long)sw <= q.valid_bytes;
-    };
-    while (nf > 0 && !inside(nf - 1)) nf -= 8;
-    if (nf > 0 && !inside(0)) nf = 0;
-    *nfast = nf;
+    const long long nf = frames_inside(q, n);
     if (nf == 0) return SP_OK;
     const float2 *tw14 = nullptr;
-    int rc = get_rc_table(e, n, &tw14), occ = 0;
+    const int rc = get_rc_table(e, n, &tw14);
     if (rc) return rc;
-    CU(fn(log2n, &q, 0, e->stream, tw14, &occ));
-    if (occ < 1) { *nfast = 0; return SP_OK; }
-    Params r = q;
-    r.chunk_frames = nf;
-    r.ntiles = (nf + tile - 1) / tile;
-    const int grid = (int)(r.ntiles < e->sm_count ? r.ntiles : e->sm_count);
-    prof_begin(e);
-    CU(fn(log2n, &r, grid, e->stream, tw14, nullptr));
-    prof_end(e);
-    e->launches++;
-    return SP_OK;
+    return launch_fused(e, q, nf, (nf + tile - 1) / tile, 1, nfast,
+                        [&](const Params &r, int grid, int *occ) { return k.rc(log2n, &r, grid, e->stream, tw14, occ); }, no_setup);
 }
 
 // Enqueue all kernels of a job on e->stream (bracketed by the timing events).
@@ -1028,7 +987,7 @@ static int enqueue_begin(sp_engine *e, Job &j)
     e->launches = 0;
     // device time: a message whose frames go through render_r64_kernel is timed by that kernel and finalize_kernel
     // (%globaltimer), so that no event sits between the finalize_kernel of one message and the render of the next
-    j.stamp = pdl_enabled() && !j.pipelined && j.plan.sub_r == 1 && j.plan.log2k == 12 && fused_eligible(j.p, true, true) && r64_for(j.p.format);
+    j.stamp = pdl_enabled() && !j.pipelined && route(j.plan, j.p.format, j.p) == Route::r64;
     if (e->acc_dirty) {
         j.pdl = false;
         // first render, or the previous one was abandoned before finalize_kernel could clean up: zero every accumulator once
@@ -1056,47 +1015,33 @@ static int enqueue_begin(sp_engine *e, Job &j)
 static int enqueue_frames(sp_engine *e, Job &j, Params &p)
 {
     const int fmt = p.format;
+    const sp::Kernels &k = kernels_for(fmt);
+    const Route fused = route(j.plan, fmt, p);
     const size_t smem = sp::main_smem_bytes(j.plan.smem_x, p.cmap_len, j.plan.log2k > 8 ? 15 * ((1 << j.plan.log2k) / 256) : 0);
     int occ = 0;
     if (j.plan.sub_r == 1) {
         Params q = p;
-        if (j.plan.log2k == 12 && fused_eligible(p, /* waterfall rows in the store warps */ true, /* split-real in the FFT warps */ true) && r64_for(fmt)) {
-            long long nfast = 0;
-            int rc = launch_r64_kernel(e, r64_for(fmt), q, &nfast, j.pdl && pdl_enabled(), j.stamp);
-            if (rc) return rc;
-            q.chunk_first += nfast;
-            q.chunk_frames -= nfast;
-            if (j.stamp && nfast == 0) {                      // no frame went through it: time the message with events
-                j.stamp = e->stamped = false;
-                CU(cudaEventRecord(e->ev0, e->stream));
-            }
-        }
-        // N = 64 .. 1024, spectrogram layout: the warp-synchronous kernel (SP_W_MAX: largest log2 N it takes, default 10; 0 = off)
-        static const int w_max = getenv("SP_W_MAX") ? atoi(getenv("SP_W_MAX")) : 10;
-        if (j.plan.log2k >= 6 && j.plan.log2k <= w_max && j.plan.log2k <= 10 && fused_eligible(p, /* waterfall rows in the store warps */ true, /* split-real in the FFT warps */ true) && w_for(fmt)) {
-            long long nfast = 0;
-            int rc = launch_w_kernel(e, w_for(fmt), j.plan.log2k, q, &nfast);
-            if (rc) return rc;
-            q.chunk_first += nfast;
-            q.chunk_frames -= nfast;
-        }
-        if (j.plan.log2k == 11 && fused_eligible(q, true) && rc_for(fmt) && q.chunk_frames >= 8) {
-            long long nfast = 0;
-            int rc = launch_rc_kernel(e, rc_for(fmt), j.plan.log2k, q, &nfast);
-            if (rc) return rc;
-            q.chunk_first += nfast;
-            q.chunk_frames -= nfast;
+        long long nfast = 0;
+        int rc = SP_OK;
+        if (fused == Route::r64) rc = launch_r64_kernel(e, k, q, &nfast, j.pdl && pdl_enabled(), j.stamp);
+        else if (fused == Route::w) rc = launch_w_kernel(e, k, j.plan.log2k, q, &nfast);
+        else if (fused == Route::rc) rc = launch_rc_kernel(e, k, j.plan.log2k, q, &nfast);
+        if (rc) return rc;
+        q.chunk_first += nfast;
+        q.chunk_frames -= nfast;
+        if (j.stamp && nfast == 0) {                          // no frame went through render_r64_kernel: time the message with events
+            j.stamp = e->stamped = false;
+            CU(cudaEventRecord(e->ev0, e->stream));
         }
         if (q.chunk_frames > 0) {
-            render_fn fn = render_for(fmt);
-            if (!fn) return fail(e, SP_E_CUDA, "no render kernel linked for format %d", fmt);
-            CU(fn(j.plan.log2k, &q, 0, smem, e->stream, &occ));
+            if (!k.render) return fail(e, SP_E_CUDA, "no render kernel linked for format %d", fmt);
+            CU(k.render(j.plan.log2k, &q, 0, smem, e->stream, &occ));
             if (occ < 1) return fail(e, SP_E_CUDA, "render kernel does not fit an SM (smem %zu)", smem);
             q.ntiles = (q.chunk_frames + j.plan.tile - 1) / j.plan.tile;
             const long long cap = (long long)e->sm_count * occ;
             const int grid = (int)(q.ntiles < cap ? q.ntiles : cap);
             prof_begin(e);
-            CU(fn(j.plan.log2k, &q, grid, smem, e->stream, nullptr));
+            CU(k.render(j.plan.log2k, &q, grid, smem, e->stream, nullptr));
             prof_end(e);
             e->launches++;
         }
@@ -1105,9 +1050,8 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         // 4096-point kernel in sub-frame mode, chunk by chunk
         const int R = j.plan.sub_r;
         const int n = p.n_full;
-        render_fn fn = sp_rl_cf32 ? sp_rl_cf32 : sp_rl_rt;   // sub-frame input is always complex fp32
-        prepass_fn pf = prepass_for(fmt);
-        if (!fn || !pf) return fail(e, SP_E_CUDA, "no kernels linked for the four-step path");
+        const sp::Kernels &sub = kernels_for(SP_CF32);        // sub-frame input is always complex fp32
+        if (!sub.render || !k.prepass) return fail(e, SP_E_CUDA, "no kernels linked for the four-step path");
         const float2 *tw_full = nullptr;
         int rc = get_twiddles(e, n, &tw_full);
         if (rc) return rc;
@@ -1127,7 +1071,7 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         // chunk and finish it in spectrum_epilogue_kernel
         const bool tap = p.channel_mode != 0;
         if (tap && (rc = ensure(e, e->spec, (size_t)ch * (size_t)n * 8))) return rc;
-        CU(fn(12, &p, 0, smem, e->stream, &occ));
+        CU(sub.render(12, &p, 0, smem, e->stream, &occ));
         if (occ < 1) return fail(e, SP_E_CUDA, "render kernel does not fit an SM (smem %zu)", smem);
         const long long nf = p.nframes;
         sp::init_minmax_kernel<<<(unsigned)((nf + 255) / 256), 256, 0, e->stream>>>((unsigned *)p.fmin, (unsigned *)p.fmax, nf);
@@ -1140,24 +1084,23 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         // The ring form is as fast or faster where the scratch round trip hurts most - n = 32768 / 65536 on long captures (C3, C5) -
         // and slower elsewhere, so it is chosen there; SP_FOURSTEP=ring / hbm forces one form (tests, A/B runs).
         const char *force = getenv("SP_FOURSTEP");
-        const bool force_hbm = getenv("SP_NO_BIG") || (force && !strcmp(force, "hbm")), force_ring = force && !strcmp(force, "ring");
+        const bool force_hbm = force && !strcmp(force, "hbm"), force_ring = force && !strcmp(force, "ring");
         const bool ring = force_ring || (!force_hbm && (R == 8 || R == 16) && (double)nf * (double)n >= 536870912.0);
-        if (!tap && fused_eligible(p) && big_for(fmt) && ring) {
-            Params q = p;
-            if ((rc = launch_big_kernel(e, big_for(fmt), q, &big_done))) return rc;
+        if (fused == Route::fourstep && ring) {
+            if ((rc = launch_big_kernel(e, k, p, &big_done))) return rc;
         } else release_l2_window(e);                          // the HBM-scratch form wants the whole cache
         for (long long c0 = big_done; c0 < nf; c0 += ch) {
             Params q = p;
             q.chunk_first = c0;
             q.chunk_frames = (nf - c0 < ch) ? nf - c0 : ch;
-            CU(pf(R, &q, (float2 *)e->scratch.p, tw_full, e->stream));
+            CU(k.prepass(R, &q, (float2 *)e->scratch.p, tw_full, e->stream));
             q.sub_in = (const float2 *)e->scratch.p;
             e->launches++;
             Params full = q;                                   // what the epilogue kernel sees
             if (tap) { q.spec_out = (float2 *)e->spec.p; q.image = nullptr; q.db_out = nullptr; q.channel_mode = 0; }
-            if (fused_eligible(q) && sp_r64_cf32) {
+            if (fused == Route::fourstep && sub.r64) {
                 long long nfast = 0;
-                if ((rc = launch_r64_kernel(e, sp_r64_cf32, q, &nfast))) return rc;
+                if ((rc = launch_r64_kernel(e, sub, q, &nfast))) return rc;
                 q.sub_in += (size_t)nfast * (size_t)R * 4096;
                 q.chunk_first += nfast;
                 q.chunk_frames -= nfast;
@@ -1167,7 +1110,7 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
                 const long long cap = (long long)e->sm_count * occ;
                 const int grid = (int)(q.ntiles < cap ? q.ntiles : cap);
                 prof_begin(e);
-                CU(fn(12, &q, grid, smem, e->stream, nullptr));
+                CU(sub.render(12, &q, grid, smem, e->stream, nullptr));
                 prof_end(e);
                 e->launches++;
             }

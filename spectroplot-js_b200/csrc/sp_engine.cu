@@ -957,8 +957,7 @@ static int get_w_table(sp_engine *e, int n, int P, const float2 **out)
 // render_w_kernel: N = 64 .. 1024
 static int launch_w_kernel(sp_engine *e, const sp::Kernels &k, int log2n, const Params &q, long long *nfast)
 {
-    const int n = 1 << log2n, P = log2n <= 6 ? 8 : (log2n <= 8 ? 16 : 32), T = n / P, FW = 32 / T, NW = P <= 16 ? SP_W_NW16 : SP_W_NW32, WSH = n == 64 ? 4 : 2;
-    const int tile = 2 * NW * WSH * FW;
+    const int n = 1 << log2n, P = 1 << sp::w_log2p(log2n), tile = sp::w_tile_frames(log2n);
     const long long nf = frames_inside(q, n);
     if (nf == 0) return SP_OK;
     const float2 *twW = nullptr;

@@ -128,18 +128,17 @@ static cudaError_t launch_r64(int sub, const Params *p, int grid, cudaStream_t s
     return launch_r64_v<FMT, false>(*p, grid, st, tw14, tm, pdl, occ_out);
 }
 
-// N = 2048 as 64 x 32 (sp_kernel_rc.cuh): same CTA shape as the 64 x 64 kernel.  render_w_kernel took over N = 256 .. 1024 in
-// round 2 (both layouts); the template still covers C = 4 .. 32.
+// N = 2048 as 64 x 32 (sp_kernel_rc.cuh): same CTA shape as the 64 x 64 kernel.  N = 256 .. 1024 go to render_w_kernel.
 template <int FMT>
 static cudaError_t launch_rc(int log2n, const Params *p, int grid, cudaStream_t st, const float2 *tw14, int *occ_out)
 {
-    using B = RcCfg<5, FMT>;
+    using B = RcCfg<FMT>;
     if (log2n != 11) return cudaErrorInvalidValue;
     if constexpr (!B::OK) {
         if (occ_out) *occ_out = 0;
         return occ_out ? cudaSuccess : cudaErrorInvalidValue;
     } else {
-        return launch_kernel<render_rc_kernel<5, FMT>>(grid, B::THREADS, B::SMEM_BYTES, B::SMEM_BYTES, false, st, occ_out, *p, tw14);
+        return launch_kernel<render_rc_kernel<FMT>>(grid, B::THREADS, B::SMEM_BYTES, B::SMEM_BYTES, false, st, occ_out, *p, tw14);
     }
 }
 

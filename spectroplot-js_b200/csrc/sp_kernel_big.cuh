@@ -17,7 +17,7 @@
 // (persisting access-policy window), so the pre-pass output never reaches HBM: DRAM traffic = input + image.
 // Replaces the hot loops of reference lib/worker.js:68-137 (+ lib/samples.js:313-400, lib/fft_nayuki.js:54-96) for n > 4096.
 #pragma once
-#include "sp_kernel_r64.cuh"
+#include "sp_fused.cuh"
 
 namespace sp {
 
@@ -238,10 +238,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
     const int s = tid >> 6, t = tid & 63;
     float2 *X = reinterpret_cast<float2 *>(s_x + (size_t)s * B::X_BYTES);
 
-    for (int i = tid; i < JH_SIZE; i += B::THREADS) s_jh[i] = 0;
-    const int cmax = p.cmap_len - 1;
-    const JhConst jc = jh_const(p);
-    for (int i = tid; i < 256; i += B::THREADS) s_lut[i] = i <= cmax ? p.lut[jc.rev ? cmax - i : i] : 0u;
+    const JhConst jc = fused_prologue(p, s_jh, s_lut, tid, B::THREADS);
     for (int i = tid; i < T * B::TW_PITCH; i += B::THREADS) s_tw[i] = tw14[i];
     const unsigned jh_base = smem_u32(s_jh) - (JH_MAGIC_BITS << 2);
     const int nfull = p.n_full, R = g.R;
@@ -280,8 +277,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
                         const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;   // :117
                         uint4 a, b;
-                        a.x = lut_at(lut_base, w[0], j); a.y = lut_at(lut_base, w[1], j); a.z = lut_at(lut_base, w[2], j); a.w = lut_at(lut_base, w[3], j);
-                        b.x = lut_at(lut_base, w[4], j); b.y = lut_at(lut_base, w[5], j); b.z = lut_at(lut_base, w[6], j); b.w = lut_at(lut_base, w[7], j);
+                        lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
                     }
                 }
@@ -290,11 +286,9 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
                     const int fl = 8 * h + ht;
                     const long long xl = p.chunk_first + xr0 + ht;
                     const uint2 m0 = s_mm[fl * 2], m1 = s_mm[fl * 2 + 1];
-                    const unsigned umn = min(m0.x, m1.x), umx = max(m0.y, m1.y);
-                    const float mn = fminf(0.0f, fmaf(fast_log2(__uint_as_float(umn)), p.c1, p.c0));       // lib/worker.js:82,102
-                    const float mx = fmaxf(-200.0f, fmaf(fast_log2(__uint_as_float(umx)), p.c1, p.c0));    // lib/worker.js:83,103
-                    atomicMin(reinterpret_cast<unsigned *>(p.fmin) + xl, f2ord(mn));
-                    atomicMax(reinterpret_cast<unsigned *>(p.fmax) + xl, f2ord(mx));
+                    const float2 db = frame_db(min(m0.x, m1.x), max(m0.y, m1.y), p);
+                    atomicMin(reinterpret_cast<unsigned *>(p.fmin) + xl, f2ord(db.x));
+                    atomicMax(reinterpret_cast<unsigned *>(p.fmax) + xl, f2ord(db.y));
                 }
                 __syncwarp();                                   // this warp is done reading the half (and s_mm)
                 if ((ht & 31) == 0) mbar_arrive(s_empty + h);
@@ -382,31 +376,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
 
                 // ---------------- pass A: DFT-64 over the slow input digit, twiddle W_4096^{t*k0} ----------------
                 dft64_between(v, [&] { stream_barrier(s); });               // the previous frame's rows have been read back
-                {
-                    // the exchange stores Z[k0][t] ride between the twiddle products (see render_r64_kernel)
-                    const float4 *twp = reinterpret_cast<const float4 *>(s_tw + t * B::TW_PITCH);
-                    float2 w[8];                                            // w[j] = W^{t*j}, j = 1..7
-                    const float4 a = twp[0], b = twp[1], c = twp[2], d = twp[3];
-                    w[1] = make_float2(a.x, a.y); w[2] = make_float2(a.z, a.w); w[3] = make_float2(b.x, b.y); w[4] = make_float2(b.z, b.w);
-                    w[5] = make_float2(c.x, c.y); w[6] = make_float2(c.z, c.w); w[7] = make_float2(d.x, d.y);
-#pragma unroll
-                    for (int j = 1; j < 8; j++) v[j] = cmul(v[j], w[j]);
-#pragma unroll
-                    for (int k = 0; k < 8; k++) cst(X + k * B::XP + t, v[k]);
-                    float2 hi[8];                                           // hi[i] = W^{t*8i}, i = 1..7
-                    hi[1] = make_float2(d.z, d.w);
-                    const float4 e = twp[4], f = twp[5], gq = twp[6];
-                    hi[2] = make_float2(e.x, e.y); hi[3] = make_float2(e.z, e.w); hi[4] = make_float2(f.x, f.y);
-                    hi[5] = make_float2(f.z, f.w); hi[6] = make_float2(gq.x, gq.y); hi[7] = make_float2(gq.z, gq.w);
-#pragma unroll
-                    for (int i = 1; i < 8; i++) {
-                        v[8 * i] = cmul(v[8 * i], hi[i]);
-#pragma unroll
-                        for (int j = 1; j < 8; j++) v[8 * i + j] = cmul(v[8 * i + j], cun(cmul(cpk(hi[i]), w[j])));
-#pragma unroll
-                        for (int k = 8 * i; k < 8 * i + 8; k++) cst(X + k * B::XP + t, v[k]);
-                    }
-                }
+                twiddle_store64(v, reinterpret_cast<const float4 *>(s_tw + t * B::TW_PITCH), [&](int k) { return X + k * B::XP + t; });
                 stream_barrier(s);
                 // ---------------- pass B: thread k0 = t, DFT-64 over b ----------------
                 {
@@ -422,57 +392,13 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
                 dft<64>(v);                                                 // v[k1] is bin t + 64*k1 of the sub-sequence
 
                 // ---------------- per-bin epilogue (lib/worker.js:85-122) ----------------
-                unsigned umin_i = 0x7f800000u, umax_i = 0u;
+                BinMinMax<true> bm;
                 unsigned *stg = s_stage + fl * B::ST_PITCH + t;
 #pragma unroll
-                for (int m = 0; m < 16; m++) {
-                    unsigned yb[4];
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const float2 vi = cun(v[4 * m + j]);
-                        const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                        // unsigned order on the bit patterns: a NaN wins the max (and is sorted out below), never the min
-                        umin_i = min(umin_i, __float_as_uint(abs2));
-                        umax_i = max(umax_i, __float_as_uint(abs2));
-                        const float l2 = fast_log2(abs2);
-                        float Y;
-                        const float Sx = jh_eval(l2, jc, Y);         // 2^23 + joint index, 2^23 + (cmax - colour index)
-                        red_shared_inc_addr(jh_base + (__float_as_uint(Sx) << 2));
-                        yb[j] = __float_as_uint(Y);
-                    }
-                    stg[m * 64] = __byte_perm(__byte_perm(yb[0], yb[1], 0x0040), __byte_perm(yb[2], yb[3], 0x0040), 0x5410);
-                }
-                unsigned umn = __reduce_min_sync(0xffffffffu, umin_i), umx = __reduce_max_sync(0xffffffffu, umax_i);
-                if (umn < 0x00800000u || umx >= 0x7f800000u) {
-                    // rare (warp-uniform): |X|^2 == 0 (flushed), +inf or NaN in this sub-sequence: see render_r64_kernel
-                    unsigned nzero = 0, nbad = 0, nnan = 0;
-                    float mn = __int_as_float(0x7f800000), mx = 0.0f;
-#pragma unroll
-                    for (int i = 0; i < 64; i++) {
-                        const float2 vi = cun(v[i]);
-                        const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                        nzero += abs2 < 1.17549435e-38f ? 1u : 0u;
-                        nbad += !(abs2 <= 3.402823466e38f) ? 1u : 0u;
-                        nnan += abs2 != abs2 ? 1u : 0u;
-                        mn = fminf(mn, abs2 < 1.17549435e-38f ? 0.0f : abs2);
-                        mx = fmaxf(mx, abs2);
-                    }
-                    nzero = __reduce_add_sync(0xffffffffu, nzero);
-                    nbad = __reduce_add_sync(0xffffffffu, nbad);
-                    nnan = __reduce_add_sync(0xffffffffu, nnan);
-                    umn = __reduce_min_sync(0xffffffffu, __float_as_uint(mn));
-                    umx = __reduce_max_sync(0xffffffffu, __float_as_uint(mx));
-                    if ((t & 31) == 0) {
-                        if (nzero) atomicAdd(&s_jh[JH_ZERO], nzero);
-                        if (nbad) atomicAdd(&s_jh[JH_BAD], nbad);
-                        if (nnan) {
-                            float Yn;
-                            const float Sn = jh_eval(__int_as_float(0x7fffffff), jc, Yn);
-                            atomicSub(&s_jh[__float_as_uint(Sn) - JH_MAGIC_BITS], nnan);
-                            atomicAdd(&s_jh[JH_NAN], nnan);
-                        }
-                    }
-                }
+                for (int m = 0; m < 16; m++) stg[m * 64] = epilogue4(v + 4 * m, bm, jc, jh_base, true, 0u);
+                unsigned umn = __reduce_min_sync(0xffffffffu, bm.lo()), umx = __reduce_max_sync(0xffffffffu, bm.hi());
+                if (umn < 0x00800000u || umx >= 0x7f800000u)    // rare (warp-uniform)
+                    fixup_nonfinite(v, true, (t & 31) == 0, true, s_jh, jc, WarpMin(), WarpMax(), umn, umx);
                 if ((t & 31) == 0) s_mm[fl * 2 + (t >> 5)] = make_uint2(umn, umx);
                 if (step & 1) {                 // this warp has staged its last frame of half step/2 (and its s_mm entries)
                     __syncwarp();
@@ -497,8 +423,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
     }
 
     __syncthreads();
-    for (int i = tid; i < JH_SIZE; i += B::THREADS)
-        if (s_jh[i]) atomicAdd(&p.j_hist[i], (unsigned long long)s_jh[i]);
+    flush_joint_hist(p, s_jh, tid, B::THREADS);
 }
 
 } // namespace sp

@@ -24,14 +24,7 @@
 // Replaces the hot loops of reference lib/worker.js:68-137 (+ lib/samples.js:313-400,
 // lib/fft_nayuki.js:54-96).
 #pragma once
-#include "sp_prims.cuh"
-
-#ifndef SP_XP
-#define SP_XP 0             // timing-only experiment switches (wrong output): 1 conflict-free histogram addresses, 2 no histogram atomics,
-#endif                      // 4 no window, 8 no product twiddles, 16 no log2 / joint index
-#ifndef SP_R64_TMA
-#define SP_R64_TMA 1        // image rows through RGBA tiles + cp.async.bulk.tensor stores, window coefficients from L1-cached global memory
-#endif
+#include "sp_fused.cuh"
 
 namespace sp {
 
@@ -43,44 +36,18 @@ template <int FMT, bool SUB> struct R64Cfg {
     static constexpr bool OK = SUB || ((FMT != FMT_RUNTIME) && SWB <= 8);       // raw frame fits the exchange buffer
     static constexpr int XP = 66;                                                // exchange row pitch (float2): LDS.128 conflict-free
     static constexpr int X_BYTES = 64 * XP * 8;                                  // 33 792 >= 4096 * 8 + 32
-    static constexpr int WIN_PITCH = 64;                                         // floats per thread row, rotated by 4*t (conflict-free LDS.128)
     static constexpr int TW_PITCH = 14;                                          // float2 per thread row: w^1..w^7, w^8, w^16 .. w^56
     static constexpr int ST_PITCH = 1026;                                        // staging words per frame (1024 used)
     static constexpr int RING = 4;                                               // tile indices handed from the store warps' ticket thread to the CTA
-    // SP_R64_TMA: the 16 KB the window table took hold the store warps' RGBA tiles (one 4 KB tile per warp: four boxes of
-    // 32 rows x 8 frames), and the window comes from global memory (p.window_t, 16 KB: it stays in the 28 KB of L1 that the
-    // shared-memory carve-out leaves, because nothing else of this kernel goes through L1 any more)
-    static constexpr bool TMA = SP_R64_TMA != 0;
-    static constexpr int TILE_BYTES = TMA ? (STORE_THREADS / 32) * 4096 : 0;
+    // the store warps' RGBA tiles (one 4 KB tile per warp: four boxes of 32 rows x 8 frames) for the tensor-TMA row stores; the
+    // window comes from global memory (p.window_t, 16 KB: it stays in the 28 KB of L1 that the shared-memory carve-out leaves,
+    // because nothing else of this kernel goes through L1)
+    static constexpr int TILE_BYTES = (STORE_THREADS / 32) * 4096;
     static constexpr size_t SMEM_BYTES = (size_t)STREAMS * X_BYTES + (size_t)F * ST_PITCH * 4 + (size_t)JH_SIZE * 4
-                                       + ((SUB || TMA) ? 0 : (size_t)T * WIN_PITCH * 4) + TILE_BYTES + (size_t)T * TW_PITCH * 8 + 1024 /* LUT */
+                                       + TILE_BYTES + (size_t)T * TW_PITCH * 8 + 1024 /* LUT */
                                        + (size_t)F * 2 * 8 /* s_mm */ + (size_t)2 * F * 8 /* s_fmid */ + 192 + 1024 /* LUT alignment */;
     static_assert(SMEM_BYTES <= 232448, "render_r64_kernel: dynamic shared memory above the 227 KB an sm_100 CTA may have");
 };
-
-// RGBA of byte j of a staged word: table base on a 1 KB boundary of the shared window
-__device__ __forceinline__ unsigned lut_at(unsigned lut_base, unsigned word, int j)
-{
-    const unsigned a = ((j == 0 ? word << 2 : word >> (8 * j - 2)) & 0x3fcu) | lut_base;
-    unsigned v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
-    return v;
-}
-
-// one row segment of 8 pixels: a 256-bit store when every image row is 32-byte aligned (width % 8 == 0), else 8 words
-__device__ __forceinline__ void store_row8(uint32_t *rowp, uint4 a, uint4 b, bool aligned)
-{
-    if (aligned) st_global_256(rowp, a, b);
-    else {
-        rowp[0] = a.x; rowp[1] = a.y; rowp[2] = a.z; rowp[3] = a.w;
-        rowp[4] = b.x; rowp[5] = b.y; rowp[6] = b.z; rowp[7] = b.w;
-    }
-}
-
-__device__ __forceinline__ void stream_barrier(int stream)
-{
-    asm volatile("bar.sync %0, 64;" ::"r"(stream + 1) : "memory");
-}
 
 // tw14: [64][14] float2 = W_4096^{t*k}, k = 1..7, 8, 16, 24, 32, 40, 48, 56
 // OPT = false: the plain spectrogram kernel (the headline path, nothing else compiled in); OPT = true: the same kernel with
@@ -98,11 +65,10 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     const unsigned lut_base = (smem_u32(smem_r64) + 1023u) & ~1023u;
     unsigned char *s_x = smem_r64 + (lut_base - smem_u32(smem_r64)) + 1024;           // [4][X_BYTES] exchange / raw frame
     unsigned *s_lut = reinterpret_cast<unsigned *>(s_x - 1024);                       // [256] RGBA indexed by the staged byte (cmax - g, or g when range < 0)
-    unsigned char *s_tiles = s_x + B::STREAMS * B::X_BYTES;                          // [4 store warps][4 boxes][32 rows][32 B] RGBA, 1 KB aligned (SP_R64_TMA)
+    unsigned char *s_tiles = s_x + B::STREAMS * B::X_BYTES;                          // [4 store warps][4 boxes][32 rows][32 B] RGBA, 1 KB aligned
     unsigned *s_stage = reinterpret_cast<unsigned *>(s_tiles + B::TILE_BYTES);       // [16][1026] colour bytes (4 bins per word)
     unsigned *s_jh = s_stage + F * B::ST_PITCH;                                       // [JH_SIZE] joint histogram
-    float *s_win = reinterpret_cast<float *>(s_jh + JH_SIZE);                         // [64][64] (row t: window[64 a + t] at (a + 4t) mod 64)
-    float2 *s_tw = reinterpret_cast<float2 *>(s_win + ((SUB || B::TMA) ? 0 : T * B::WIN_PITCH));  // [64][14]
+    float2 *s_tw = reinterpret_cast<float2 *>(s_jh + JH_SIZE);                       // [64][14]
     uint2 *s_mm = reinterpret_cast<uint2 *>(s_tw + T * B::TW_PITCH);                  // [16][2] per-warp min/max bit patterns of |X|^2
     float2 *s_fmid = reinterpret_cast<float2 *>(s_mm + F * 2);                       // [2 tile parities][16] raw mid sample of each frame
     uint64_t *s_mbar = reinterpret_cast<uint64_t *>(s_fmid + 2 * F);                  // [4]
@@ -120,13 +86,8 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
     unsigned char *raw = reinterpret_cast<unsigned char *>(X);
     uint64_t *mbar = s_mbar + s;
 
-    for (int i = tid; i < JH_SIZE; i += B::THREADS) s_jh[i] = 0;
-    const int cmax = p.cmap_len - 1;
-    const JhConst jc = jh_const(p);
-    for (int i = tid; i < 256; i += B::THREADS) s_lut[i] = i <= cmax ? p.lut[jc.rev ? cmax - i : i] : 0u;
+    const JhConst jc = fused_prologue(p, s_jh, s_lut, tid, B::THREADS);
     for (int i = tid; i < T * B::TW_PITCH; i += B::THREADS) s_tw[i] = tw14[i];
-    if constexpr (!SUB && !B::TMA)
-        for (int i = tid; i < N; i += B::THREADS) s_win[(i & 63) * B::WIN_PITCH + (((i >> 6) + 4 * (i & 63)) & 63)] = p.window[i];
     const unsigned jh_base = smem_u32(s_jh) - (JH_MAGIC_BITS << 2);      // address of joint bin j = S.bits * 4 + jh_base (mod 2^32)
     const int nfull = p.n_full, sub_r = p.sub_r;
 
@@ -225,7 +186,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                         }
                     }
                 }
-                if constexpr (B::TMA && !SUB) {
+                if constexpr (!SUB) {
                     if (p.use_tma && live && (!OPT || !p.waterfall)) {
                         // RGBA tiles + tensor-TMA stores.  In iteration i this warp holds bins kb .. kb + 31 (kb = 32*(w & 1) + 64*(4m + j))
                         // for j = 0..3: four boxes of 32 consecutive image rows y0 .. y0 + 31, y0 = (n/2 - kb - 31) mod n (row r of a
@@ -249,8 +210,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
 #pragma unroll
                             for (int j = 0; j < 4; j++) {
                                 uint4 a, b;
-                                a.x = lut_at(lut_base, w[0], j); a.y = lut_at(lut_base, w[1], j); a.z = lut_at(lut_base, w[2], j); a.w = lut_at(lut_base, w[3], j);
-                                b.x = lut_at(lut_base, w[4], j); b.y = lut_at(lut_base, w[5], j); b.z = lut_at(lut_base, w[6], j); b.w = lut_at(lut_base, w[7], j);
+                                lut_row8(lut_base, w, j, a, b);
                                 *reinterpret_cast<uint4 *>(tile + j * 1024 + toff) = a;
                                 *reinterpret_cast<uint4 *>(tile + j * 1024 + (toff ^ 16u)) = b;
                                 if (k0 + 64 * (4 * m + j) == N / 2)        // bin n/2 -> image row 0
@@ -269,7 +229,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     }
                 }
 #pragma unroll 1
-                for (int i = 0; i < ((live && (!OPT || SUB || !p.waterfall) && !(B::TMA && !SUB && p.use_tma)) ? 8 : 0); i++) {
+                for (int i = 0; i < ((live && (!OPT || SUB || !p.waterfall) && !(!SUB && p.use_tma)) ? 8 : 0); i++) {
                     // bins k0 + 64*(4m + j), j = 0..3, of the half's 8 frames: one 32-byte sector per row
                     const int id = ht + B::STORE_THREADS * i, k0 = id & 63, m = id >> 6;
                     const unsigned *src = s_stage + (8 * h) * B::ST_PITCH + m * 64 + k0;
@@ -283,10 +243,8 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                         const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;   // :117
                         uint4 a, b;
-                        if (!(p.dbg & 4)) {
-                            a.x = lut_at(lut_base, w[0], j); a.y = lut_at(lut_base, w[1], j); a.z = lut_at(lut_base, w[2], j); a.w = lut_at(lut_base, w[3], j);
-                            b.x = lut_at(lut_base, w[4], j); b.y = lut_at(lut_base, w[5], j); b.z = lut_at(lut_base, w[6], j); b.w = lut_at(lut_base, w[7], j);
-                        } else { a = make_uint4(w[0], w[1], w[2], w[3]); b = make_uint4(w[4], w[5], w[6], w[7]); }
+                        if (!(p.dbg & 4)) lut_row8(lut_base, w, j, a, b);
+                        else { a = make_uint4(w[0], w[1], w[2], w[3]); b = make_uint4(w[4], w[5], w[6], w[7]); }
                         if (!(p.dbg & 1)) store_row8(rowp, a, b, rows_aligned);
                     }
                 }
@@ -295,13 +253,11 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     const int fl = 8 * h + ht;
                     const long long xl = p.chunk_first + xr0 + fl;
                     const uint2 m0 = s_mm[fl * 2], m1 = s_mm[fl * 2 + 1];
-                    const unsigned umn = min(m0.x, m1.x), umx = max(m0.y, m1.y);
-                    const float mn = fminf(0.0f, fmaf(fast_log2(__uint_as_float(umn)), p.c1, p.c0));       // lib/worker.js:82,102
-                    const float mx = fmaxf(-200.0f, fmaf(fast_log2(__uint_as_float(umx)), p.c1, p.c0));    // lib/worker.js:83,103
+                    const float2 db = frame_db(min(m0.x, m1.x), max(m0.y, m1.y), p);
                     if constexpr (SUB) {
-                        atomicMin(reinterpret_cast<unsigned *>(p.fmin) + xl, f2ord(mn));
-                        atomicMax(reinterpret_cast<unsigned *>(p.fmax) + xl, f2ord(mx));
-                    } else { p.fmin[xl] = mn; p.fmax[xl] = mx; p.fmid[xl] = s_fmid[(kk & 1) * F + fl]; }
+                        atomicMin(reinterpret_cast<unsigned *>(p.fmin) + xl, f2ord(db.x));
+                        atomicMax(reinterpret_cast<unsigned *>(p.fmax) + xl, f2ord(db.y));
+                    } else { p.fmin[xl] = db.x; p.fmax[xl] = db.y; p.fmid[xl] = s_fmid[(kk & 1) * F + fl]; }
                 }
                 __syncwarp();                                   // this warp is done reading the half (and s_mm)
                 if ((ht & 31) == 0) mbar_arrive(s_empty + h);
@@ -309,7 +265,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
             tile = ring_get(++kk);
             if (ht == 0 && tile < p.ntiles) ring_put(kk + 1, ticket());
         }
-        if constexpr (B::TMA && !SUB) bulk_wait_read0();        // the tiles must outlive the last tensor stores
+        if constexpr (!SUB) bulk_wait_read0();        // the tiles must outlive the last tensor stores
     } else {
     // ================= FFT warps: four frame streams =================
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(B::FFT_REGS));
@@ -350,11 +306,11 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     for (int n1 = 0; n1 < 8; n1++) v[8 * n1 + n0] = cld(reinterpret_cast<const float2 *>(raw) + T * (8 * n1 + n0) + t);
             } else {
                 const unsigned char *rp = raw + s_off[s * 2 + fpar];
-                const float4 *wrow = B::TMA ? p.window_t + t : reinterpret_cast<const float4 *>(s_win + t * B::WIN_PITCH);
+                const float4 *wrow = p.window_t + t;
 #pragma unroll
                 for (int qq = 0; qq < 16; qq++) {
                     const int q = 2 * (qq & 7) + (qq >> 3);
-                    const float4 w = (SP_XP & 4) ? make_float4(1.f, 1.f, 1.f, 1.f) : B::TMA ? __ldg(wrow + 64 * q) : wrow[(q + t) & 15];
+                    const float4 w = __ldg(wrow + 64 * q);
                     cf d[4];
 #pragma unroll
                     for (int c = 0; c < 4; c++) d[c] = decode_raw_cf<FMT>(rp, T * (4 * q + c) + t, p.format);
@@ -368,31 +324,8 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
             fpar ^= 1;
             // ---------------- pass A: DFT-64 over the slow input digit; the raw frame is released between its two stages ----------------
             dft64_between(v, [&] { stream_barrier(s); });
-            {
-                // twiddles W^{t*k}, each product followed by its exchange store Z[k0][t] (the stores ride between the FFMA2)
-                const float4 *twp = reinterpret_cast<const float4 *>(s_tw + t * B::TW_PITCH);
-                float2 w[8];                                            // w[j] = W^{t*j}, j = 1..7
-                const float4 a = twp[0], b = twp[1], c = twp[2], d = twp[3];
-                w[1] = make_float2(a.x, a.y); w[2] = make_float2(a.z, a.w); w[3] = make_float2(b.x, b.y); w[4] = make_float2(b.z, b.w);
-                w[5] = make_float2(c.x, c.y); w[6] = make_float2(c.z, c.w); w[7] = make_float2(d.x, d.y);
-#pragma unroll
-                for (int j = 1; j < 8; j++) v[j] = cmul(v[j], w[j]);
-#pragma unroll
-                for (int j = 0; j < 8; j++) cst(X + j * B::XP + t, v[j]);
-                float2 hi[8];                                           // hi[i] = W^{t*8i}, i = 1..7
-                hi[1] = make_float2(d.z, d.w);
-                const float4 e = twp[4], f = twp[5], g = twp[6];
-                hi[2] = make_float2(e.x, e.y); hi[3] = make_float2(e.z, e.w); hi[4] = make_float2(f.x, f.y);
-                hi[5] = make_float2(f.z, f.w); hi[6] = make_float2(g.x, g.y); hi[7] = make_float2(g.z, g.w);
-#pragma unroll
-                for (int i = 1; i < 8; i++) {
-                    v[8 * i] = cmul(v[8 * i], hi[i]);
-#pragma unroll
-                    for (int j = 1; j < 8; j++) v[8 * i + j] = cmul(v[8 * i + j], (SP_XP & 8) ? w[j] : cun(cmul(cpk(hi[i]), w[j])));
-#pragma unroll
-                    for (int j = 0; j < 8; j++) cst(X + (8 * i + j) * B::XP + t, v[8 * i + j]);
-                }
-            }
+            // twiddles W^{t*k}, each product followed by its exchange store Z[k0][t]
+            twiddle_store64(v, reinterpret_cast<const float4 *>(s_tw + t * B::TW_PITCH), [&](int k) { return X + k * B::XP + t; });
             stream_barrier(s);
             // ---------------- pass B: thread k0 = t, DFT-64 over b; v[k1] is bin t + 64*k1 ----------------
             {
@@ -464,75 +397,14 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     }
 
                     // ---------------- per-bin epilogue (lib/worker.js:85-122) ----------------
-                    float amin = __int_as_float(0x7f800000), amax = 0.0f, prev = 0.0f;
-                    unsigned umin_i = 0x7f800000u, umax_i = 0u;
+                    BinMinMax<FLOAT_IN> bm;
                     unsigned *stg = s_stage + fl * B::ST_PITCH + t;
 #pragma unroll
-                    for (int m = 0; m < 16; m++) {
-                        unsigned yb[4];
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            const float2 vi = cun(v[4 * m + j]);
-                            const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                            if constexpr (FLOAT_IN) {
-                                // unsigned order on the bit patterns: a NaN wins the max (and is sorted out below), never the min
-                                umin_i = min(umin_i, __float_as_uint(abs2));
-                                umax_i = max(umax_i, __float_as_uint(abs2));
-                            } else if (j & 1) {                          // 3-input min / max: one FMNMX3 per two bins
-                                amin = fmin3(amin, prev, abs2);
-                                amax = fmax3(amax, prev, abs2);
-                            } else prev = abs2;
-                            const float l2 = (SP_XP & 16) ? abs2 : fast_log2(abs2);
-                            float Y;
-                            const float S = (SP_XP & 16) ? (Y = l2, __uint_as_float((__float_as_uint(l2) >> 20) + JH_MAGIC_BITS)) : jh_eval(l2, jc, Y);          // 2^23 + joint index, 2^23 + (cmax - colour index)
-                            if constexpr ((SP_XP & 1) != 0) red_shared_inc_addr(smem_u32(s_jh) + ((tid & 31) << 2) + (__float_as_uint(S) & 0x380u));
-                            else if constexpr (!(SP_XP & 2)) red_shared_inc_addr(jbase + (__float_as_uint(S) << 2));
-                            yb[j] = __float_as_uint(Y);
-                        }
-                        // bins t + 64*(4m .. 4m+3) of frame fl: four colour bytes in one word
-                        stg[m * 64] = __byte_perm(__byte_perm(yb[0], yb[1], 0x0040), __byte_perm(yb[2], yb[3], 0x0040), 0x5410);
-                    }
-                    unsigned umn, umx;
-                    if constexpr (FLOAT_IN) {
-                        umn = __reduce_min_sync(0xffffffffu, umin_i);
-                        umx = __reduce_max_sync(0xffffffffu, umax_i);
-                    } else {
-                        // |X|^2 >= 0: the bit patterns order like the values
-                        umn = __reduce_min_sync(0xffffffffu, __float_as_uint(amin));
-                        umx = __reduce_max_sync(0xffffffffu, __float_as_uint(amax));
-                    }
-                    if (umn < 0x00800000u || umx >= 0x7f800000u) {
-                        // rare (warp-uniform): the frame holds |X|^2 == 0 (flushed: d0 = -inf), +inf or NaN.  Count them for
-                        // the bin-0 fix-ups (lib/worker.js:105-106: ~~(+-Infinity) == ~~NaN == 0) and redo min / max the way
-                        // the reference's `<` / `>` see them (NaN never wins).
-                        unsigned nzero = 0, nbad = 0, nnan = 0;
-                        float mn = __int_as_float(0x7f800000), mx = 0.0f;
-#pragma unroll
-                        for (int i = 0; i < 64; i++) {
-                            const float2 vi = cun(v[i]);
-                            const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                            nzero += abs2 < 1.17549435e-38f ? 1u : 0u;
-                            nbad += !(abs2 <= 3.402823466e38f) ? 1u : 0u;
-                            nnan += abs2 != abs2 ? 1u : 0u;
-                            mn = fminf(mn, abs2 < 1.17549435e-38f ? 0.0f : abs2);
-                            mx = fmaxf(mx, abs2);
-                        }
-                        nzero = __reduce_add_sync(0xffffffffu, nzero);
-                        nbad = __reduce_add_sync(0xffffffffu, nbad);
-                        nnan = __reduce_add_sync(0xffffffffu, nnan);
-                        umn = __reduce_min_sync(0xffffffffu, __float_as_uint(mn));
-                        umx = __reduce_max_sync(0xffffffffu, __float_as_uint(mx));
-                        if ((t & 31) == 0 && valid) {
-                            if (nzero) atomicAdd(&s_jh[JH_ZERO], nzero);
-                            if (nbad) atomicAdd(&s_jh[JH_BAD], nbad);
-                            if (nnan) {                 // NaN pixels were counted under the joint index sat(NaN) = 0 yields: move them
-                                float Yn;
-                                const float Sn = jh_eval(__int_as_float(0x7fffffff), jc, Yn);
-                                atomicSub(&s_jh[__float_as_uint(Sn) - JH_MAGIC_BITS], nnan);
-                                atomicAdd(&s_jh[JH_NAN], nnan);
-                            }
-                        }
-                    }
+                    for (int m = 0; m < 16; m++)                        // bins t + 64*(4m .. 4m+3) of frame fl: four colour bytes in one word
+                        stg[m * 64] = epilogue4(v + 4 * m, bm, jc, jbase, true, 0u);
+                    unsigned umn = __reduce_min_sync(0xffffffffu, bm.lo()), umx = __reduce_max_sync(0xffffffffu, bm.hi());
+                    if (umn < 0x00800000u || umx >= 0x7f800000u)        // rare (warp-uniform)
+                        fixup_nonfinite(v, true, (t & 31) == 0, valid, s_jh, jc, WarpMin(), WarpMax(), umn, umx);
                     if ((t & 31) == 0) s_mm[fl * 2 + (t >> 5)] = make_uint2(umn, umx);
                     if (step & 1) {                 // this warp has staged its last frame of half step/2 (and its s_mm entries)
                         __syncwarp();
@@ -548,8 +420,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
 
     __syncthreads();
     griddep_wait();                         // (the FFT warps' first global write)
-    for (int i = tid; i < JH_SIZE; i += B::THREADS)
-        if (s_jh[i]) atomicAdd(&p.j_hist[i], (unsigned long long)s_jh[i]);
+    flush_joint_hist(p, s_jh, tid, B::THREADS);
 }
 
 } // namespace sp

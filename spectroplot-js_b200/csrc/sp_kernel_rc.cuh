@@ -1,36 +1,36 @@
-// sp_kernel_rc.cuh — the 64-points-per-thread render kernel for N = 64 * C, C = 4, 8, 16, 32 (N = 256 .. 2048).
+// sp_kernel_rc.cuh — the 64-points-per-thread render kernel for N = 2048 = 64 x C, C = 32.
 //
 // Same machine as render_r64_kernel (sp_kernel_r64.cuh), with the frame folded differently:
-//   * N = 64 x C: C threads transform a frame, each holding 64 complex points: dft<64> over the slow input digit
-//     (stride C), twiddle W_N^{t*k0}, ONE shared-memory exchange, then 64 / C row transforms dft<C> per thread
-//     (thread t owns rows k0 = t*64/C .. +64/C-1, bins k0 + 64*k1);
-//   * a stream of 64 threads therefore works on FS = 64 / C frames at a time, its raw frames prefetched by FS bulk
-//     copies (TMA) on one mbarrier into the stream's exchange buffer;
-//   * joint histogram (one shared-memory atomic per pixel), colour bytes staged in two halves of 512 / C frames,
-//     store warpgroup with full / empty mbarriers, setmaxnreg — exactly as in render_r64_kernel; a lane of the store
-//     warps still writes one 32-byte sector (8 frames of one row), and adjacent lanes take adjacent 8-frame groups,
-//     so a row receives 64 .. 128 contiguous bytes per instruction.
-// Only full tiles of 1024 / C frames inside the buffer come here (spectrogram layout, cmap_len <= 256); the engine
-// routes everything else through render_kernel.
+//   * N = 64 x C: C = 32 threads (one warp) transform a frame, each holding 64 complex points: dft<64> over the slow input
+//     digit (stride C), twiddle W_N^{t*k0}, ONE shared-memory exchange, then RPT = 64 / C = 2 row transforms dft<C> per
+//     thread (thread t owns rows k0 = 2t, 2t + 1, bins k0 + 64*k1);
+//   * a stream of 64 threads therefore works on FS = 2 frames at a time, its raw frames prefetched by FS bulk copies
+//     (TMA) on one mbarrier into the stream's exchange buffer;
+//   * joint histogram (one shared-memory atomic per pixel), colour bytes staged in two halves of 16 frames, store
+//     warpgroup with full / empty mbarriers, setmaxnreg — exactly as in render_r64_kernel; a lane of the store warps
+//     still writes one 32-byte sector (8 frames of one row), and adjacent lanes take the two 8-frame groups of a half,
+//     so a row receives 64 contiguous bytes per instruction.
+// Only full tiles of 32 frames inside the buffer come here (spectrogram layout, cmap_len <= 256); the engine routes
+// everything else through render_kernel.
 // Replaces the hot loops of reference lib/worker.js:68-137 (+ lib/samples.js:313-400, lib/fft_nayuki.js:54-96).
 #pragma once
-#include "sp_kernel_r64.cuh"
+#include "sp_fused.cuh"
 
 namespace sp {
 
-template <int LOG2C, int FMT> struct RcCfg {
-    static constexpr int C = 1 << LOG2C, N = 64 * C, RPT = 64 / C, FS = 64 / C;   // threads per frame, rows per thread, frames per stream step
+template <int FMT> struct RcCfg {
+    static constexpr int C = 32, N = 64 * C, RPT = 64 / C, FS = 64 / C;          // threads per frame, rows per thread, frames per stream step
     static constexpr int STREAMS = 4, FFT_THREADS = 256, STORE_THREADS = 128, THREADS = FFT_THREADS + STORE_THREADS;
     static constexpr int STEPS = 4, SF = STREAMS * FS, F = STEPS * SF, HF = F / 2;  // frames per step / tile / staging half
     static constexpr int FFT_REGS = 232, STORE_REGS = 40;
     static constexpr int SWB = sample_width(FMT == FMT_RUNTIME ? CF64 : FMT);
     static constexpr bool OK = (FMT != FMT_RUNTIME) && SWB <= 8;
     static constexpr int XP = 66;                                                // float2 per 64-point chunk (LDS.128 conflict-free)
-    static constexpr int FP = C * XP + (C < 16 ? 16 - C : 0);                    // float2 per frame of the exchange buffer
+    static constexpr int FP = C * XP;                                            // float2 per frame of the exchange buffer
     static constexpr int RAWP = N * SWB + 32;                                    // bytes per raw frame slot
     static constexpr int X_BYTES = (FS * FP * 8 > FS * RAWP ? FS * FP * 8 : FS * RAWP) + 15 & ~15;
-    static constexpr int G = HF / 8 < 4 ? HF / 8 : 4;                            // adjacent lanes of a store warp = adjacent 8-frame groups
-    static constexpr int FPW = N / 4 + (G == 2 ? 2 : 1);                         // staging words per frame
+    static constexpr int G = HF / 8;                                             // adjacent lanes of a store warp = adjacent 8-frame groups
+    static constexpr int FPW = N / 4 + 2;                                        // staging words per frame
     static constexpr int HALF_WORDS = HF * FPW;
     static constexpr int TW_PITCH = 14;
     static constexpr size_t SMEM_BYTES = (size_t)STREAMS * X_BYTES + (size_t)2 * HALF_WORDS * 4 + (size_t)JH_SIZE * 4 + (size_t)N * 4
@@ -39,10 +39,10 @@ template <int LOG2C, int FMT> struct RcCfg {
 };
 
 // tw14: [C][14] float2 = W_N^{t*k}, k = 1..7, 8, 16, 24, 32, 40, 48, 56
-template <int LOG2C, int FMT>
+template <int FMT>
 __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const float2 *__restrict__ tw14)
 {
-    using B = RcCfg<LOG2C, FMT>;
+    using B = RcCfg<FMT>;
     constexpr int C = B::C, N = B::N, RPT = B::RPT, FS = B::FS, F = B::F, HF = B::HF;
     constexpr bool FLOAT_IN = FMT == CF32 || FMT == CF64 || FMT == FMT_RUNTIME;   // |X|^2 may be +inf / NaN
     extern __shared__ __align__(128) unsigned char smem_rc[];
@@ -67,10 +67,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
     float2 *X = reinterpret_cast<float2 *>(xs) + fi * B::FP;                     // this frame's exchange area
     uint64_t *mbar = s_mbar + s;
 
-    for (int i = tid; i < JH_SIZE; i += B::THREADS) s_jh[i] = 0;
-    const int cmax = p.cmap_len - 1;
-    const JhConst jc = jh_const(p);
-    for (int i = tid; i < 256; i += B::THREADS) s_lut[i] = i <= cmax ? p.lut[jc.rev ? cmax - i : i] : 0u;
+    const JhConst jc = fused_prologue(p, s_jh, s_lut, tid, B::THREADS);
     for (int i = tid; i < C * B::TW_PITCH; i += B::THREADS) s_tw[i] = tw14[i];
     for (int i = tid; i < N; i += B::THREADS) s_win[(i % C) * 64 + (((i / C) + 4 * (i % C)) & 63)] = p.window[i];
     const unsigned jh_base = smem_u32(s_jh) - (JH_MAGIC_BITS << 2);
@@ -125,7 +122,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
                     // waterfall layout (lib/worker.js:116): frame x is image row nframes - 1 - x, bin b is column (b + n/2 - 1) mod n.
                     // Item = (frame, m, o): o = tc*RPT + r runs over 64 consecutive bins, so the lanes of a store write
                     // consecutive columns (128 contiguous bytes); the staged word of (m, o) sits at m*64 + r*C + tc.
-                    constexpr int MG = C / 4 > 0 ? C / 4 : 1;           // 64-bin groups per staged byte position
+                    constexpr int MG = C / 4;                           // 64-bin groups per staged byte position
 #pragma unroll 1
                     for (int i = 0; i < HF * MG * 64 / B::STORE_THREADS; i++) {
                         const int id = ht + B::STORE_THREADS * i, o = id & 63, rest = id >> 6;
@@ -156,8 +153,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
                         const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0 + 8 * grp;   // :117
                         uint4 a, b;
-                        a.x = lut_at(lut_base, w[0], j); a.y = lut_at(lut_base, w[1], j); a.z = lut_at(lut_base, w[2], j); a.w = lut_at(lut_base, w[3], j);
-                        b.x = lut_at(lut_base, w[4], j); b.y = lut_at(lut_base, w[5], j); b.z = lut_at(lut_base, w[6], j); b.w = lut_at(lut_base, w[7], j);
+                        lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
                     }
                 }
@@ -166,8 +162,9 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
                     if (xr0 + HF * h + fl >= p.chunk_frames) break;
                     const long long xl = p.chunk_first + xr0 + HF * h + fl;
                     const uint2 mm = s_mm[HF * h + fl];
-                    p.fmin[xl] = fminf(0.0f, fmaf(fast_log2(__uint_as_float(mm.x)), p.c1, p.c0));        // lib/worker.js:82,102
-                    p.fmax[xl] = fmaxf(-200.0f, fmaf(fast_log2(__uint_as_float(mm.y)), p.c1, p.c0));     // lib/worker.js:83,103
+                    const float2 db = frame_db(mm.x, mm.y, p);
+                    p.fmin[xl] = db.x;
+                    p.fmax[xl] = db.y;
                 }
                 __syncwarp();                                   // this warp is done reading the half (and s_mm)
                 if ((ht & 31) == 0) mbar_arrive(s_empty + h);
@@ -178,8 +175,6 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(B::FFT_REGS));
     unsigned fpar = 0;                      // parity of this stream's step counter (mbarrier phase, s_off slot)
     if (ts == 0 && tile < p.ntiles) stage(tile * F + s * FS, 0);
-    constexpr unsigned GROUP_BASE_MASK = C == 32 ? 0xffffffffu : ((1u << (C & 31)) - 1u);
-    const unsigned gmask = GROUP_BASE_MASK << ((ts & 31) / C * C);               // lanes of this frame
 
     while (tile < p.ntiles) {
         const long long xr0 = tile * F;
@@ -215,7 +210,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
             dft64_between(v, [&] { stream_barrier(s); });               // every thread of the stream has consumed its raw frame
             {
                 // each twiddled row goes straight to the 64-point chunk k0 / RPT (owner thread) at (k0 % RPT) * C + t: the
-                // exchange stores ride between the twiddle products (see render_r64_kernel)
+                // exchange stores ride between the twiddle products
                 const float4 *twp = reinterpret_cast<const float4 *>(s_tw + t * B::TW_PITCH);
                 float2 w[8], hi[8];                                     // w[j] = W^{t*j}, hi[i] = W^{t*8i}
                 const float4 a = twp[0], b = twp[1], c = twp[2], d = twp[3], e = twp[4], f = twp[5], g = twp[6];
@@ -263,73 +258,16 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
             }
 
             // ---------------- per-bin epilogue (lib/worker.js:85-122) ----------------
-            float amin = __int_as_float(0x7f800000), amax = 0.0f, prev = 0.0f;
-            unsigned umin_i = 0x7f800000u, umax_i = 0u;
+            BinMinMax<FLOAT_IN> bm;
             unsigned *stg = s_stage + half * B::HALF_WORDS + (fl - half * HF) * B::FPW + t;
 #pragma unroll
             for (int r = 0; r < RPT; r++)
 #pragma unroll
-                for (int m = 0; m < C / 4; m++) {
-                    unsigned yb[4];
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const float2 vi = cun(v[r * C + 4 * m + j]);
-                        const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                        if constexpr (FLOAT_IN) {
-                            umin_i = min(umin_i, __float_as_uint(abs2));
-                            umax_i = max(umax_i, __float_as_uint(abs2));
-                        } else if (j & 1) {
-                            amin = fmin3(amin, prev, abs2);
-                            amax = fmax3(amax, prev, abs2);
-                        } else prev = abs2;
-                        const float l2 = fast_log2(abs2);
-                        float Y;
-                        const float S = jh_eval(l2, jc, Y);
-                        red_shared_inc_addr(valid ? jh_base + (__float_as_uint(S) << 2) : dump);
-                        yb[j] = __float_as_uint(Y);
-                    }
-                    // bins (t*RPT + r) + 64*(4m .. 4m+3): four colour bytes in one word at m*64 + r*C + t
-                    stg[m * 64 + r * C] = __byte_perm(__byte_perm(yb[0], yb[1], 0x0040), __byte_perm(yb[2], yb[3], 0x0040), 0x5410);
-                }
-            unsigned umn, umx;
-            if constexpr (FLOAT_IN) {
-                umn = __reduce_min_sync(gmask, umin_i);
-                umx = __reduce_max_sync(gmask, umax_i);
-            } else {
-                umn = __reduce_min_sync(gmask, __float_as_uint(amin));
-                umx = __reduce_max_sync(gmask, __float_as_uint(amax));
-            }
-            if (__any_sync(0xffffffffu, umn < 0x00800000u || umx >= 0x7f800000u)) {
-                // rare (warp-uniform): a frame of this warp holds |X|^2 == 0 (flushed), +inf or NaN: see render_r64_kernel
-                unsigned nzero = 0, nbad = 0, nnan = 0;
-                float mn = __int_as_float(0x7f800000), mx = 0.0f;
-#pragma unroll
-                for (int i = 0; i < 64; i++) {
-                    const float2 vi = cun(v[i]);
-                    const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                    nzero += abs2 < 1.17549435e-38f ? 1u : 0u;
-                    nbad += !(abs2 <= 3.402823466e38f) ? 1u : 0u;
-                    nnan += abs2 != abs2 ? 1u : 0u;
-                    mn = fminf(mn, abs2 < 1.17549435e-38f ? 0.0f : abs2);
-                    mx = fmaxf(mx, abs2);
-                }
-                if (!valid) nzero = nbad = nnan = 0;
-                nzero = __reduce_add_sync(0xffffffffu, nzero);
-                nbad = __reduce_add_sync(0xffffffffu, nbad);
-                nnan = __reduce_add_sync(0xffffffffu, nnan);
-                umn = __reduce_min_sync(gmask, __float_as_uint(mn));
-                umx = __reduce_max_sync(gmask, __float_as_uint(mx));
-                if ((ts & 31) == 0) {
-                    if (nzero) atomicAdd(&s_jh[JH_ZERO], nzero);
-                    if (nbad) atomicAdd(&s_jh[JH_BAD], nbad);
-                    if (nnan) {
-                        float Yn;
-                        const float Sn = jh_eval(__int_as_float(0x7fffffff), jc, Yn);
-                        atomicSub(&s_jh[__float_as_uint(Sn) - JH_MAGIC_BITS], nnan);
-                        atomicAdd(&s_jh[JH_NAN], nnan);
-                    }
-                }
-            }
+                for (int m = 0; m < C / 4; m++)     // bins (t*RPT + r) + 64*(4m .. 4m+3): four colour bytes in one word at m*64 + r*C + t
+                    stg[m * 64 + r * C] = epilogue4(v + r * C + 4 * m, bm, jc, jh_base, valid, dump);
+            unsigned umn = __reduce_min_sync(0xffffffffu, bm.lo()), umx = __reduce_max_sync(0xffffffffu, bm.hi());
+            if (__any_sync(0xffffffffu, umn < 0x00800000u || umx >= 0x7f800000u))   // rare (warp-uniform)
+                fixup_nonfinite(v, valid, (ts & 31) == 0, true, s_jh, jc, WarpMin(), WarpMax(), umn, umx);
             if (t == 0) s_mm[fl] = make_uint2(umn, umx);
             if (step & 1) {                 // this warp has staged its last frames of the half (and their s_mm entries)
                 __syncwarp();
@@ -342,8 +280,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
     } // FFT warps
 
     __syncthreads();
-    for (int i = tid; i < JH_SIZE; i += B::THREADS)
-        if (s_jh[i]) atomicAdd(&p.j_hist[i], (unsigned long long)s_jh[i]);
+    flush_joint_hist(p, s_jh, tid, B::THREADS);
 }
 
 } // namespace sp

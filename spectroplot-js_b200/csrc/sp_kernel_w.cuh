@@ -20,38 +20,25 @@
 // (dB tap, longer colormaps, remainder frames) stays on render_kernel.  Replaces the hot loops of reference lib/worker.js:68-137 (+ lib/samples.js:313-400,
 // lib/fft_nayuki.js:54-96).
 #pragma once
-#include "sp_kernel_r64.cuh"
-
-// tuning knobs (A/B builds, profiles/r02_w_kernel_tuning.txt): FFT warps per CTA for P <= 16 / P = 32 (multiples of 4: setmaxnreg
-// works on warpgroups) and whether the P = 32 twiddles live in registers (8 warps x 232 registers: adopted, +4 % at N = 512) or in
-// shared memory (12 warps x 152 registers)
-#ifndef SP_W_NW16
-#define SP_W_NW16 16
-#endif
-#ifndef SP_W_NW32
-#define SP_W_NW32 8
-#endif
-#ifndef SP_W_TWREG32
-#define SP_W_TWREG32 1
-#endif
-#ifndef SP_W_SEP
-#define SP_W_SEP 1
-#endif
-#ifndef SP_W_SG
-#define SP_W_SG 1
-#endif
-#ifndef SP_W_SG_MAXT
-#define SP_W_SG_MAXT 32     // largest T that shares a bulk copy between two warp-steps (A/B: 8 = round-2 build before the last change)
-#endif
-#ifndef SP_W_STSB
-#define SP_W_STSB 1         // exchange stores between the twiddle products (0: in a row after them; the same within noise at N = 512)
-#endif
+#include "sp_fused.cuh"
 
 namespace sp {
 
+// The shape of render_w_kernel for N = 2^log2n, which the engine's tile count needs as well: N = P x T with P = 8, 16, 32;
+// NW FFT warps (A/B: profiles/r02_w_kernel_tuning.txt; for P = 32 8 warps of 232 registers that hold the twiddles beat
+// 12 warps of 152 that read them from shared memory); WSH warp-steps of FW = 32 / T frames per warp and staging half.
+constexpr int w_log2p(int log2n) { return log2n <= 6 ? 3 : (log2n <= 8 ? 4 : 5); }
+constexpr int w_warps(int P) { return P <= 16 ? 16 : 8; }
+constexpr int w_steps(int N) { return N == 64 ? 4 : 2; }
+constexpr int w_tile_frames(int log2n)              // frames of a tile: two staging halves
+{
+    return 2 * w_warps(1 << w_log2p(log2n)) * w_steps(1 << log2n) * (32 >> (log2n - w_log2p(log2n)));
+}
+
 template <int LOG2P, int LOG2T, int FMT> struct WCfg {
     static constexpr int P = 1 << LOG2P, T = 1 << LOG2T, N = P * T, FW = 32 / T, Q = P / T;
-    static constexpr int NW = P <= 16 ? SP_W_NW16 : SP_W_NW32;                   // FFT warps
+    static_assert(LOG2P == w_log2p(LOG2P + LOG2T), "the P x T split of N is w_log2p's");
+    static constexpr int NW = w_warps(P);                                        // FFT warps
     static_assert(NW % 4 == 0, "setmaxnreg is a warpgroup (4 warps) operation: the FFT warps must fill whole warpgroups (a mixed one hangs)");
     static constexpr int FFT_THREADS = 32 * NW, STORE_THREADS = 128, THREADS = FFT_THREADS + STORE_THREADS;
     static constexpr int STORE_REGS = 40;
@@ -59,8 +46,8 @@ template <int LOG2P, int LOG2T, int FMT> struct WCfg {
     static constexpr int LAUNCH_REGS = (65536 / THREADS) / 8 * 8 > 255 ? 248 : (65536 / THREADS) / 8 * 8;
     static constexpr int FFT_REGS_RAW = (THREADS * LAUNCH_REGS - STORE_THREADS * STORE_REGS) / FFT_THREADS / 8 * 8;
     static constexpr int FFT_REGS = FFT_REGS_RAW > 232 ? 232 : FFT_REGS_RAW;
-    static constexpr int WSH = N == 64 ? 4 : 2;                                  // warp-steps per warp and staging half
-    static constexpr int HF = NW * WSH * FW, F = 2 * HF;                         // frames per staging half / tile
+    static constexpr int WSH = w_steps(N);                                       // warp-steps per warp and staging half
+    static constexpr int F = w_tile_frames(LOG2P + LOG2T), HF = F / 2;           // frames per tile / staging half (NW * WSH * FW)
     static constexpr int SWB = sample_width(FMT == FMT_RUNTIME ? CF64 : FMT);
     static constexpr bool OK = (FMT != FMT_RUNTIME) && SWB <= 8 && T <= P && T >= 8;
     static constexpr int XP = T + 2;                                             // exchange row pitch (float2): LDS.128 of 8 lanes conflict-free
@@ -72,24 +59,17 @@ template <int LOG2P, int LOG2T, int FMT> struct WCfg {
     static_assert(RAWP % 16 == 0, "raw slots are bulk-copy destinations");
     static constexpr int FPITCH = (HF + 31) / 32 * 32 + FW;                      // staging words per word column: STS.32 of a warp conflict-free
     static constexpr int HALF_WORDS = (N / 4) * FPITCH;
-    static constexpr bool TW_SMEM = P > 16 && !SP_W_TWREG32;                     // twiddles from shared memory (31 per thread do not fit 152 registers)
     // The bulk copy, its position arithmetic (double) and its barrier serve TWO consecutive warp-steps = 2 FW consecutive frames wherever
     // the doubled raw area still fits shared memory (every shape for samples of up to 4 bytes): ncu put 22 % of the FFT warps' time of
     // the N = 128 kernel, and 11 % at N = 512, into that per-step bookkeeping
-    static constexpr size_t SMEM_REST = (size_t)2 * HALF_WORDS * 4 + (size_t)JH_SIZE * 4 + (TW_SMEM ? (size_t)T * 32 * 8 : 0) + 1024 /* LUT */
+    static constexpr size_t SMEM_REST = (size_t)2 * HALF_WORDS * 4 + (size_t)JH_SIZE * 4 + 1024 /* LUT */
                                       + (size_t)F * 8 /* s_mm */ + (size_t)NW * 8 + 64 + 128 + 1024 /* LUT alignment */;
     static constexpr size_t SMEM_SG2 = (size_t)NW * (((2 * FW * RAWP + 15) & ~15) + ((FW * FSTR * 8 + 15) & ~15)) + (size_t)NW * 2 * 2 * FW * 4 + SMEM_REST;
-    static constexpr int SG = (SP_W_SG && SP_W_SEP && T <= SP_W_SG_MAXT && WSH % 2 == 0 && SMEM_SG2 <= 232448) ? 2 : 1, FWS = FW * SG;
-#if SP_W_SEP
+    static constexpr int SG = (WSH % 2 == 0 && SMEM_SG2 <= 232448) ? 2 : 1, FWS = FW * SG;
     // the raw frames and the exchange area of a warp do not share bytes: the exchange stores need no "raw frame consumed" fence (they
     // ride between the twiddle products) and the next frames' bulk copy starts as soon as the warp has decoded, not after pass B
     static constexpr int RAW_BYTES = (FWS * RAWP + 15) & ~15;
     static constexpr int XBYTES = RAW_BYTES + ((FW * FSTR * 8 + 15) & ~15);
-    static constexpr bool STS_BETWEEN = SP_W_STSB != 0;
-#else
-    static constexpr int RAW_BYTES = 0;
-    static constexpr int XBYTES = ((FW * FSTR * 8 > FW * RAWP ? FW * FSTR * 8 : FW * RAWP) + 15) & ~15;
-#endif
     static constexpr size_t SMEM_BYTES = (size_t)NW * XBYTES + (size_t)NW * 2 * FWS * 4 /* s_off */ + SMEM_REST;
 };
 
@@ -131,8 +111,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
     unsigned *s_lut = reinterpret_cast<unsigned *>(s_x - 1024);                  // [256] RGBA indexed by the staged byte
     unsigned *s_stage = reinterpret_cast<unsigned *>(s_x + NW * B::XBYTES);      // [2][N/4][FPITCH] colour bytes: word column x frame
     unsigned *s_jh = s_stage + 2 * B::HALF_WORDS;                                // [JH_SIZE] joint histogram
-    float2 *s_tw = reinterpret_cast<float2 *>(s_jh + JH_SIZE);                   // [T][32] (P = 32 only; row t rotated by 2t entries: LDS.128 conflict-free)
-    uint2 *s_mm = reinterpret_cast<uint2 *>(s_tw + (B::TW_SMEM ? T * 32 : 0));   // [F] per-frame min/max bit patterns of |X|^2
+    uint2 *s_mm = reinterpret_cast<uint2 *>(s_jh + JH_SIZE);                     // [F] per-frame min/max bit patterns of |X|^2
     uint64_t *s_mbar = reinterpret_cast<uint64_t *>(s_mm + F);                   // [NW] raw frames landed
     uint64_t *s_full = s_mbar + NW;                                              // [2] staging half holds HF finished frames
     uint64_t *s_empty = s_full + 2;                                              // [2] staging half has been stored
@@ -145,12 +124,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
     float2 *X = reinterpret_cast<float2 *>(xs + B::RAW_BYTES) + f * B::FSTR;     // this frame's exchange area
     uint64_t *mbar = s_mbar + (warp < NW ? warp : 0);
 
-    for (int i = tid; i < JH_SIZE; i += B::THREADS) s_jh[i] = 0;
-    const int cmax = p.cmap_len - 1;
-    const JhConst jc = jh_const(p);
-    for (int i = tid; i < 256; i += B::THREADS) s_lut[i] = i <= cmax ? p.lut[jc.rev ? cmax - i : i] : 0u;
-    if constexpr (B::TW_SMEM)
-        for (int i = tid; i < T * P; i += B::THREADS) { const int tt = i % T, k = i / T; s_tw[tt * 32 + ((k + 2 * tt) & 31)] = twW[i]; }
+    const JhConst jc = fused_prologue(p, s_jh, s_lut, tid, B::THREADS);
     const unsigned jh_base = smem_u32(s_jh) - (JH_MAGIC_BITS << 2);
     const int nfull = p.n_full;
 
@@ -271,8 +245,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                         const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0 + 8 * g;   // :117
                         uint4 a, b;
-                        a.x = lut_at(lut_base, w[0], j); a.y = lut_at(lut_base, w[1], j); a.z = lut_at(lut_base, w[2], j); a.w = lut_at(lut_base, w[3], j);
-                        b.x = lut_at(lut_base, w[4], j); b.y = lut_at(lut_base, w[5], j); b.z = lut_at(lut_base, w[6], j); b.w = lut_at(lut_base, w[7], j);
+                        lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
                     }
                 }
@@ -281,8 +254,9 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                     if (xr0 + HF * h + fl >= p.chunk_frames) break;
                     const long long xl = p.chunk_first + xr0 + HF * h + fl;
                     const uint2 mm = s_mm[HF * h + fl];
-                    p.fmin[xl] = fminf(0.0f, fmaf(fast_log2(__uint_as_float(mm.x)), p.c1, p.c0));        // lib/worker.js:82,102
-                    p.fmax[xl] = fmaxf(-200.0f, fmaf(fast_log2(__uint_as_float(mm.y)), p.c1, p.c0));     // lib/worker.js:83,103
+                    const float2 db = frame_db(mm.x, mm.y, p);
+                    p.fmin[xl] = db.x;
+                    p.fmax[xl] = db.y;
                 }
                 __syncwarp();                                   // this warp is done reading the half (and s_mm)
                 if ((ht & 31) == 0) mbar_arrive(s_empty + h);
@@ -296,11 +270,9 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
     float win[P];
 #pragma unroll
     for (int a = 0; a < P; a++) win[a] = p.window[t + T * a];
-    float2 tw[B::TW_SMEM ? 1 : P];
-    if constexpr (!B::TW_SMEM) {
+    float2 tw[P];
 #pragma unroll
-        for (int k = 1; k < P; k++) tw[k] = twW[k * T + t];
-    }
+    for (int k = 1; k < P; k++) tw[k] = twW[k * T + t];
     // frames of warp-step (h, j) of a tile: h*HF + ((j/SG)*NW + warp)*FWS + (j%SG)*FW .. + FW - 1 (a warp's SG consecutive steps = FWS consecutive frames)
     auto step_first = [&](long long tl, int h, int j) -> long long { return tl * F + h * HF + ((j / SG) * NW + warp) * FWS + (j % SG) * FW; };
     if (tile < p.ntiles) stage(step_first(tile, 0, 0), 0);
@@ -333,48 +305,15 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
 
             // ---------------- pass A: DFT-P over the slow input digit, twiddle W_N^{t*k0} ----------------
             dft<P>(v);
-            if constexpr (B::TW_SMEM) {
-                const float4 *twp = reinterpret_cast<const float4 *>(s_tw + t * 32);
+            cst(X + t, v[0]);
 #pragma unroll
-                for (int i = 0; i < P / 2; i++) {
-                    const float4 w4 = twp[(i + t) & 15];                 // W^{t*2i}, W^{t*(2i+1)}
-                    if (i > 0) v[2 * i] = cmul(v[2 * i], make_float2(w4.x, w4.y));
-                    v[2 * i + 1] = cmul(v[2 * i + 1], make_float2(w4.z, w4.w));
-                }
-#if SP_W_SEP
-#pragma unroll
-                for (int k = 0; k < P; k++) cst(X + k * B::XP + t, v[k]);
-#endif
-            } else {
-#if SP_W_SEP
-                if constexpr (B::STS_BETWEEN) {
-                    cst(X + t, v[0]);
-#pragma unroll
-                    for (int k = 1; k < P; k++) { v[k] = cmul(v[k], tw[k]); cst(X + k * B::XP + t, v[k]); }   // Z[k0][t], between the products
-                } else {
-#pragma unroll
-                    for (int k = 1; k < P; k++) v[k] = cmul(v[k], tw[k]);
-#pragma unroll
-                    for (int k = 0; k < P; k++) cst(X + k * B::XP + t, v[k]);
-                }
-#else
-#pragma unroll
-                for (int k = 1; k < P; k++) v[k] = cmul(v[k], tw[k]);
-#endif
-            }
-#if !SP_W_SEP
-            __syncwarp();                                               // every lane has consumed its raw frame
-#pragma unroll
-            for (int k = 0; k < P; k++) cst(X + k * B::XP + t, v[k]);   // Z[k0][t]
-#endif
+            for (int k = 1; k < P; k++) { v[k] = cmul(v[k], tw[k]); cst(X + k * B::XP + t, v[k]); }   // Z[k0][t], between the products
             __syncwarp();                                               // the rows are complete (and every lane has decoded its raw frame)
             auto prefetch = [&]() {
                 if (hj + 1 < 2 * B::WSH) stage(step_first(tile, (hj + 1) / B::WSH, (hj + 1) % B::WSH), fpar);
                 else if (next_tile < p.ntiles) stage(step_first(next_tile, 0, 0), fpar);
             };
-#if SP_W_SEP
             if (r == SG - 1) prefetch();                                // the raw area is free: start the bulk copy of the warp's next frames
-#endif
             // ---------------- pass B: thread u = t owns rows k0 = u + T*q: Q transforms of length T ----------------
 #pragma unroll
             for (int q = 0; q < Q; q++) {
@@ -387,9 +326,6 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
             }
             __syncwarp();                                               // the exchange area is free (next step's stores, split-real below)
             const bool split = OPT && p.channel_mode;
-#if !SP_W_SEP
-            if (!split) prefetch();                                     // shared bytes: split-real needs the buffer once more, see below
-#endif
             if (j == 0) mbar_wait(s_empty + h, (kk + 1) & 1);           // the store warps are done with this staging half (previous tile)
 #pragma unroll
             for (int q = 0; q < Q; q++) {
@@ -424,80 +360,22 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                         v[r] = nv;
                     }
                     __syncwarp();                                       // now the buffer is free
-#if !SP_W_SEP
-                    prefetch();
-#endif
                 }
             }
 
             // ---------------- per-bin epilogue (lib/worker.js:85-122) ----------------
-            float amin = __int_as_float(0x7f800000), amax = 0.0f, prev = 0.0f;
-            unsigned umin_i = 0x7f800000u, umax_i = 0u;
+            BinMinMax<FLOAT_IN> bm;
             unsigned *stg = s_stage + h * B::HALF_WORDS + t * B::FPITCH + fh;
 #pragma unroll
             for (int q = 0; q < Q; q++)
 #pragma unroll
-                for (int m = 0; m < T / 4; m++) {
-                    unsigned yb[4];
-#pragma unroll
-                    for (int jj = 0; jj < 4; jj++) {
-                        const float2 vi = cun(v[q * T + 4 * m + jj]);
-                        const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                        if constexpr (FLOAT_IN) {
-                            umin_i = min(umin_i, __float_as_uint(abs2));
-                            umax_i = max(umax_i, __float_as_uint(abs2));
-                        } else if (jj & 1) {
-                            amin = fmin3(amin, prev, abs2);
-                            amax = fmax3(amax, prev, abs2);
-                        } else prev = abs2;
-                        const float l2 = fast_log2(abs2);
-                        float Y;
-                        const float S = jh_eval(l2, jc, Y);
-                        red_shared_inc_addr(valid ? jh_base + (__float_as_uint(S) << 2) : dump);
-                        yb[jj] = __float_as_uint(Y);
-                    }
-                    // bins (t + T*q) + P*(4m .. 4m+3): four colour bytes in one word of column (q*(T/4) + m)*T + t
-                    stg[((q * (T / 4) + m) * T) * B::FPITCH] = __byte_perm(__byte_perm(yb[0], yb[1], 0x0040), __byte_perm(yb[2], yb[3], 0x0040), 0x5410);
-                }
-            unsigned umn, umx;
-            if constexpr (FLOAT_IN) {
-                umn = group_min<T>(umin_i);
-                umx = group_max<T>(umax_i);
-            } else {
-                umn = group_min<T>(__float_as_uint(amin));
-                umx = group_max<T>(__float_as_uint(amax));
-            }
-            if (__any_sync(0xffffffffu, umn < 0x00800000u || umx >= 0x7f800000u)) {
-                // rare (warp-uniform): a frame of this warp holds |X|^2 == 0 (flushed), +inf or NaN: see render_r64_kernel
-                unsigned nzero = 0, nbad = 0, nnan = 0;
-                float mn = __int_as_float(0x7f800000), mx = 0.0f;
-#pragma unroll
-                for (int i = 0; i < P; i++) {
-                    const float2 vi = cun(v[i]);
-                    const float abs2 = fmaf(vi.x, vi.x, vi.y * vi.y);
-                    nzero += abs2 < 1.17549435e-38f ? 1u : 0u;
-                    nbad += !(abs2 <= 3.402823466e38f) ? 1u : 0u;
-                    nnan += abs2 != abs2 ? 1u : 0u;
-                    mn = fminf(mn, abs2 < 1.17549435e-38f ? 0.0f : abs2);
-                    mx = fmaxf(mx, abs2);
-                }
-                if (!valid) nzero = nbad = nnan = 0;
-                nzero = __reduce_add_sync(0xffffffffu, nzero);
-                nbad = __reduce_add_sync(0xffffffffu, nbad);
-                nnan = __reduce_add_sync(0xffffffffu, nnan);
-                umn = group_min<T>(__float_as_uint(mn));
-                umx = group_max<T>(__float_as_uint(mx));
-                if (lane == 0) {
-                    if (nzero) atomicAdd(&s_jh[JH_ZERO], nzero);
-                    if (nbad) atomicAdd(&s_jh[JH_BAD], nbad);
-                    if (nnan) {
-                        float Yn;
-                        const float Sn = jh_eval(__int_as_float(0x7fffffff), jc, Yn);
-                        atomicSub(&s_jh[__float_as_uint(Sn) - JH_MAGIC_BITS], nnan);
-                        atomicAdd(&s_jh[JH_NAN], nnan);
-                    }
-                }
-            }
+                for (int m = 0; m < T / 4; m++)     // bins (t + T*q) + P*(4m .. 4m+3): four colour bytes in one word of column (q*(T/4) + m)*T + t
+                    stg[((q * (T / 4) + m) * T) * B::FPITCH] = epilogue4(v + q * T + 4 * m, bm, jc, jh_base, valid, dump);
+            auto gmin = [](unsigned x) { return group_min<T>(x); };
+            auto gmax = [](unsigned x) { return group_max<T>(x); };
+            unsigned umn = gmin(bm.lo()), umx = gmax(bm.hi());
+            if (__any_sync(0xffffffffu, umn < 0x00800000u || umx >= 0x7f800000u))   // rare (warp-uniform)
+                fixup_nonfinite(v, valid, lane == 0, true, s_jh, jc, gmin, gmax, umn, umx);
             if (t == 0) s_mm[h * HF + fh] = make_uint2(umn, umx);
             if (j == B::WSH - 1) {          // this warp has staged its last frames of the half (and their s_mm entries)
                 __syncwarp();
@@ -510,8 +388,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
     } // FFT warps
 
     __syncthreads();
-    for (int i = tid; i < JH_SIZE; i += B::THREADS)
-        if (s_jh[i]) atomicAdd(&p.j_hist[i], (unsigned long long)s_jh[i]);
+    flush_joint_hist(p, s_jh, tid, B::THREADS);
 }
 
 } // namespace sp

@@ -118,6 +118,9 @@ struct DevBuf {
 // where a shard's image goes inside the caller's [n][total width] picture (multi-device engines; spectrogram layout)
 struct Placement { long long pitch_frames; long long col0; };
 
+// kinds of twiddle table (get_table)
+enum class Tw { full, big, passA, passB, tw14, w };
+
 struct sp_engine {
     std::vector<sp_engine *> subs;           // ndev > 1: one single-device engine per GPU; this object only dispatches
     std::vector<sp_ncclComm_t> comms;        // ndev > 1: one NCCL communicator per device (ncclCommInitAll), empty when NCCL is unavailable
@@ -130,7 +133,7 @@ struct sp_engine {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string err;
     std::string plan;
-    std::map<int, float2 *> tw, twA, twB;    // twiddle tables by n (full / pass A / pass B)
+    std::map<std::pair<Tw, int>, float2 *> tw;   // twiddle tables by (kind, n)
     DevBuf pin[2], pimg[2];                  // pipeline: double-buffered input bytes / image tiles
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_in[2] = { nullptr, nullptr }, ev_comp[2] = { nullptr, nullptr }, ev_out[2] = { nullptr, nullptr }, ev_setup = nullptr;
@@ -147,11 +150,11 @@ struct sp_engine {
     bool prof_this = false;
     std::vector<float> h_window, h_window_t; // last uploaded window / LUT (upload only on change)
     std::vector<uint32_t> h_lut;
-    double *stats_src = nullptr;
+    double *stats_src = nullptr;             // dBfs min / max of the last prepared render (set by prepare)
     // sp_render_async: up to two host-buffer messages in flight (the copy-out tail of one overlaps the copy-in head of the next)
     struct Inflight {
         cudaEvent_t done = nullptr, reply = nullptr;
-        uint8_t *bounce = nullptr;           // pinned: [16 stats][W mins][W maxs][W amps][8 * 1000 cB][8 * cmap_len c]
+        uint8_t *bounce = nullptr;           // pinned: stats and the five small reply arrays (layout: Bounce)
         size_t bounce_cap = 0;
         sp_reply *rp = nullptr;
         long long width = 0;
@@ -302,8 +305,6 @@ extern "C" void sp_destroy(sp_engine *e)
     cudaSetDevice(e->dev);
     cudaDeviceSynchronize();
     for (auto &kv : e->tw) cudaFree(kv.second);
-    for (auto &kv : e->twA) cudaFree(kv.second);
-    for (auto &kv : e->twB) cudaFree(kv.second);
     DevBuf *bufs[] = { &e->in, &e->zin, &e->spec, &e->image, &e->fmin, &e->fmax, &e->fmid, &e->gauges, &e->hist, &e->jhist, &e->stats, &e->mm,
                        &e->lut, &e->window, &e->window_t, &e->acc, &e->jhtab, &e->ring, &e->ringctl, &e->scratch, &e->db, &e->synth_lut, &e->pin[0], &e->pin[1],
                        &e->pimg[0], &e->pimg[1], &e->tilectr, &e->tstamp };
@@ -354,13 +355,36 @@ static int ilog2_exact(int n)
     return -1;
 }
 
-static int upload_table(sp_engine *e, std::map<int, float2 *> &cache, int key, const std::vector<float2> &h, const float2 **out)
+// first sample of global frame x (lib/worker.js:72)
+static long long frame_pos(double stride, long long x) { return (long long)(0.5 + stride * (double)x); }
+
+// The samples that global frames [x0, x0 + count) read, as a piece of a buffer that starts at sample buf_first and holds
+// byte_length bytes: sample s0 and bytes [b0, b1) of the buffer.  The start is rounded down to 16 samples (any format's byte
+// offset stays 16-byte aligned), the end is the last frame's start + n.  The piece takes the samples its frames read and nothing
+// more: a shard's buffer may extend past its frames (a caller may pass the whole capture with a frame sub-range).  The ragged tail
+// (< 1 sample, or whatever lies between the last frame and the end of the capture) travels only with the piece that holds the
+// message's last frame (msg_last).
+struct Span { long long s0; unsigned long long b0, b1; };
+static Span frame_span(double stride, int n, int sw, long long x0, long long count, long long buf_first, unsigned long long byte_length,
+                       bool msg_last)
+{
+    long long s0 = frame_pos(stride, x0);
+    const long long s1 = frame_pos(stride, x0 + count - 1) + n;
+    s0 -= s0 % 16;
+    if (s0 < buf_first) s0 = buf_first;
+    unsigned long long b0 = (unsigned long long)(s0 - buf_first) * sw, b1 = (unsigned long long)(s1 - buf_first) * sw;
+    if (b1 > byte_length || msg_last) b1 = byte_length;
+    if (b0 > b1) b0 = b1;
+    return { s0, b0, b1 };
+}
+
+static int upload_table(sp_engine *e, std::pair<Tw, int> key, const std::vector<float2> &h, const float2 **out)
 {
     float2 *d = nullptr;
     CU(cudaMalloc(&d, sizeof(float2) * h.size()));
     CU(cudaMemcpyAsync(d, h.data(), sizeof(float2) * h.size(), cudaMemcpyHostToDevice, e->stream));
     CU(cudaStreamSynchronize(e->stream));
-    cache[key] = d;
+    e->tw[key] = d;
     *out = d;
     return SP_OK;
 }
@@ -369,74 +393,65 @@ static inline float2 twid(long long num, long long den)   // exp(-2 pi j num / d
     const double a = 2.0 * M_PI * (double)(num % den) / (double)den;
     return make_float2((float)cos(a), (float)-sin(a));
 }
-// full table W_n^i (pre-pass of the four-step sizes)
-static int get_twiddles(sp_engine *e, int n, const float2 **out)
+// The table of one kind for size n, built and uploaded on first use:
+//   full   [n]          W_n^i                                   pre-pass of the four-step sizes
+//   big    [R-1][4096]  W_n^{j*k}, k = 1 .. R-1, j fastest      pre-pass of render_big_kernel, n = R * 4096 (coalesced loads)
+//   passA  [15][n/16]   W_n^{t*k}, k = 1 .. 15                  render_kernel, n >= 32
+//   passB  [15][n/256]  W_{n/16}^{b*k}, k = 1 .. 15             render_kernel, n >= 512
+//   tw14   [n/64][14]   W_n^{t*k}, k = 1 .. 7, 8, 16, .., 56    render_r64_kernel (n = 4096), render_rc_kernel (n = 2048)
+//   w      [P][n/P]     W_n^{t*k}, k = 0 .. P-1                 render_w_kernel (P from w_log2p)
+static int get_table(sp_engine *e, Tw kind, int n, const float2 **out)
 {
-    auto it = e->tw.find(n);
+    auto it = e->tw.find({ kind, n });
     if (it != e->tw.end()) { *out = it->second; return SP_OK; }
-    std::vector<float2> h((size_t)n);
-    for (int i = 0; i < n; i++) h[i] = twid(i, n);
-    return upload_table(e, e->tw, n, h, out);
+    std::vector<float2> h;
+    switch (kind) {
+    case Tw::full:
+        h.resize((size_t)n);
+        for (int i = 0; i < n; i++) h[i] = twid(i, n);
+        break;
+    case Tw::big: {
+        const int R = n / 4096;
+        h.resize((size_t)(R - 1) * 4096);
+        for (int k = 1; k < R; k++) for (int j = 0; j < 4096; j++) h[(size_t)(k - 1) * 4096 + j] = twid((long long)j * k, n);
+        break;
+    }
+    case Tw::passA: {
+        const int T = n / 16;
+        h.resize((size_t)15 * T);
+        for (int k = 1; k < 16; k++) for (int t = 0; t < T; t++) h[(size_t)(k - 1) * T + t] = twid((long long)t * k, n);
+        break;
+    }
+    case Tw::passB: {
+        const int RL = n / 256, N1 = n / 16;
+        h.resize((size_t)15 * RL);
+        for (int k = 1; k < 16; k++) for (int b = 0; b < RL; b++) h[(size_t)(k - 1) * RL + b] = twid((long long)b * k, N1);
+        break;
+    }
+    case Tw::tw14: {
+        static const int ks[14] = { 1, 2, 3, 4, 5, 6, 7, 8, 16, 24, 32, 40, 48, 56 };
+        const int c = n / 64;
+        h.resize((size_t)c * 14);
+        for (int t = 0; t < c; t++) for (int i = 0; i < 14; i++) h[(size_t)t * 14 + i] = twid((long long)t * ks[i], n);
+        break;
+    }
+    case Tw::w: {
+        const int P = 1 << sp::w_log2p(ilog2_exact(n)), T = n / P;
+        h.resize((size_t)n);
+        for (int k = 0; k < P; k++) for (int t = 0; t < T; t++) h[(size_t)k * T + t] = twid((long long)t * k, n);
+        break;
+    }
+    }
+    return upload_table(e, { kind, n }, h, out);
 }
-// pre-pass twiddles of render_big_kernel: [R - 1][4096] = W_n^{j*k}, k = 1 .. R-1, j fastest (coalesced loads)
-static int get_big_twiddles(sp_engine *e, int n, const float2 **out)
-{
-    auto it = e->tw.find(-n);
-    if (it != e->tw.end()) { *out = it->second; return SP_OK; }
-    const int R = n / 4096;
-    std::vector<float2> h((size_t)(R - 1) * 4096);
-    for (int k = 1; k < R; k++) for (int j = 0; j < 4096; j++) h[(size_t)(k - 1) * 4096 + j] = twid((long long)j * k, n);
-    return upload_table(e, e->tw, -n, h, out);
-}
-// pass-A table [15][T]: W_N^{t*k}; pass-B table [15][RL]: W_{N/16}^{b*k}  (k = 1..15)
+// render_kernel's pass tables; null for the sizes that need none
 static int get_pass_tables(sp_engine *e, int log2k, const float2 **twA, const float2 **twB)
 {
-    const int N = 1 << log2k;
     *twA = *twB = nullptr;
-    if (log2k <= 4) return SP_OK;                        // single-pass sizes need no twiddles
-    const int T = N / 16;
-    auto it = e->twA.find(N);
-    if (it != e->twA.end()) *twA = it->second;
-    else {
-        std::vector<float2> h((size_t)15 * T);
-        for (int k = 1; k < 16; k++) for (int t = 0; t < T; t++) h[(size_t)(k - 1) * T + t] = twid((long long)t * k, N);
-        int rc = upload_table(e, e->twA, N, h, twA);
-        if (rc) return rc;
-    }
-    if (log2k <= 8) return SP_OK;
-    const int RL = N / 256, N1 = N / 16;
-    auto ib = e->twB.find(N);
-    if (ib != e->twB.end()) *twB = ib->second;
-    else {
-        std::vector<float2> h((size_t)15 * RL);
-        for (int k = 1; k < 16; k++) for (int b = 0; b < RL; b++) h[(size_t)(k - 1) * RL + b] = twid((long long)b * k, N1);
-        int rc = upload_table(e, e->twB, N, h, twB);
-        if (rc) return rc;
-    }
-    return SP_OK;
-}
-
-// 64 x 64 path table: tw14 [64][14] = W_4096^{t*k}, k = 1..7, 8, 16, .., 56
-static int get_r64_table(sp_engine *e, const float2 **tw14)
-{
-    static const int ks[14] = { 1, 2, 3, 4, 5, 6, 7, 8, 16, 24, 32, 40, 48, 56 };
-    auto it = e->twA.find(-64);
-    if (it != e->twA.end()) { *tw14 = it->second; return SP_OK; }
-    std::vector<float2> h((size_t)64 * 14);
-    for (int t = 0; t < 64; t++) for (int i = 0; i < 14; i++) h[(size_t)t * 14 + i] = twid((long long)t * ks[i], 4096);
-    return upload_table(e, e->twA, -64, h, tw14);
-}
-
-// 64 x C path table (N = 512, 1024, 2048): tw14 [C][14] = W_N^{t*k}, k = 1..7, 8, 16, .., 56
-static int get_rc_table(sp_engine *e, int n, const float2 **tw14)
-{
-    static const int ks[14] = { 1, 2, 3, 4, 5, 6, 7, 8, 16, 24, 32, 40, 48, 56 };
-    auto it = e->twA.find(-100000 - n);
-    if (it != e->twA.end()) { *tw14 = it->second; return SP_OK; }
-    const int c = n / 64;
-    std::vector<float2> h((size_t)c * 14);
-    for (int t = 0; t < c; t++) for (int i = 0; i < 14; i++) h[(size_t)t * 14 + i] = twid((long long)t * ks[i], n);
-    return upload_table(e, e->twA, -100000 - n, h, tw14);
+    int rc = SP_OK;
+    if (log2k > 4) rc = get_table(e, Tw::passA, 1 << log2k, twA);
+    if (!rc && log2k > 8) rc = get_table(e, Tw::passB, 1 << log2k, twB);
+    return rc;
 }
 
 struct Plan {
@@ -589,8 +604,8 @@ static int validate(sp_engine *e, const sp_request *rq, bool shard, double *samp
             return fail(e, SP_E_RANGE, "frame range [%lld, %lld) outside total width %lld", (long long)rq->frame_first,
                         (long long)(rq->frame_first + rq->width), (long long)total_width);
         // the shard buffer must cover every sample its frames read
-        const long long p_first = (long long)(0.5 + *stride * (double)rq->frame_first);
-        const long long p_last = (long long)(0.5 + *stride * (double)(rq->frame_first + rq->width - 1)) + rq->n;
+        const long long p_first = frame_pos(*stride, rq->frame_first);
+        const long long p_last = frame_pos(*stride, rq->frame_first + rq->width - 1) + rq->n;
         const long long have_first = (long long)rq->buffer_first_sample;
         const double have_last = (double)have_first + (double)rq->byte_length / sp::sample_width(rq->format);
         if (p_first < have_first || ((double)p_last > have_last && (double)p_last <= sc))
@@ -803,8 +818,7 @@ static long long frames_inside(const Params &q, int len)
 {
     const long long sw = sp::sample_width(q.format);
     auto inside = [&](long long xr) {
-        const long long xgl = q.frame_first + q.chunk_first + xr;
-        const long long p0 = (long long)(0.5 + q.stride * (double)xgl) - q.sample_base;       // lib/worker.js:72
+        const long long p0 = frame_pos(q.stride, q.frame_first + q.chunk_first + xr) - q.sample_base;
         return p0 >= 0 && (unsigned long long)(p0 + len) * (unsigned long long)sw <= q.valid_bytes;
     };
     long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (a multiple of 8 frames)
@@ -847,7 +861,7 @@ static int launch_r64_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
     const long long nf = sub ? q.chunk_frames / 8 * 8 : frames_inside(q, 4096);   // the last tile may be partial (8 of 16 frames)
     if (nf == 0) return SP_OK;
     const float2 *tw14 = nullptr;
-    int rc = get_r64_table(e, &tw14);
+    int rc = get_table(e, Tw::tw14, 4096, &tw14);
     if (rc) return rc;
     CUtensorMap tm;
     memset(&tm, 0, sizeof tm);
@@ -896,7 +910,7 @@ static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
         if (L > S) L = S;
         if (L < 1) L = 1;
         const float2 *twT = nullptr;
-        if ((rc = get_r64_table(e, &tw14)) || (rc = get_big_twiddles(e, n, &twT))) return rc;
+        if ((rc = get_table(e, Tw::tw14, 4096, &tw14)) || (rc = get_table(e, Tw::big, n, &twT))) return rc;
         if ((rc = ensure(e, e->ring, (size_t)S * block_bytes)) || (rc = ensure(e, e->ringctl, 4 * (size_t)(1 + 2 * 64) + 64 + 64))) return rc;
         if (e->l2_window != (size_t)S * block_bytes && !getenv("SP_BIG_NO_L2PIN")) {
             // keep the ring in L2: persisting lines for the ring's address range, everything else streams through the rest
@@ -944,24 +958,14 @@ static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
     return launch_fused(e, q, nf, e->sm_count, 2, nfast, launch, setup);
 }
 
-// render_w_kernel table: [P][T] = W_N^{t*k}, k = 0 .. P-1 (N = P * T)
-static int get_w_table(sp_engine *e, int n, int P, const float2 **out)
-{
-    auto it = e->twA.find(-200000 - n);
-    if (it != e->twA.end()) { *out = it->second; return SP_OK; }
-    const int T = n / P;
-    std::vector<float2> h((size_t)n);
-    for (int k = 0; k < P; k++) for (int t = 0; t < T; t++) h[(size_t)k * T + t] = twid((long long)t * k, n);
-    return upload_table(e, e->twA, -200000 - n, h, out);
-}
 // render_w_kernel: N = 64 .. 1024
 static int launch_w_kernel(sp_engine *e, const sp::Kernels &k, int log2n, const Params &q, long long *nfast)
 {
-    const int n = 1 << log2n, P = 1 << sp::w_log2p(log2n), tile = sp::w_tile_frames(log2n);
+    const int n = 1 << log2n, tile = sp::w_tile_frames(log2n);
     const long long nf = frames_inside(q, n);
     if (nf == 0) return SP_OK;
     const float2 *twW = nullptr;
-    const int rc = get_w_table(e, n, P, &twW);
+    const int rc = get_table(e, Tw::w, n, &twW);
     if (rc) return rc;
     return launch_fused(e, q, nf, (nf + tile - 1) / tile, 1, nfast,
                         [&](const Params &r, int grid, int *occ) { return k.w(log2n, &r, grid, e->stream, twW, occ); }, no_setup);
@@ -974,10 +978,27 @@ static int launch_rc_kernel(sp_engine *e, const sp::Kernels &k, int log2n, const
     const long long nf = frames_inside(q, n);
     if (nf == 0) return SP_OK;
     const float2 *tw14 = nullptr;
-    const int rc = get_rc_table(e, n, &tw14);
+    const int rc = get_table(e, Tw::tw14, n, &tw14);
     if (rc) return rc;
     return launch_fused(e, q, nf, (nf + tile - 1) / tile, 1, nfast,
                         [&](const Params &r, int grid, int *occ) { return k.rc(log2n, &r, grid, e->stream, tw14, occ); }, no_setup);
+}
+
+// render_kernel (in sub-frame mode for n > 4096) over every frame of the chunk q, in one slot of the profiling ring.  It is the
+// kernel that takes what the fused kernels leave, so unlike launch_fused a kernel that does not fit an SM is an error.
+static int launch_render_kernel(sp_engine *e, const sp::Kernels &k, const Plan &pl, Params q)
+{
+    const size_t smem = sp::main_smem_bytes(pl.smem_x, q.cmap_len, pl.log2k > 8 ? 15 * ((1 << pl.log2k) / 256) : 0);
+    int occ = 0;
+    CU(k.render(pl.log2k, &q, 0, smem, e->stream, &occ));
+    if (occ < 1) return fail(e, SP_E_CUDA, "render kernel does not fit an SM (smem %zu)", smem);
+    q.ntiles = (q.chunk_frames + pl.tile - 1) / pl.tile * pl.sub_r;
+    const long long cap = (long long)e->sm_count * occ;
+    prof_begin(e);
+    CU(k.render(pl.log2k, &q, (int)(q.ntiles < cap ? q.ntiles : cap), smem, e->stream, nullptr));
+    prof_end(e);
+    e->launches++;
+    return SP_OK;
 }
 
 // Enqueue all kernels of a job on e->stream (bracketed by the timing events).
@@ -1016,8 +1037,6 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
     const int fmt = p.format;
     const sp::Kernels &k = kernels_for(fmt);
     const Route fused = route(j.plan, fmt, p);
-    const size_t smem = sp::main_smem_bytes(j.plan.smem_x, p.cmap_len, j.plan.log2k > 8 ? 15 * ((1 << j.plan.log2k) / 256) : 0);
-    int occ = 0;
     if (j.plan.sub_r == 1) {
         Params q = p;
         long long nfast = 0;
@@ -1034,44 +1053,29 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         }
         if (q.chunk_frames > 0) {
             if (!k.render) return fail(e, SP_E_CUDA, "no render kernel linked for format %d", fmt);
-            CU(k.render(j.plan.log2k, &q, 0, smem, e->stream, &occ));
-            if (occ < 1) return fail(e, SP_E_CUDA, "render kernel does not fit an SM (smem %zu)", smem);
-            q.ntiles = (q.chunk_frames + j.plan.tile - 1) / j.plan.tile;
-            const long long cap = (long long)e->sm_count * occ;
-            const int grid = (int)(q.ntiles < cap ? q.ntiles : cap);
-            prof_begin(e);
-            CU(k.render(j.plan.log2k, &q, grid, smem, e->stream, nullptr));
-            prof_end(e);
-            e->launches++;
+            if ((rc = launch_render_kernel(e, k, j.plan, q))) return rc;
         }
     } else {
-        // four-step path for n > 4096: radix-R pre-pass into an L2-sized scratch, then the
+        // four-step path for n > 4096: radix-R pre-pass into a scratch, then the
         // 4096-point kernel in sub-frame mode, chunk by chunk
         const int R = j.plan.sub_r;
         const int n = p.n_full;
         const sp::Kernels &sub = kernels_for(SP_CF32);        // sub-frame input is always complex fp32
         if (!sub.render || !k.prepass) return fail(e, SP_E_CUDA, "no kernels linked for the four-step path");
         const float2 *tw_full = nullptr;
-        int rc = get_twiddles(e, n, &tw_full);
+        int rc = get_table(e, Tw::full, n, &tw_full);
         if (rc) return rc;
-        // frames per chunk: a 1 GB scratch by default.  An L2-sized scratch (<= 96 MB) keeps the 16 B/sample of scratch
-        // traffic out of HBM but leaves each launch with about one wave of tiles; measured on B200 the large chunk wins
-        // (C5: 2.10 -> 1.56 ms, C3 x1: 1.28 -> 0.70 ms, profiles/r01_fourstep_scratch_sweep.txt).  SP_SCRATCH_MB overrides.
-        long long ch = (long long)(((size_t)1024 << 20) / ((size_t)n * 8));
-        if (const char *s = getenv("SP_SCRATCH_MB"))
-            if (atoi(s) > 0) ch = (long long)(((size_t)atoi(s) << 20) / ((size_t)n * 8));
-        ch = ch / 16 * 16;
-        if (ch < 16) ch = 16;
-        ch = ch / 8 * 8;
-        if (ch < 8) ch = 8;
+        // frames per chunk: a 1 GB scratch (2^27 / n frames of n complex floats: a power of two, at least 512).  An L2-sized
+        // scratch (<= 96 MB) keeps the 16 B/sample of scratch traffic out of HBM but leaves each launch with about one wave of
+        // tiles; measured on B200 the large chunk wins (C5: 2.10 -> 1.56 ms, C3 x1: 1.28 -> 0.70 ms,
+        // profiles/r01_fourstep_scratch_sweep.txt).
+        long long ch = (1LL << 27) / n;
         if (ch > p.nframes) ch = (p.nframes + 7) / 8 * 8;
         if ((rc = ensure(e, e->scratch, (size_t)ch * (size_t)n * 8))) return rc;
         // split-real pairs bin k with bin n-k, which live in different sub-sequences: tap the whole spectrum of the
         // chunk and finish it in spectrum_epilogue_kernel
         const bool tap = p.channel_mode != 0;
         if (tap && (rc = ensure(e, e->spec, (size_t)ch * (size_t)n * 8))) return rc;
-        CU(sub.render(12, &p, 0, smem, e->stream, &occ));
-        if (occ < 1) return fail(e, SP_E_CUDA, "render kernel does not fit an SM (smem %zu)", smem);
         const long long nf = p.nframes;
         sp::init_minmax_kernel<<<(unsigned)((nf + 255) / 256), 256, 0, e->stream>>>((unsigned *)p.fmin, (unsigned *)p.fmax, nf);
         e->launches++;
@@ -1104,15 +1108,7 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
                 q.chunk_first += nfast;
                 q.chunk_frames -= nfast;
             }
-            if (q.chunk_frames > 0) {
-                q.ntiles = ((q.chunk_frames + 7) / 8) * R;
-                const long long cap = (long long)e->sm_count * occ;
-                const int grid = (int)(q.ntiles < cap ? q.ntiles : cap);
-                prof_begin(e);
-                CU(sub.render(12, &q, grid, smem, e->stream, nullptr));
-                prof_end(e);
-                e->launches++;
-            }
+            if (q.chunk_frames > 0 && (rc = launch_render_kernel(e, sub, j.plan, q))) return rc;
             if (tap) {
                 const long long tiles = full.chunk_frames * (n / 256);
                 const long long cap = (long long)e->sm_count * 8;
@@ -1169,8 +1165,10 @@ static int finish(sp_engine *e, sp_reply *rp);
 // frame-range shard of the SAME message (global stride, global frame indices), so the result is
 // bit-identical to the single-shot path; histograms accumulate across chunks, min / max / gauges
 // are finalised once.  Host memory should be page-locked (sp_host_alloc_pinned) for real overlap.
+// Frames per chunk of a message that takes this path, 0 for one that does not.
 static long long pipeline_chunk_frames(const sp_request *rq)
 {
+    if ((rq->flags & (SP_F_BUFFER_ON_DEVICE | SP_F_REPLY_ON_DEVICE)) || rq->width <= 0 || rq->n <= 0 || rq->byte_length == 0) return 0;
     const char *env = getenv("SP_PIPE_MB");                  // chunk size in MB; 0 disables the pipeline
     const long long mb = env ? atoll(env) : 16;     // 16 MB: best of 8..128 on B200 + PCIe 5 (profiles/r01_e2e_chunk_sweep.txt)
     if (mb <= 0) return 0;
@@ -1182,6 +1180,27 @@ static long long pipeline_chunk_frames(const sp_request *rq)
     if (ch < 64) ch = 64;
     return (rq->width >= 3 * ch) ? ch : 0;       // short messages: single shot
 }
+
+// Enqueue the copies of job j's five small reply arrays (gauges, histograms) to the non-null arrays of dst, in host memory.
+static int copy_reply(sp_engine *e, const Job &j, const sp_reply &dst)
+{
+    const size_t W = (size_t)j.width;
+    if (dst.gauge_mins) CU(cudaMemcpyAsync(dst.gauge_mins, j.d_gmin, W, cudaMemcpyDeviceToHost, e->stream));
+    if (dst.gauge_maxs) CU(cudaMemcpyAsync(dst.gauge_maxs, j.d_gmax, W, cudaMemcpyDeviceToHost, e->stream));
+    if (dst.gauge_amps) CU(cudaMemcpyAsync(dst.gauge_amps, j.d_gamp, W, cudaMemcpyDeviceToHost, e->stream));
+    if (dst.cB_hist) CU(cudaMemcpyAsync(dst.cB_hist, j.d_cb, 8 * SP_CB_HIST_SIZE, cudaMemcpyDeviceToHost, e->stream));
+    if (dst.c_hist) CU(cudaMemcpyAsync(dst.c_hist, j.d_c, 8 * (size_t)j.p.cmap_len, cudaMemcpyDeviceToHost, e->stream));
+    return SP_OK;
+}
+
+// Byte offsets in sp_render_async's pinned bounce buffer for a message of W frames: [16 stats][W mins][W maxs][W amps], padded to
+// 16 bytes, then [8 * SP_CB_HIST_SIZE cB][8 * cmap_len c], room for SP_MAX_CMAP colours.
+struct Bounce {
+    size_t gmin, gmax, gamp, cb, c, bytes;
+    explicit Bounce(long long W)
+        : gmin(16), gmax(16 + (size_t)W), gamp(16 + 2 * (size_t)W), cb(16 + (3 * (size_t)W + 15) / 16 * 16), c(cb + 8 * SP_CB_HIST_SIZE),
+          bytes(c + 8 * (size_t)SP_MAX_CMAP) {}
+};
 
 static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, long long ch, const Placement *pl,
                             sp_engine::Inflight *slot = nullptr)
@@ -1204,7 +1223,7 @@ static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Jo
     }
     int rc;
     // worst-case chunk input: ch frames at the global stride plus the window-length halo
-    const size_t in_cap = (size_t)(((double)ch * (stride > n ? stride : stride) + 2.0 * n + 64) * sw) + 64;
+    const size_t in_cap = (size_t)(((double)ch * stride + 2.0 * n + 64) * sw) + 64;
     const size_t img_cap = (size_t)4 * (size_t)ch * (size_t)n;
     for (int i = 0; i < 2; i++)
         if ((rc = ensure(e, e->pin[i], in_cap)) || (rc = ensure(e, e->pimg[i], img_cap))) return rc;
@@ -1216,31 +1235,22 @@ static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Jo
     for (long long c = 0; c < nchunks; c++) {
         const int b = (int)(c & 1);
         const long long x0 = c * ch, cw = (W - x0 < ch) ? W - x0 : ch;
-        // samples this chunk reads: [pos(x0), pos(x0 + cw - 1) + n), start rounded down to 16 samples
-        long long s0 = (long long)(0.5 + stride * (double)(g_first + x0));
-        long long s1 = (long long)(0.5 + stride * (double)(g_first + x0 + cw - 1)) + n;
-        s0 -= s0 % 16;
-        if (s0 < buf_first) s0 = buf_first;
-        unsigned long long b0 = (unsigned long long)(s0 - buf_first) * sw, b1 = (unsigned long long)(s1 - buf_first) * sw;
-        // The chunk takes the samples its frames read and nothing more: a shard's buffer may extend past its frames (a caller may
-        // pass the whole capture with a frame sub-range).  The ragged tail (< 1 sample, or whatever lies between the last frame
-        // and the end of the capture) travels only with the chunk that holds the message's last global frame.
         const bool msg_last = c == nchunks - 1 && (!shard || g_first + W == rq->total_width);
-        if (b1 > rq->byte_length || msg_last) b1 = rq->byte_length;
-        if (b0 > b1) b0 = b1;
-        if (b1 - b0 + 16 > in_cap) return fail(e, SP_E_RANGE, "internal: pipeline chunk larger than its buffer");
+        const Span span = frame_span(stride, n, sw, g_first + x0, cw, buf_first, rq->byte_length, msg_last);
+        const size_t bytes = span.b1 - span.b0;
+        if (bytes + 16 > in_cap) return fail(e, SP_E_RANGE, "internal: pipeline chunk larger than its buffer");
         // input buffer b is free once the render of its previous user is done (chunk c-2, or a chunk of the previous message:
         // sp_render_async keeps two messages in flight)
         if (c >= 2 || e->pipe_used[b]) CU(cudaStreamWaitEvent(e->s_h2d, e->ev_comp[b], 0));
-        CU(cudaMemcpyAsync(e->pin[b].p, (const uint8_t *)rq->buffer + b0, b1 - b0, cudaMemcpyHostToDevice, e->s_h2d));
+        CU(cudaMemcpyAsync(e->pin[b].p, (const uint8_t *)rq->buffer + span.b0, bytes, cudaMemcpyHostToDevice, e->s_h2d));
         CU(cudaEventRecord(e->ev_in[b], e->s_h2d));
         // render: needs the input, and image tile b drained by the D2H of chunk c-2
         CU(cudaStreamWaitEvent(e->stream, e->ev_in[b], 0));
         if ((c >= 2 || e->pipe_used[b]) && e->ev_out_valid[b]) CU(cudaStreamWaitEvent(e->stream, e->ev_out[b], 0));
         Params q = j.p;
         q.buf = (const uint8_t *)e->pin[b].p;
-        q.valid_bytes = b1 - b0;
-        q.sample_base = s0;
+        q.valid_bytes = bytes;
+        q.sample_base = span.s0;
         q.frame_first = g_first + x0;
         q.nframes = cw;
         q.chunk_first = 0;
@@ -1267,13 +1277,12 @@ static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Jo
         // asynchronous form: the small reply arrays go through the slot's pinned bounce buffer (the caller's arrays may be pageable,
         // which would make the copies synchronous); the message is complete when they and the last image tiles have arrived
         uint8_t *b = slot->bounce;
-        CU(cudaMemcpyAsync(b, e->stats_src ? (void *)e->stats_src : e->stats.p, 16, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(b + 16, j.d_gmin, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(b + 16 + W, j.d_gmax, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(b + 16 + 2 * W, j.d_gamp, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-        uint8_t *hb = b + 16 + ((3 * W + 15) / 16) * 16;
-        CU(cudaMemcpyAsync(hb, j.d_cb, 8 * SP_CB_HIST_SIZE, cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(hb + 8 * SP_CB_HIST_SIZE, j.d_c, 8 * (size_t)rq->cmap_len, cudaMemcpyDeviceToHost, e->stream));
+        const Bounce at(W);
+        sp_reply dst = {};
+        dst.gauge_mins = b + at.gmin; dst.gauge_maxs = b + at.gmax; dst.gauge_amps = b + at.gamp;
+        dst.cB_hist = (uint64_t *)(b + at.cb); dst.c_hist = (uint64_t *)(b + at.c);
+        CU(cudaMemcpyAsync(b, e->stats_src, 16, cudaMemcpyDeviceToHost, e->stream));
+        if ((rc = copy_reply(e, j, dst))) return rc;
         CU(cudaEventRecord(slot->reply, e->stream));
         CU(cudaStreamWaitEvent(e->s_done, slot->reply, 0));
         for (int i = 0; i < 2; i++)
@@ -1282,11 +1291,7 @@ static int render_pipelined(sp_engine *e, const sp_request *rq, sp_reply *rp, Jo
         slot->launches = e->launches;
         return SP_OK;
     }
-    if (rp->gauge_mins) CU(cudaMemcpyAsync(rp->gauge_mins, j.d_gmin, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-    if (rp->gauge_maxs) CU(cudaMemcpyAsync(rp->gauge_maxs, j.d_gmax, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-    if (rp->gauge_amps) CU(cudaMemcpyAsync(rp->gauge_amps, j.d_gamp, (size_t)W, cudaMemcpyDeviceToHost, e->stream));
-    if (rp->cB_hist) CU(cudaMemcpyAsync(rp->cB_hist, j.d_cb, 8 * SP_CB_HIST_SIZE, cudaMemcpyDeviceToHost, e->stream));
-    if (rp->c_hist) CU(cudaMemcpyAsync(rp->c_hist, j.d_c, 8 * (size_t)rq->cmap_len, cudaMemcpyDeviceToHost, e->stream));
+    if ((rc = copy_reply(e, j, *rp))) return rc;
     CU(cudaStreamSynchronize(e->s_d2h));
     return finish(e, rp);
 }
@@ -1295,7 +1300,7 @@ static int finish(sp_engine *e, sp_reply *rp)
 {
     double st[2];
     unsigned long long ts[2] = { 0, 0 };
-    CU(cudaMemcpyAsync(st, e->stats_src ? (void *)e->stats_src : e->stats.p, 16, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(st, e->stats_src, 16, cudaMemcpyDeviceToHost, e->stream));
     if (e->stamped) CU(cudaMemcpyAsync(ts, e->tstamp.p, 16, cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     rp->dBfs_min = st[0];
@@ -1388,8 +1393,7 @@ extern "C" int sp_render_shards(sp_engine *e, const sp_request *rqs, sp_reply *r
 static int render_one(sp_engine *e, const sp_request *rq, sp_reply *rp, const Placement *pl)
 {
     Job j;
-    const bool host_io = !(rq->flags & (SP_F_BUFFER_ON_DEVICE | SP_F_REPLY_ON_DEVICE));
-    const long long ch = (host_io && rq->width > 0 && rq->n > 0 && rq->byte_length > 0) ? pipeline_chunk_frames(rq) : 0;
+    const long long ch = pipeline_chunk_frames(rq);
     j.pipelined = ch > 0;
     int rc = prepare(e, rq, rp, j, false, nullptr);
     if (rc) return rc;
@@ -1404,11 +1408,7 @@ static int render_one(sp_engine *e, const sp_request *rq, sp_reply *rp, const Pl
             else
                 CU(cudaMemcpyAsync(rp->image, j.d_image, 4 * W * (size_t)rq->n, cudaMemcpyDeviceToHost, e->stream));
         }
-        if (rp->gauge_mins) CU(cudaMemcpyAsync(rp->gauge_mins, j.d_gmin, W, cudaMemcpyDeviceToHost, e->stream));
-        if (rp->gauge_maxs) CU(cudaMemcpyAsync(rp->gauge_maxs, j.d_gmax, W, cudaMemcpyDeviceToHost, e->stream));
-        if (rp->gauge_amps) CU(cudaMemcpyAsync(rp->gauge_amps, j.d_gamp, W, cudaMemcpyDeviceToHost, e->stream));
-        if (rp->cB_hist) CU(cudaMemcpyAsync(rp->cB_hist, j.d_cb, 8 * SP_CB_HIST_SIZE, cudaMemcpyDeviceToHost, e->stream));
-        if (rp->c_hist) CU(cudaMemcpyAsync(rp->c_hist, j.d_c, 8 * (size_t)rq->cmap_len, cudaMemcpyDeviceToHost, e->stream));
+        if ((rc = copy_reply(e, j, *rp))) return rc;
     }
     return finish(e, rp);
 }
@@ -1439,7 +1439,6 @@ static int render_multi(sp_engine *e, const sp_request *rq, sp_reply *rp)
     const double sc = (double)rq->byte_length / (double)sw;
     const double stride = (sc - (double)n) / (double)(W - 1);                      // lib/worker.js:50, global
     auto cut = [&](int g) { return g >= G ? W : (g * W / G) / 8 * 8; };
-    auto pos = [&](long long x) { return (long long)(0.5 + stride * (double)x); }; // lib/worker.js:72
     struct Part { sp_request rq; sp_reply rp; Placement pl; std::vector<uint64_t> cb, c; int rc = 0; bool used = false; };
     std::vector<Part> parts((size_t)G);
     int last_used = -1;
@@ -1449,20 +1448,15 @@ static int render_multi(sp_engine *e, const sp_request *rq, sp_reply *rp)
         if (x1 <= x0) continue;
         Part &pt = parts[(size_t)g];
         pt.used = true;
-        long long s0 = pos(x0);
-        s0 -= s0 % 16;                                                             // any format's byte offset stays 16-byte aligned
-        const long long s1 = pos(x1 - 1) + n;
-        unsigned long long b0 = (unsigned long long)s0 * sw, b1 = (unsigned long long)s1 * sw;
-        if (b1 > rq->byte_length || g == last_used) b1 = rq->byte_length;          // a ragged tail travels with the last shard
-        if (b0 > b1) b0 = b1;
+        const Span span = frame_span(stride, (int)n, sw, x0, x1 - x0, 0, rq->byte_length, g == last_used);
         pt.rq = *rq;
-        pt.rq.buffer = (const uint8_t *)rq->buffer + b0;
-        pt.rq.byte_length = b1 - b0;
+        pt.rq.buffer = (const uint8_t *)rq->buffer + span.b0;
+        pt.rq.byte_length = span.b1 - span.b0;
         pt.rq.width = x1 - x0;
         pt.rq.total_byte_length = rq->byte_length;
         pt.rq.total_width = W;
         pt.rq.frame_first = x0;
-        pt.rq.buffer_first_sample = (uint64_t)s0;
+        pt.rq.buffer_first_sample = (uint64_t)span.s0;
         memset(&pt.rp, 0, sizeof pt.rp);
         pt.pl = Placement{ W, x0 };
         if (rp->image) pt.rp.image = rq->waterfall ? rp->image + (size_t)4 * n * (size_t)(W - x1) : rp->image;   // rows [W - x1, W - x0)
@@ -1521,16 +1515,16 @@ static int wait_slot(sp_engine *e, sp_engine::Inflight &s)
     sp_reply *rp = s.rp;
     const size_t W = (size_t)s.width;
     const uint8_t *b = s.bounce;
+    const Bounce at(s.width);
     double st[2];
     memcpy(st, b, 16);
     rp->dBfs_min = st[0];
     rp->dBfs_max = st[1];
-    if (rp->gauge_mins) memcpy(rp->gauge_mins, b + 16, W);
-    if (rp->gauge_maxs) memcpy(rp->gauge_maxs, b + 16 + W, W);
-    if (rp->gauge_amps) memcpy(rp->gauge_amps, b + 16 + 2 * W, W);
-    const uint8_t *hb = b + 16 + ((3 * W + 15) / 16) * 16;
-    if (rp->cB_hist) memcpy(rp->cB_hist, hb, 8 * SP_CB_HIST_SIZE);
-    if (rp->c_hist) memcpy(rp->c_hist, hb + 8 * SP_CB_HIST_SIZE, 8 * (size_t)s.cmap_len);
+    if (rp->gauge_mins) memcpy(rp->gauge_mins, b + at.gmin, W);
+    if (rp->gauge_maxs) memcpy(rp->gauge_maxs, b + at.gmax, W);
+    if (rp->gauge_amps) memcpy(rp->gauge_amps, b + at.gamp, W);
+    if (rp->cB_hist) memcpy(rp->cB_hist, b + at.cb, 8 * SP_CB_HIST_SIZE);
+    if (rp->c_hist) memcpy(rp->c_hist, b + at.c, 8 * (size_t)s.cmap_len);
     rp->device_ms = 0.0;                      // (per-message device time is not tracked for overlapping messages)
     rp->kernel_launches = s.launches;
     s.busy = false;
@@ -1547,15 +1541,14 @@ extern "C" int sp_render_async(sp_engine *e, const sp_request *rq, sp_reply *rp,
     if (rc) return rc;
     *ticket = e->next_ticket;
     s.ticket = e->next_ticket++;
-    const bool host_io = !(rq->flags & (SP_F_BUFFER_ON_DEVICE | SP_F_REPLY_ON_DEVICE));
-    const long long ch = (host_io && rq->width > 0 && rq->n > 0 && rq->byte_length > 0) ? pipeline_chunk_frames(rq) : 0;
+    const long long ch = pipeline_chunk_frames(rq);
     if (ch <= 0) return render_one(e, rq, rp, nullptr);    // short or device-resident message: nothing to overlap, done on return
     if (!s.done) {
         CU(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&s.reply, cudaEventDisableTiming));
     }
     if (!e->s_done) CU(cudaStreamCreateWithFlags(&e->s_done, cudaStreamNonBlocking));
-    const size_t need = 16 + (((size_t)3 * (size_t)rq->width + 15) / 16) * 16 + 8 * (size_t)(SP_CB_HIST_SIZE + SP_MAX_CMAP);
+    const size_t need = Bounce(rq->width).bytes;
     if (s.bounce_cap < need) {
         if (s.bounce) cudaFreeHost(s.bounce);
         s.bounce = nullptr; s.bounce_cap = 0;

@@ -23,7 +23,7 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
         out = eng.render(pin_in.array, "CS16", n, width, ww, 1 / wt, 6, 30, cm, out_image=pin_img.array)
         ts.append(time.perf_counter() - t0)
     ms = 1e3 * min(ts[1:])
-    print(json.dumps(dict(pipe_mb=os.environ.get("SP_PIPE_MB"), ramp=os.environ.get("SP_PIPE_RAMP", "1"), ms=ms, gsamples_s=S / ms / 1e6, launches=out["kernel_launches"],
+    print(json.dumps(dict(pipe_mb=os.environ.get("SP_PIPE_MB"), ms=ms, gsamples_s=S / ms / 1e6, launches=out["kernel_launches"],
                           gbs_each_way=S * 4 / ms / 1e6)), flush=True)
     if os.environ.get("SP_PIPE_MB") == "32":
         # raw copies: H2D alone, D2H alone, both at once
@@ -39,12 +39,6 @@ if len(sys.argv) > 1 and sys.argv[1] == "child":
         for name, f in (("h2d", h2d), ("d2h", d2h), ("both", lambda: (h2d(), d2h()))):
             f(); dt = min(t(f) for _ in range(3))
             print(json.dumps(dict(raw=name, ms=dt * 1e3, gbs=S * 4 / dt / 1e9)), flush=True)
-    sys.exit(0)
-if len(sys.argv) > 1 and sys.argv[1] == "ramp":      # A/B of the chunk-size ramp (SP_PIPE_RAMP), twice, on one box
-    for rep in range(2):
-        for mb in ("8", "16", "32"):
-            for ramp in ("0", "1"):
-                subprocess.run([sys.executable, __file__, "child"], env=dict(os.environ, SP_PIPE_MB=mb, SP_PIPE_RAMP=ramp))
     sys.exit(0)
 for mb in ("8", "16", "32", "64", "128", "0"):
     env = dict(os.environ, SP_PIPE_MB=mb)

@@ -29,14 +29,6 @@ __host__ __device__ constexpr int element_size(int f)
 
 // ------------------------------------------------------------------ JS helpers
 
-// `~~v` for a float: truncate toward zero; NaN, +-Inf and anything outside int32 give 0
-// (the reference wraps modulo 2^32 out there; those magnitudes do not occur on this path).
-__device__ __forceinline__ int js_trunc(float v)
-{
-    int r = __float2int_rz(v);              // NaN -> 0, saturating
-    return (fabsf(v) < 2147483648.0f) ? r : 0;
-}
-
 // log2 for the dB conversion: one MUFU.LG2 (flush-to-zero variant: a power below 1.2e-38, i.e.
 // more than 60 dB below the -120 dBFS floor of the parity contract, reads as 0 -> -inf like an
 // exact zero).  Relative error 2^-22: 4e-7 dB.

@@ -738,7 +738,6 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
         p.jC = (float)(-color_norm * c1 / cmaxd);
         p.jD = (float)((cmaxd - (block_norm_db + rq->gain) * color_norm) / cmaxd);
     }
-    { static const char *dbg = getenv("SP_DEBUG_SKIP"); p.dbg = dbg ? atoi(dbg) : 0; }
     p.waterfall = rq->waterfall ? 1 : 0;
     p.channel_mode = rq->channel_mode ? 1 : 0;
     p.sub_r = j.plan.sub_r;
@@ -910,9 +909,11 @@ static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
         if (L > S) L = S;
         if (L < 1) L = 1;
         const float2 *twT = nullptr;
+        // ringctl: BigArgs::ctl for up to 64 slots, then BigArgs::stats at the next 64-byte boundary
+        const size_t ctl_bytes = 4 * (size_t)(1 + 2 * 64), stats_off = (ctl_bytes + 63) & ~(size_t)63;
         if ((rc = get_table(e, Tw::tw14, 4096, &tw14)) || (rc = get_table(e, Tw::big, n, &twT))) return rc;
-        if ((rc = ensure(e, e->ring, (size_t)S * block_bytes)) || (rc = ensure(e, e->ringctl, 4 * (size_t)(1 + 2 * 64) + 64 + 64))) return rc;
-        if (e->l2_window != (size_t)S * block_bytes && !getenv("SP_BIG_NO_L2PIN")) {
+        if ((rc = ensure(e, e->ring, (size_t)S * block_bytes)) || (rc = ensure(e, e->ringctl, stats_off + 64))) return rc;
+        if (e->l2_window != (size_t)S * block_bytes) {
             // keep the ring in L2: persisting lines for the ring's address range, everything else streams through the rest
             cudaDeviceProp prop;
             CU(cudaGetDeviceProperties(&prop, e->dev));
@@ -932,7 +933,7 @@ static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
             }
             e->l2_window = want;
         }
-        CU(cudaMemsetAsync(e->ringctl.p, 0, 4 * (size_t)(1 + 2 * 64), e->stream));
+        CU(cudaMemsetAsync(e->ringctl.p, 0, ctl_bytes, e->stream));
         g.ring = (float2 *)e->ring.p;
         g.twT = twT;
         g.ctl = (unsigned *)e->ringctl.p;
@@ -940,18 +941,17 @@ static int launch_big_kernel(sp_engine *e, const sp::Kernels &k, const Params &q
         g.lead = L;
         g.nblocks = nf / 8;
         g.R = R;
-        g.dbg = getenv("SP_BIG_DBG") ? atoi(getenv("SP_BIG_DBG")) : 0;
-        // SP_BIG_STATS=1: per-phase SM cycle sums of the launch (development), printed when the engine is destroyed / next launch
+        // SP_BIG_STATS=1: per-phase SM cycle sums of the launch (development), printed at the next launch
         static const bool want_stats = getenv("SP_BIG_STATS") != nullptr;
         if (want_stats) {
-            g.stats = (unsigned long long *)((unsigned char *)e->ringctl.p + ((4 * (size_t)(1 + 2 * 64) + 63) & ~(size_t)63));
-            unsigned long long h[8];
+            g.stats = (unsigned long long *)((unsigned char *)e->ringctl.p + stats_off);
+            unsigned long long h[6];
             CU(cudaMemcpyAsync(h, g.stats, sizeof h, cudaMemcpyDeviceToHost, e->stream));   // the PREVIOUS launch's sums (stream order)
             CU(cudaStreamSynchronize(e->stream));
             if (h[4] || h[5])
-                fprintf(stderr, "[big] P: %llu items, wait %.0f work %.0f (first frame landed after %.0f, 8-frame loop %.0f) cycles/item | F: %llu tiles, wait %.0f work %.0f cycles/tile\n", h[4],
-                        h[4] ? (double)h[0] / h[4] : 0.0, h[4] ? (double)h[1] / h[4] : 0.0, h[4] ? (double)h[6] / h[4] : 0.0, h[4] ? (double)h[7] / h[4] : 0.0, h[5], h[5] ? (double)h[2] / h[5] : 0.0, h[5] ? (double)h[3] / h[5] : 0.0);
-            CU(cudaMemsetAsync(g.stats, 0, 64, e->stream));
+                fprintf(stderr, "[big] P: %llu items, wait %.0f work %.0f cycles/item | F: %llu tiles, wait %.0f work %.0f cycles/tile\n", h[4],
+                        h[4] ? (double)h[0] / h[4] : 0.0, h[4] ? (double)h[1] / h[4] : 0.0, h[5], h[5] ? (double)h[2] / h[5] : 0.0, h[5] ? (double)h[3] / h[5] : 0.0);
+            CU(cudaMemsetAsync(g.stats, 0, sizeof h, e->stream));
         }
         return SP_OK;
     };

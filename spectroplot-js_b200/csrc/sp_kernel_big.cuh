@@ -28,8 +28,10 @@ struct BigArgs {
     int slots, lead;           // S, L
     long long nblocks;         // blocks of 8 frames rendered by this launch (frames chunk_first .. chunk_first + 8*nblocks)
     int R;
-    int dbg;                   // timing experiments (wrong output): 1 no ring stores, 2 no dft / twiddle in the pre-pass, 4 no fence
-    unsigned long long *stats; // optional [8]: SM cycles summed over CTAs (thread 0's clock): P wait, P work, F wait, F work, P items, F items, idle tail
+    // optional [6] (SP_BIG_STATS): SM cycles summed over CTAs (thread 0's clock): P wait, P work, F wait, F work, P items, F items.
+    // Without these hooks ptxas keeps the queue item and its decode in vector registers instead of uniform ones, and the ring
+    // form of the packed formats runs 5 - 8 % slower (profiles/r05_switches_ab.txt).
+    unsigned long long *stats;
 };
 
 struct BigCfg {
@@ -182,22 +184,18 @@ __device__ __forceinline__ void big_prepass_tma(const Params &p, const BigArgs &
         for (int q = 0; q < PPT; q++) {
 #pragma unroll
             for (int a = 0; a < R; a++) v[q][a] = cscale(v[q][a], CACHE ? w[a][q] : __ldg(p.window + 4096 * a + j + q));
-            if (!(g.dbg & 2)) {
-                dft<R>(v[q]);
+            dft<R>(v[q]);
 #pragma unroll
-                for (int k = 1; k < R; k++) v[q][k] = cmul(v[q][k], CACHE ? tw[k][q] : __ldg(g.twT + (size_t)(k - 1) * 4096 + j + q));
-            }
+            for (int k = 1; k < R; k++) v[q][k] = cmul(v[q][k], CACHE ? tw[k][q] : __ldg(g.twT + (size_t)(k - 1) * 4096 + j + q));
         }
         float2 *dst = slot + (size_t)f * frame_f2 + j;
-        if (!(g.dbg & 1)) {
 #pragma unroll
-            for (int k = 0; k < R; k++) {
-                if constexpr (PPT == 2) {
-                    const float2 x0 = cun(v[0][k]), x1 = cun(v[1][k]);
-                    *reinterpret_cast<float4 *>(dst + (size_t)k * 4096) = make_float4(x0.x, x0.y, x1.x, x1.y);
-                } else cst(dst + (size_t)k * 4096, v[0][k]);
-            }
-        } else if (cre(v[0][0]) == 1234.5f) cst(dst, v[0][1]);
+        for (int k = 0; k < R; k++) {
+            if constexpr (PPT == 2) {
+                const float2 x0 = cun(v[0][k]), x1 = cun(v[1][k]);
+                *reinterpret_cast<float4 *>(dst + (size_t)k * 4096) = make_float4(x0.x, x0.y, x1.x, x1.y);
+            } else cst(dst + (size_t)k * 4096, v[0][k]);
+        }
     }
 }
 template <int R, int FMT>
@@ -346,7 +344,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
                 case 32: big_prepass_any<32, FMT>(p, g, blk, (int)sub, ring, tid, s_x, s_pbar, s_poff, tpar); break;
                 default: big_prepass_any<64, FMT>(p, g, blk, (int)sub, ring, tid, s_x, s_pbar, s_poff, tpar); break;
                 }
-                if (!(g.dbg & 4)) __threadfence();
+                __threadfence();
                 fft_barrier();
                 if (tid == 0) {
                     atomicAdd(p_cnt + slot, 1u);

@@ -243,9 +243,8 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                         const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;   // :117
                         uint4 a, b;
-                        if (!(p.dbg & 4)) lut_row8(lut_base, w, j, a, b);
-                        else { a = make_uint4(w[0], w[1], w[2], w[3]); b = make_uint4(w[4], w[5], w[6], w[7]); }
-                        if (!(p.dbg & 1)) store_row8(rowp, a, b, rows_aligned);
+                        lut_row8(lut_base, w, j, a, b);
+                        store_row8(rowp, a, b, rows_aligned);
                     }
                 }
                 if (ht < 8 && live) {

@@ -156,7 +156,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         // overlapping frames (hop < N): ONE copy of the span, every frame decodes from its own offset in it
         const long long span = p0[FWS - 1] - p0[0] + N;
-        if (FWS > 1 && span < (long long)FWS * N && span * B::SWB + 32 <= FWS * B::RAWP && !(p.dbg & 16)) {     // (SP_DEBUG_SKIP=16: per-frame copies, for the A/B of the reuse counters)
+        if (FWS > 1 && span < (long long)FWS * N && span * B::SWB + 32 <= FWS * B::RAWP) {
             const unsigned long long o0 = (unsigned long long)p0[0] * B::SWB, a0 = o0 & ~15ull;
             const unsigned bytes = (unsigned)(((o0 - a0) + (unsigned long long)span * B::SWB + 15) & ~15ull);
 #pragma unroll

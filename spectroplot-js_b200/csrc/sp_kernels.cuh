@@ -57,8 +57,6 @@ struct Params {
     unsigned long long *j_hist;    // [JH_SIZE]
     float jA, jB, jC, jD;          // see jh_eval()
     int use_tma;                   // render_r64_kernel: image rows leave through tensor-TMA stores (width % 4 == 0, 16-byte aligned image)
-    int dbg;                       // SP_DEBUG_SKIP bit mask (performance experiments only): 1 image stores, 4 LUT lookups (store warps of render_r64_kernel),
-                                   // 16 no span staging in render_w_kernel (every frame copied on its own)
     unsigned long long *tile_ctr;  // render_r64_kernel: the launch's tile counter, zero at launch and left at zero by the launch
     unsigned long long *t_stamp;   // render_r64_kernel: %globaltimer at the start of CTA 0 goes to t_stamp[0] (null: not recorded)
 };

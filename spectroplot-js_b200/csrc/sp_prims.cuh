@@ -40,11 +40,6 @@ __device__ __forceinline__ void st_global_256(void *p, uint4 a, uint4 b)
     asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w),
                  "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
 }
-__device__ __forceinline__ void red_shared_inc(unsigned *p)
-{
-    asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(smem_u32(p)) : "memory");
-}
-
 __device__ __forceinline__ void red_shared_inc_addr(unsigned addr)
 {
     asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(addr) : "memory");

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Round-2 evidence visit (one B200): parity suite, bench (both arms), ncu launch list, ncu --set full of the three new / changed
-# kernel families, hop-overlap counters of render_w_kernel with and without span staging, size sweep.
+# kernel families, size sweep.
 # usage (under gpurun): bash tools/gpu_round2.sh TAG
 TAG=${1:-r2}; OUT=gpurun_out; mkdir -p $OUT
 nvidia-smi --query-gpu=name,clocks.sm,clocks.max.sm,power.draw --format=csv > $OUT/smi_$TAG.txt; nproc > $OUT/nproc_$TAG.txt
@@ -15,11 +15,6 @@ timeout -s KILL 400 ncu --set full --clock-control none --import-source on -k re
     python tools/sweep.py X:CS16:512:1:26 1 > $OUT/ncu_full_w_$TAG.log 2>&1
 SP_FOURSTEP=ring timeout -s KILL 400 ncu --set full --clock-control none --import-source on -k regex:render_big -s 3 -c 1 -f -o $OUT/prof_big_$TAG \
     python tools/sweep.py C5 1 > $OUT/ncu_full_big_$TAG.log 2>&1
-M=gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum,lts__t_sectors_op_read.sum,lts__t_sector_op_read_hit_rate.pct,l1tex__data_pipe_lsu_wavefronts_mem_shared_op_ld.sum,smsp__inst_executed.sum
-for dbg in 0 16; do
-  SP_DEBUG_SKIP=$dbg timeout -s KILL 400 ncu --metrics $M --clock-control none -k regex:render_w_ -c 40 --csv --log-file $OUT/overlap_w_dbg${dbg}_$TAG.csv \
-      python tools/sweep.py X:CS16:128:1:24,X:CS16:128:2:24,X:CS16:128:4:24,X:CS16:128:8:24,X:CS16:256:4:24,X:CS16:512:4:24 1 > $OUT/overlap_w_dbg${dbg}_$TAG.log 2>&1
-done
 CASES=$(for n in 64 128 256 512 1024 2048 4096 8192 16384 32768 65536 131072; do echo -n "X:CS16:$n:1:26,"; done)
 timeout -s KILL 600 python tools/sweep.py ${CASES}C1,C2,C2-hann,C2-z2,C2-z4,C2-z8 5 > $OUT/sweep_$TAG.jsonl 2> $OUT/sweep_$TAG.err
 tail -3 $OUT/pytest_gpu_$TAG.log; cut -c1-400 $OUT/bench_$TAG.json; tail -3 $OUT/bench_$TAG.err; ls -la $OUT | tail -25

@@ -8,8 +8,6 @@ cp $G/bench_$TAG.json $P/r02_bench.json
 cp $G/bench_ref_$TAG.json $P/r02_bench_ref.json
 cp $G/launches_$TAG.csv $P/r02_launches.csv
 cp $G/sweep_$TAG.jsonl $P/r02_sweep.jsonl
-cp $G/overlap_w_dbg0_$TAG.csv $P/r02_overlap_w_dbg0.csv
-cp $G/overlap_w_dbg16_$TAG.csv $P/r02_overlap_w_dbg16.csv
 cp $G/pytest_gpu_$TAG.log $P/r02_pytest_gpu.log
 for k in r64 w big; do
   [ -f $G/prof_${k}_$TAG.ncu-rep ] && bash tools/ncu_sum.sh $G/prof_${k}_$TAG.ncu-rep > $P/r02_ncu_summary_$k.txt

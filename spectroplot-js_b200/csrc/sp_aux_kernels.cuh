@@ -125,7 +125,7 @@ __global__ void decode_kernel(const uint8_t *buf, unsigned long long valid_bytes
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     const long long s = first + i;
-    const bool inside = s >= 0 && (unsigned long long)(s + 1) * (unsigned)sample_width(fmt) <= valid_bytes;
+    const bool inside = samples_inside(s, 1, sample_width(fmt), valid_bytes);
     out[i] = inside ? decode_fast<FMT_RUNTIME>(buf, s, fmt) : decode_checked(buf, s, fmt, valid_bytes);
 }
 

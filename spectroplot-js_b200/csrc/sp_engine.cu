@@ -119,7 +119,7 @@ struct DevBuf {
 struct Placement { long long pitch_frames; long long col0; };
 
 // kinds of twiddle table (get_table)
-enum class Tw { full, big, passA, passB, tw14, w };
+enum class Tw { big, passA, passB, tw14, w };
 
 struct sp_engine {
     std::vector<sp_engine *> subs;           // ndev > 1: one single-device engine per GPU; this object only dispatches
@@ -355,9 +355,6 @@ static int ilog2_exact(int n)
     return -1;
 }
 
-// first sample of global frame x (lib/worker.js:72)
-static long long frame_pos(double stride, long long x) { return (long long)(0.5 + stride * (double)x); }
-
 // The samples that global frames [x0, x0 + count) read, as a piece of a buffer that starts at sample buf_first and holds
 // byte_length bytes: sample s0 and bytes [b0, b1) of the buffer.  The start is rounded down to 16 samples (any format's byte
 // offset stays 16-byte aligned), the end is the last frame's start + n.  The piece takes the samples its frames read and nothing
@@ -368,8 +365,8 @@ struct Span { long long s0; unsigned long long b0, b1; };
 static Span frame_span(double stride, int n, int sw, long long x0, long long count, long long buf_first, unsigned long long byte_length,
                        bool msg_last)
 {
-    long long s0 = frame_pos(stride, x0);
-    const long long s1 = frame_pos(stride, x0 + count - 1) + n;
+    long long s0 = sp::frame_pos(stride, x0);
+    const long long s1 = sp::frame_pos(stride, x0 + count - 1) + n;
     s0 -= s0 % 16;
     if (s0 < buf_first) s0 = buf_first;
     unsigned long long b0 = (unsigned long long)(s0 - buf_first) * sw, b1 = (unsigned long long)(s1 - buf_first) * sw;
@@ -394,8 +391,8 @@ static inline float2 twid(long long num, long long den)   // exp(-2 pi j num / d
     return make_float2((float)cos(a), (float)-sin(a));
 }
 // The table of one kind for size n, built and uploaded on first use:
-//   full   [n]          W_n^i                                   pre-pass of the four-step sizes
-//   big    [R-1][4096]  W_n^{j*k}, k = 1 .. R-1, j fastest      pre-pass of render_big_kernel, n = R * 4096 (coalesced loads)
+//   big    [R-1][4096]  W_n^{j*k}, k = 1 .. R-1, j fastest      pre-passes of the four-step sizes, n = R * 4096: render_big_kernel
+//                                                               and prepass_kernel (coalesced loads)
 //   passA  [15][n/16]   W_n^{t*k}, k = 1 .. 15                  render_kernel, n >= 32
 //   passB  [15][n/256]  W_{n/16}^{b*k}, k = 1 .. 15             render_kernel, n >= 512
 //   tw14   [n/64][14]   W_n^{t*k}, k = 1 .. 7, 8, 16, .., 56    render_r64_kernel (n = 4096), render_rc_kernel (n = 2048)
@@ -406,10 +403,6 @@ static int get_table(sp_engine *e, Tw kind, int n, const float2 **out)
     if (it != e->tw.end()) { *out = it->second; return SP_OK; }
     std::vector<float2> h;
     switch (kind) {
-    case Tw::full:
-        h.resize((size_t)n);
-        for (int i = 0; i < n; i++) h[i] = twid(i, n);
-        break;
     case Tw::big: {
         const int R = n / 4096;
         h.resize((size_t)(R - 1) * 4096);
@@ -604,8 +597,8 @@ static int validate(sp_engine *e, const sp_request *rq, bool shard, double *samp
             return fail(e, SP_E_RANGE, "frame range [%lld, %lld) outside total width %lld", (long long)rq->frame_first,
                         (long long)(rq->frame_first + rq->width), (long long)total_width);
         // the shard buffer must cover every sample its frames read
-        const long long p_first = frame_pos(*stride, rq->frame_first);
-        const long long p_last = frame_pos(*stride, rq->frame_first + rq->width - 1) + rq->n;
+        const long long p_first = sp::frame_pos(*stride, rq->frame_first);
+        const long long p_last = sp::frame_pos(*stride, rq->frame_first + rq->width - 1) + rq->n;
         const long long have_first = (long long)rq->buffer_first_sample;
         const double have_last = (double)have_first + (double)rq->byte_length / sp::sample_width(rq->format);
         if (p_first < have_first || ((double)p_last > have_last && (double)p_last <= sc))
@@ -812,14 +805,11 @@ static bool image_tensor_map(CUtensorMap *tm, uint8_t *image, long long width, i
 
 // The leading whole groups of 8 frames of the chunk q whose `len` samples lie inside the buffer: the same frames whatever the
 // chunking or sharding, so pipelined / sharded renders stay bit-identical to the single shot.  The fused kernels stage raw frames
-// in whole 16-byte units, which the buffer's readable slack covers as long as the frame itself lies inside.
+// in whole 16-byte units (sp::staged_extent), which the buffer's readable slack covers as long as the frame itself lies inside.
 static long long frames_inside(const Params &q, int len)
 {
-    const long long sw = sp::sample_width(q.format);
-    auto inside = [&](long long xr) {
-        const long long p0 = frame_pos(q.stride, q.frame_first + q.chunk_first + xr) - q.sample_base;
-        return p0 >= 0 && (unsigned long long)(p0 + len) * (unsigned long long)sw <= q.valid_bytes;
-    };
+    const int sw = sp::sample_width(q.format);
+    auto inside = [&](long long xr) { return sp::samples_inside(sp::frame_start(q, xr), len, sw, q.valid_bytes); };
     long long nf = q.chunk_frames / 8 * 8;                 // the last tile may be partial (a multiple of 8 frames)
     while (nf > 0 && !inside(nf - 1)) nf -= 8;
     if (nf > 0 && !inside(0)) nf = 0;
@@ -1062,8 +1052,8 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
         const int n = p.n_full;
         const sp::Kernels &sub = kernels_for(SP_CF32);        // sub-frame input is always complex fp32
         if (!sub.render || !k.prepass) return fail(e, SP_E_CUDA, "no kernels linked for the four-step path");
-        const float2 *tw_full = nullptr;
-        int rc = get_table(e, Tw::full, n, &tw_full);
+        const float2 *twT = nullptr;
+        int rc = get_table(e, Tw::big, n, &twT);
         if (rc) return rc;
         // frames per chunk: a 1 GB scratch (2^27 / n frames of n complex floats: a power of two, at least 512).  An L2-sized
         // scratch (<= 96 MB) keeps the 16 B/sample of scratch traffic out of HBM but leaves each launch with about one wave of
@@ -1096,7 +1086,7 @@ static int enqueue_frames(sp_engine *e, Job &j, Params &p)
             Params q = p;
             q.chunk_first = c0;
             q.chunk_frames = (nf - c0 < ch) ? nf - c0 : ch;
-            CU(k.prepass(R, &q, (float2 *)e->scratch.p, tw_full, e->stream));
+            CU(k.prepass(R, &q, (float2 *)e->scratch.p, twT, e->stream));
             q.sub_in = (const float2 *)e->scratch.p;
             e->launches++;
             Params full = q;                                   // what the epilogue kernel sees

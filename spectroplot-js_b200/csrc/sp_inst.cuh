@@ -15,7 +15,7 @@ namespace sp {
 // nothing; a kernel that is not built for the format answers 0.
 struct Kernels {
     cudaError_t (*render)(int log2n, const Params *p, int grid, size_t smem, cudaStream_t st, int *occ_out);
-    cudaError_t (*prepass)(int r, const Params *p, float2 *out, const float2 *tw_full, cudaStream_t st);
+    cudaError_t (*prepass)(int r, const Params *p, float2 *out, const float2 *twT, cudaStream_t st);
     cudaError_t (*r64)(int sub, const Params *p, int grid, cudaStream_t st, const float2 *tw14, const CUtensorMap *tm, int pdl, int *occ_out);
     cudaError_t (*rc)(int log2n, const Params *p, int grid, cudaStream_t st, const float2 *tw14, int *occ_out);
     cudaError_t (*w)(int log2n, const Params *p, int grid, cudaStream_t st, const float2 *twW, int *occ_out);
@@ -80,18 +80,18 @@ static cudaError_t launch_render(int log2n, const Params *p, int grid, size_t sm
 }
 
 template <int FMT>
-static cudaError_t launch_prepass(int r, const Params *pp, float2 *out, const float2 *tw_full, cudaStream_t st)
+static cudaError_t launch_prepass(int r, const Params *pp, float2 *out, const float2 *twT, cudaStream_t st)
 {
     const Params &p = *pp;
     const long long threads = p.chunk_frames * 4096;
     const int grid = (int)((threads + 255) / 256);
     switch (r) {
-    case 2: prepass_kernel<2, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
-    case 4: prepass_kernel<4, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
-    case 8: prepass_kernel<8, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
-    case 16: prepass_kernel<16, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
-    case 32: prepass_kernel<32, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
-    case 64: prepass_kernel<64, FMT><<<grid, 256, 0, st>>>(p, out, tw_full); break;
+    case 2: prepass_kernel<2, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
+    case 4: prepass_kernel<4, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
+    case 8: prepass_kernel<8, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
+    case 16: prepass_kernel<16, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
+    case 32: prepass_kernel<32, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
+    case 64: prepass_kernel<64, FMT><<<grid, 256, 0, st>>>(p, out, twT); break;
     default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

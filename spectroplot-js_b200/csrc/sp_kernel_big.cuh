@@ -73,7 +73,7 @@ __device__ __forceinline__ void big_prepass(const Params &p, const BigArgs &g, l
 #pragma unroll
         for (int u = 0; u < U; u++) {
             const long long xgl = p.frame_first + p.chunk_first + blk * 8 + f0 + u;
-            const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;   // lib/worker.js:72
+            const long long p0 = frame_pos(p.stride, xgl) - p.sample_base;
 #pragma unroll
             for (int a = 0; a < R; a++) v[u][a] = decode_raw_cf<FMT>(p.buf, p0 + 4096 * a + j, p.format);
         }
@@ -81,8 +81,7 @@ __device__ __forceinline__ void big_prepass(const Params &p, const BigArgs &g, l
     auto finish = [&](cf (&v)[U][R], int f0) {
 #pragma unroll
         for (int u = 0; u < U; u++) {
-            if (j == 0)       // sample p0 + n/2 (lib/worker.js:131)
-                p.fmid[p.chunk_first + blk * 8 + f0 + u] = make_float2(cre(v[u][R / 2]) * raw_scale<FMT>(), cim(v[u][R / 2]) * raw_scale<FMT>());
+            if (j == 0) p.fmid[p.chunk_first + blk * 8 + f0 + u] = raw_mid<FMT>(v[u][R / 2]);
 #pragma unroll
             for (int a = 0; a < R; a++) v[u][a] = cscale(v[u][a], CACHE ? w[a] : __ldg(p.window + 4096 * a + j));
             dft<R>(v[u]);
@@ -140,18 +139,16 @@ __device__ __forceinline__ void big_prepass_tma(const Params &p, const BigArgs &
     auto issue = [&](int f) {
         const int b = f & 1;
         const long long xgl = p.frame_first + p.chunk_first + blk * 8 + f;
-        const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;   // lib/worker.js:72
-        const unsigned long long off = (unsigned long long)(p0 + jg * C::PTS) * SW;
-        const unsigned bytes = (((unsigned)off & 15u) + (unsigned)C::PTS * SW + 15u) & ~15u;
-        const unsigned char *src = p.buf + (off & ~15ull);
+        const Extent e = staged_extent(frame_pos(p.stride, xgl) - p.sample_base + jg * C::PTS, SW, C::PTS);
+        const unsigned char *src = p.buf + e.src;
         const unsigned dst = smem_u32(stage) + (unsigned)b * (R * SEG), bar = smem_u32(bars + b);
-        s_poff[b] = (int)(off & 15ull);
+        s_poff[b] = e.skew;
         fence_async_smem();                                        // the FFT warps' reads of this buffer (through the barrier) vs the async writes
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes * R) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(e.bytes * R) : "memory");
 #pragma unroll
         for (int a = 0; a < R; a++)
             asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(dst + a * SEG), "l"(src + (size_t)4096 * a * SW), "r"(bytes), "r"(bar) : "memory");
+                         ::"r"(dst + a * SEG), "l"(src + (size_t)4096 * a * SW), "r"(e.bytes), "r"(bar) : "memory");
     };
     if (tid == 0) { issue(0); issue(1); }
     if constexpr (CACHE) {
@@ -178,8 +175,7 @@ __device__ __forceinline__ void big_prepass_tma(const Params &p, const BigArgs &
             for (int q = 0; q < PPT; q++) v[q][a] = decode_raw_cf<FMT>(fp + a * SEG, tid * PPT + q, p.format);
         fft_barrier();                                             // everyone has read buffer b: the frame after next may land in it
         if (tid == 0 && f + 2 < 8) issue(f + 2);
-        if (j == 0)       // sample p0 + n/2 (lib/worker.js:131)
-            p.fmid[p.chunk_first + blk * 8 + f] = make_float2(cre(v[0][R / 2]) * raw_scale<FMT>(), cim(v[0][R / 2]) * raw_scale<FMT>());
+        if (j == 0) p.fmid[p.chunk_first + blk * 8 + f] = raw_mid<FMT>(v[0][R / 2]);
 #pragma unroll
         for (int q = 0; q < PPT; q++) {
 #pragma unroll
@@ -272,8 +268,7 @@ __global__ void __launch_bounds__(384, 1) render_big_kernel(const Params p, cons
 #pragma unroll
                     for (int j = 0; j < 4; j++) {
                         const int bin = k0sub + R * (k0 + 64 * (4 * m + j));
-                        const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
-                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;   // :117
+                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)image_row(bin, nfull) + x0;
                         uint4 a, b;
                         lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);

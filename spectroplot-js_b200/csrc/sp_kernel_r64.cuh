@@ -102,11 +102,10 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
             s_off[s * 2 + par] = 0;
         } else {
             const long long xgl = p.frame_first + p.chunk_first + xr;
-            const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;   // lib/worker.js:72
-            const unsigned long long off = (unsigned long long)p0 * B::SWB, a0 = off & ~15ull;
-            src = p.buf + a0;
-            bytes = (unsigned)(((off - a0) + (unsigned long long)N * B::SWB + 15) & ~15ull);
-            s_off[s * 2 + par] = (int)(off - a0);
+            const Extent e = staged_extent(frame_pos(p.stride, xgl) - p.sample_base, B::SWB, N);
+            src = p.buf + e.src;
+            bytes = e.bytes;
+            s_off[s * 2 + par] = e.skew;
         }
         tma_load_1d(raw, src, bytes, mbar);
     };
@@ -181,7 +180,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                                 const unsigned w = src[B::STORE_THREADS * i];
 #pragma unroll
                                 for (int j = 0; j < 4; j++)
-                                    rowp[(k0 + 64 * (4 * m + j) + N / 2 - 1) & (N - 1)] = lut_at(lut_base, w, j);
+                                    rowp[waterfall_col(k0 + 64 * (4 * m + j), N)] = lut_at(lut_base, w, j);
                             }
                         }
                     }
@@ -240,8 +239,7 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     for (int j = 0; j < 4; j++) {
                         const int kb = k0 + 64 * (4 * m + j);
                         const int bin = SUB ? k0sub + sub_r * kb : kb;
-                        const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
-                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;   // :117
+                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)image_row(bin, nfull) + x0;
                         uint4 a, b;
                         lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
@@ -313,9 +311,9 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                     cf d[4];
 #pragma unroll
                     for (int c = 0; c < 4; c++) d[c] = decode_raw_cf<FMT>(rp, T * (4 * q + c) + t, p.format);
-                    // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact.  The store warps write it out
-                    // (no global writes here, see griddep_wait); by parity of the tile, as this runs before the wait for the half
-                    if (q == 8 && t == 0 && valid) s_fmid[(kk & 1) * F + fl] = make_float2(cre(d[0]) * raw_scale<FMT>(), cim(d[0]) * raw_scale<FMT>());
+                    // raw sample at p0 + n/2.  The store warps write it out (no global writes here, see griddep_wait); by parity of
+                    // the tile, as this runs before the wait for the half
+                    if (q == 8 && t == 0 && valid) s_fmid[(kk & 1) * F + fl] = raw_mid<FMT>(d[0]);
                     v[4 * q] = cscale(d[0], w.x);     v[4 * q + 1] = cscale(d[1], w.y);
                     v[4 * q + 2] = cscale(d[2], w.z); v[4 * q + 3] = cscale(d[3], w.w);
                 }
@@ -350,14 +348,6 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                             // bin i = t + 64*k1 pairs with bin n - i = (64 - t) + 64*(63 - k1): thread 64 - t, register 63 - k1 (thread 0
                             // pairs with itself, register 64 - k1).  One more pass through the exchange buffer: rows written with
                             // STS.128, the partner's row read back reversed with LDS.128 (both conflict-free at this pitch).
-                            auto split_lo = [](cf a, cf b) {                    // i < n/2:  (re_i + re_p, im_i - im_p) / 2
-                                const float2 fb = cun(b);
-                                return cscale(cadd(a, cpk(fb.x, -fb.y)), 0.5f);
-                            };
-                            auto split_hi = [](cf a, cf b) {                    // i > n/2:  (im_p + im_i, -re_p + re_i) / 2, p = n - i
-                                const float2 fa = cun(a), fb = cun(b);
-                                return cscale(cadd(cpk(fa.y, fa.x), cpk(fb.y, -fb.x)), 0.5f);
-                            };
                             {
                                 float4 *wrow = reinterpret_cast<float4 *>(X + t * B::XP);
 #pragma unroll
@@ -374,8 +364,8 @@ __global__ void __launch_bounds__(384, 1) render_r64_kernel(const Params p, cons
                                     v[k1] = split_lo(a, b);
                                     v[64 - k1] = split_hi(b, a);
                                 }
-                                v[0] = cpk(fmaf(0.0f, cim(v[0]), cre(v[0])), 0.0f);   // imag[0] = 0; a NaN there reaches real[0] in the reference (NaN * 0)
-                                v[32] = cpk(0.0f, 0.0f);                        // real[n/2] = imag[0] (just zeroed), imag[n/2] = 0
+                                v[0] = split_dc(cun(v[0]));
+                                v[32] = split_nyquist();
                             } else {
                                 const float4 *prow = reinterpret_cast<const float4 *>(X + (64 - t) * B::XP);
 #pragma unroll

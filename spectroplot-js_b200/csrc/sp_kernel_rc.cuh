@@ -82,11 +82,10 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
         for (int i = 0; i < FS; i++) {
             const long long xc = xr + i < p.chunk_frames ? xr + i : p.chunk_frames - 1;   // partial last tile: redo the last frame
             const long long xgl = p.frame_first + p.chunk_first + xc;
-            const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;   // lib/worker.js:72
-            const unsigned long long off = (unsigned long long)p0 * B::SWB, a0 = off & ~15ull;
-            src[i] = p.buf + a0;
-            bytes[i] = (unsigned)(((off - a0) + (unsigned long long)N * B::SWB + 15) & ~15ull);
-            s_off[(s * 2 + par) * FS + i] = (int)(off - a0);
+            const Extent e = staged_extent(frame_pos(p.stride, xgl) - p.sample_base, B::SWB, N);
+            src[i] = p.buf + e.src;
+            bytes[i] = e.bytes;
+            s_off[(s * 2 + par) * FS + i] = e.skew;
             total += bytes[i];
         }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -131,7 +130,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
                         const unsigned w = half[fl * B::FPW + m * 64 + (o % RPT) * C + o / RPT];
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)N * (size_t)(p.nframes - 1 - (long long)(x0 + fl));
 #pragma unroll
-                        for (int j = 0; j < 4; j++) rowp[(o + 64 * (4 * m + j) + N / 2 - 1) & (N - 1)] = lut_at(lut_base, w, j);
+                        for (int j = 0; j < 4; j++) rowp[waterfall_col(o + 64 * (4 * m + j), N)] = lut_at(lut_base, w, j);
                     }
                 }
 #pragma unroll 1
@@ -150,8 +149,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
 #pragma unroll
                     for (int j = 0; j < 4; j++) {
                         const int bin = tc * RPT + r + 64 * (4 * m + j);
-                        const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
-                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0 + 8 * grp;   // :117
+                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)image_row(bin, nfull) + x0 + 8 * grp;
                         uint4 a, b;
                         lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
@@ -194,8 +192,7 @@ __global__ void __launch_bounds__(384, 1) render_rc_kernel(const Params p, const
                 const unsigned char *rp = xs + fi * B::RAWP + s_off[(s * 2 + fpar) * FS + fi];
 #pragma unroll
                 for (int a = 0; a < 64; a++) v[a] = decode_raw_cf<FMT>(rp, C * a + t, p.format);
-                // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact
-                if (t == 0 && valid) p.fmid[p.chunk_first + xr0 + fl] = make_float2(cre(v[32]) * raw_scale<FMT>(), cim(v[32]) * raw_scale<FMT>());
+                if (t == 0 && valid) p.fmid[p.chunk_first + xr0 + fl] = raw_mid<FMT>(v[32]);
                 const float4 *wrow = reinterpret_cast<const float4 *>(s_win + t * 64);
 #pragma unroll
                 for (int q = 0; q < 16; q++) {

@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
             const int i = lane < FWS ? lane : FWS - 1;
             const long long xc = xr + i < p.chunk_frames ? xr + i : p.chunk_frames - 1;   // partial last tile: redo the last frame
             const long long xgl = p.frame_first + p.chunk_first + xc;
-            const long long mine = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;   // lib/worker.js:72
+            const long long mine = frame_pos(p.stride, xgl) - p.sample_base;
 #pragma unroll
             for (int k = 0; k < FWS; k++) p0[k] = __shfl_sync(0xffffffffu, mine, k);
             if (lane != 0) return;
@@ -149,7 +149,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
             for (int i = 0; i < FWS; i++) {
                 const long long xc = xr + i < p.chunk_frames ? xr + i : p.chunk_frames - 1;
                 const long long xgl = p.frame_first + p.chunk_first + xc;
-                p0[i] = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;
+                p0[i] = frame_pos(p.stride, xgl) - p.sample_base;
             }
         }
         int *off = s_off + (warp * 2 + par) * FWS;
@@ -157,6 +157,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
         // overlapping frames (hop < N): ONE copy of the span, every frame decodes from its own offset in it
         const long long span = p0[FWS - 1] - p0[0] + N;
         if (FWS > 1 && span < (long long)FWS * N && span * B::SWB + 32 <= FWS * B::RAWP) {
+            // staged_extent(p0[0], B::SWB, span), written out: the call changes this kernel's machine code
             const unsigned long long o0 = (unsigned long long)p0[0] * B::SWB, a0 = o0 & ~15ull;
             const unsigned bytes = (unsigned)(((o0 - a0) + (unsigned long long)span * B::SWB + 15) & ~15ull);
 #pragma unroll
@@ -165,21 +166,19 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
             asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                          ::"r"(smem_u32(xs)), "l"(p.buf + a0), "r"(bytes), "r"(smem_u32(mbar)) : "memory");
         } else {
-            unsigned total = 0, bytes[FWS];
-            unsigned long long a0[FWS];
+            unsigned total = 0;
+            Extent e[FWS];
 #pragma unroll
             for (int i = 0; i < FWS; i++) {
-                const unsigned long long o = (unsigned long long)p0[i] * B::SWB;
-                a0[i] = o & ~15ull;
-                bytes[i] = (unsigned)(((o - a0[i]) + (unsigned long long)N * B::SWB + 15) & ~15ull);
-                off[i] = i * B::RAWP + (int)(o - a0[i]);
-                total += bytes[i];
+                e[i] = staged_extent(p0[i], B::SWB, N);
+                off[i] = i * B::RAWP + e[i].skew;
+                total += e[i].bytes;
             }
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(mbar)), "r"(total) : "memory");
 #pragma unroll
             for (int i = 0; i < FWS; i++)
                 asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(smem_u32(xs + i * B::RAWP)), "l"(p.buf + a0[i]), "r"(bytes[i]), "r"(smem_u32(mbar)) : "memory");
+                             ::"r"(smem_u32(xs + i * B::RAWP)), "l"(p.buf + e[i].src), "r"(e[i].bytes), "r"(smem_u32(mbar)) : "memory");
         }
     };
 
@@ -218,7 +217,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                         const unsigned w = half[wcol * B::FPITCH + fl];
                         uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)N * (size_t)(p.nframes - 1 - (long long)(x0 + fl));
 #pragma unroll
-                        for (int j = 0; j < 4; j++) rowp[((u + T * q) + P * (4 * m + j) + N / 2 - 1) & (N - 1)] = lut_at(lut_base, w, j);
+                        for (int j = 0; j < 4; j++) rowp[waterfall_col((u + T * q) + P * (4 * m + j), N)] = lut_at(lut_base, w, j);
                     }
                 }
 #pragma unroll 1
@@ -242,8 +241,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
 #pragma unroll
                     for (int j = 0; j < 4; j++) {
                         const int bin = (u + T * q) + P * (4 * m + j);
-                        const int y = (nfull / 2 - bin) & (nfull - 1);                         // lib/worker.js:90
-                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0 + 8 * g;   // :117
+                        uint32_t *rowp = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)image_row(bin, nfull) + x0 + 8 * g;
                         uint4 a, b;
                         lut_row8(lut_base, w, j, a, b);
                         store_row8(rowp, a, b, rows_aligned);
@@ -296,8 +294,7 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                 const unsigned char *rp = xs + s_off[(warp * 2 + fpar) * FWS + r * FW + f];
 #pragma unroll
                 for (int a = 0; a < P; a++) v[a] = decode_raw_cf<FMT>(rp, T * a + t, p.format);
-                // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact
-                if (t == 0 && valid) p.fmid[p.chunk_first + xr] = make_float2(cre(v[P / 2]) * raw_scale<FMT>(), cim(v[P / 2]) * raw_scale<FMT>());
+                if (t == 0 && valid) p.fmid[p.chunk_first + xr] = raw_mid<FMT>(v[P / 2]);
 #pragma unroll
                 for (int a = 0; a < P; a++) v[a] = cscale(v[a], win[a]);
             }
@@ -351,12 +348,12 @@ __global__ void __launch_bounds__(WCfg<LOG2P, LOG2T, FMT>::THREADS, 1) render_w_
                         const int q = r / T, k1 = r % T;
                         const int b = t + T * q + P * k1;
                         const cf w = cld(X + ((N - b) & (N - 1)));
-                        const float2 fa = cun(v[r]), fb = cun(w);
+                        const float2 fa = cun(v[r]);
                         cf nv;
-                        if (k1 < T / 2) nv = cscale(cadd(v[r], cpk(fb.x, -fb.y)), 0.5f);                    // i < n/2:  (re_i + re_p, im_i - im_p) / 2
-                        else nv = cscale(cadd(cpk(fa.y, fa.x), cpk(fb.y, -fb.x)), 0.5f);                     // i > n/2:  (im_p + im_i, -re_p + re_i) / 2
-                        if (q == 0 && k1 == 0 && t == 0) nv = cpk(fmaf(0.0f, fa.y, fa.x), 0.0f);             // imag[0] = 0; a NaN there reaches real[0] (NaN * 0)
-                        if (q == 0 && k1 == T / 2 && t == 0) nv = cpk(0.0f, 0.0f);                           // real[n/2] = imag[0] (just zeroed), imag[n/2] = 0
+                        if (k1 < T / 2) nv = split_lo(v[r], w);
+                        else nv = split_hi(v[r], w);
+                        if (q == 0 && k1 == 0 && t == 0) nv = split_dc(fa);
+                        if (q == 0 && k1 == T / 2 && t == 0) nv = split_nyquist();
                         v[r] = nv;
                     }
                     __syncwarp();                                       // now the buffer is free

@@ -61,6 +61,89 @@ struct Params {
     unsigned long long *t_stamp;   // render_r64_kernel: %globaltimer at the start of CTA 0 goes to t_stamp[0] (null: not recorded)
 };
 
+// ---------------------------------------------------------------------------------------------
+// The small rules of the reference that every render kernel applies, each written once.
+// ---------------------------------------------------------------------------------------------
+
+// first sample of global frame x (lib/worker.js:72): ~~(0.5 + stride * x) with the multiply and the add rounded separately,
+// as JavaScript does them.  The device form spells out the two roundings so that nothing fuses them into an FMA.  The host
+// form gives the same value because the host code is built without FMA instructions (no -mfma), so nothing contracts it.
+// The two must agree bit for bit: frames_inside routes frames with the host form, and the kernels then read with the device form.
+__host__ __device__ __forceinline__ long long frame_pos(double stride, long long x)
+{
+#ifdef __CUDA_ARCH__
+    return (long long)__dadd_rn(0.5, __dmul_rn(stride, (double)x));
+#else
+    return (long long)(0.5 + stride * (double)x);
+#endif
+}
+
+// buffer-relative first sample of chunk-relative frame xr
+__host__ __device__ __forceinline__ long long frame_start(const Params &p, long long xr)
+{
+    return frame_pos(p.stride, p.frame_first + p.chunk_first + xr) - p.sample_base;
+}
+
+// samples s0 .. s0 + count - 1, sw bytes each, lie in the buffer's valid bytes (else the reads go through decode_checked)
+__host__ __device__ __forceinline__ bool samples_inside(long long s0, long long count, unsigned sw, unsigned long long valid_bytes)
+{
+    return s0 >= 0 && (unsigned long long)(s0 + count) * sw <= valid_bytes;
+}
+
+// sample s as decode_raw gives it (the code without its scale).  A sample that may lie past a ragged buffer end (`inside`
+// false) is read by decode_checked, which gives what the reference's typed array gives there, and scaled back to the same form.
+template <int FMT> __device__ __forceinline__ cf decode_point(const Params &p, long long s, bool inside)
+{
+    if (inside) return cpk(decode_raw<FMT>(p.buf, s, p.format));
+    const float inv = 1.0f / raw_scale<FMT>();
+    const float2 d = decode_checked(p.buf, s, p.format, p.valid_bytes);
+    return cpk(d.x * inv, d.y * inv);
+}
+
+// The 16-byte units a bulk copy stages for nsamples samples of sw bytes from sample p0: source byte offset src (p0's byte
+// offset rounded down to 16), bytes (rounded up to 16), and skew, the offset of sample p0 in the staged copy.  The buffer's
+// readable slack covers the rounding whenever the samples themselves lie inside (frames_inside).
+struct Extent { unsigned long long src; unsigned bytes; int skew; };
+__device__ __forceinline__ Extent staged_extent(long long p0, int sw, long long nsamples)
+{
+    const unsigned long long off = (unsigned long long)p0 * sw, a0 = off & ~15ull;
+    return { a0, (unsigned)(((off - a0) + (unsigned long long)nsamples * sw + 15) & ~15ull), (int)(off - a0) };
+}
+
+// the raw sample p0 + n/2 of a frame (amp gauge, lib/worker.js:131-133) from its decode_raw value; the power-of-two scale is exact
+template <int FMT> __device__ __forceinline__ float2 raw_mid(cf v)
+{
+    return make_float2(cre(v) * raw_scale<FMT>(), cim(v) * raw_scale<FMT>());
+}
+
+// image row of bin `bin` of an n-point frame (lib/worker.js:90): bin n/2 is row 0
+__device__ __forceinline__ int image_row(int bin, int n) { return (n / 2 - bin) & (n - 1); }
+// column of bin `bin` in the waterfall layout, n - 1 - image_row (lib/worker.js:116)
+__device__ __forceinline__ int waterfall_col(int bin, int n) { return (bin + n / 2 - 1) & (n - 1); }
+// Split-real post-process (lib/fft_nayuki.js:103-119) of bin i, a = X[i], with its partner b = X[n - i].  Each lane is one
+// add and one multiply by 0.5, both rounded to nearest, in the packed and in the scalar form alike.
+__device__ __forceinline__ cf split_lo(cf a, cf b)     // i < n/2:  ((re_i + re_p) / 2, (im_i - im_p) / 2)
+{
+    const float2 fb = cun(b);
+    return cscale(cadd(a, cpk(fb.x, -fb.y)), 0.5f);
+}
+__device__ __forceinline__ cf split_hi(cf a, cf b)     // i > n/2:  ((im_i + im_p) / 2, (re_i - re_p) / 2)
+{
+    const float2 fa = cun(a), fb = cun(b);
+    return cscale(cadd(cpk(fa.y, fa.x), cpk(fb.y, -fb.x)), 0.5f);
+}
+// bin 0: imag[0] = 0, and a NaN there reaches real[0] in the reference (its butterflies multiply by every twiddle, NaN * 0 = NaN)
+__device__ __forceinline__ cf split_dc(float2 a) { return cpk(fmaf(0.0f, a.y, a.x), 0.0f); }
+// bin n/2: real[n/2] = imag[0] (just zeroed), imag[n/2] = 0
+__device__ __forceinline__ cf split_nyquist() { return cpk(0.0f, 0.0f); }
+// bin `bin` of an n-point frame, whichever of the four it is
+__device__ __forceinline__ cf split_bin(cf a, cf b, int bin, int n)
+{
+    if (bin == 0) return split_dc(cun(a));
+    if (bin == n / 2) return split_nyquist();
+    return bin < n / 2 ? split_lo(a, b) : split_hi(a, b);
+}
+
 // Programmatic dependent launch (render_r64_kernel, finalize_kernel).  wait: the grid this one was launched behind has completed
 // and its memory operations are visible (returns at once without such a grid).  launch_dependents: the next grid of the stream,
 // launched with cudaLaunchAttributeProgrammaticStreamSerialization, may start once every CTA of this grid has executed it or exited.
@@ -293,10 +376,9 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
                 for (int a = 0; a < P; a++) v[a] = cld(src + T * a + t);
             } else {
                 const long long xgl = p.frame_first + xl;
-                // ~~(0.5 + stride * x): separate multiply and add like JavaScript (no FMA)
-                const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;
-                const bool inside = p0 >= 0 &&
-                    (unsigned long long)(p0 + N) * (unsigned)sample_width(FMT == FMT_RUNTIME ? p.format : FMT) <= p.valid_bytes;
+                const long long p0 = frame_pos(p.stride, xgl) - p.sample_base;
+                const bool inside = samples_inside(p0, N, sample_width(FMT == FMT_RUNTIME ? p.format : FMT), p.valid_bytes);
+                // decode_point, written out: calling it adds spills (render_kernel<5, CS16>: 16 -> 80 bytes, launch bounds 256 x 2)
                 if (inside) {
 #pragma unroll
                     for (int a = 0; a < P; a++) v[a] = cpk(decode_raw<FMT>(p.buf, p0 + T * a + t, p.format));
@@ -309,8 +391,7 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
                         v[a] = cpk(d.x * inv, d.y * inv);
                     }
                 }
-                // raw sample at p0 + n/2 (lib/worker.js:131-133); the power-of-two scale is exact
-                if (t == 0 && active) p.fmid[xl] = make_float2(cre(v[P / 2]) * raw_scale<FMT>(), cim(v[P / 2]) * raw_scale<FMT>());
+                if (t == 0 && active) p.fmid[xl] = raw_mid<FMT>(v[P / 2]);
 #pragma unroll
                 for (int a = 0; a < P; a++) v[a] = cscale(v[a], win[a]);
             }
@@ -390,6 +471,7 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
                 for (int j = 0; j < C::NB; j++)
 #pragma unroll
                     for (int k = 0; k < C::RL; k++) {
+                        // split_bin, written out: calling it adds spills (render_kernel<8, FMT_RUNTIME>: 20 -> 36 bytes)
                         const int bin = kbase[j] + kstep * k;
                         const float2 a = cun(v[j * C::RL + k]);
                         const float2 b = X[(N - bin) & (N - 1)];
@@ -453,7 +535,7 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
                         const unsigned gi = min(__float2uint_rz(fmaf(fast_log2(abs2), l2c_g, l2c_g0)), cmax_u);   // (cmap_len may exceed 256)
                         if (p.db_out) p.db_out[(size_t)xl * nfull + bin] = d0;
                         if (direct) {
-                            const int y = (nfull / 2 - bin) & (nfull - 1);                     // lib/worker.js:90
+                            const int y = image_row(bin, nfull);
                             const size_t px = p.waterfall
                                 ? (size_t)nfull * (size_t)(p.nframes - 1 - xl) + (size_t)(nfull - 1 - y)   // :116
                                 : (size_t)xl + (size_t)p.nframes * (size_t)y;                              // :117
@@ -490,7 +572,7 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
                 for (int k = 0; k < C::RL; k++) {
                     const int i = j * C::RL + k;
                     const int bin = sub ? k0sub + sub_r * (kbase[j] + kstep * k) : kbase[j] + kstep * k;
-                    const int y = (nfull / 2 - bin) & (nfull - 1);
+                    const int y = image_row(bin, nfull);
                     uint32_t *row = reinterpret_cast<uint32_t *>(p.image) + (size_t)p.nframes * (size_t)y + x0;
                     uint4 a, b;
                     a.x = s_col[glo[i] & 255].x; a.y = s_col[(glo[i] >> 8) & 255].x;
@@ -544,10 +626,11 @@ __global__ void __launch_bounds__(256, 2) render_kernel(const Params p)
 // Radix-R pre-pass for n_full = R * 4096 (R = 2, 4, 8, 16): decode + window + DFT_R over the
 // slowest input digit + twiddle W_n^{b*k0}; writes R sub-sequences of 4096 points per frame,
 // which render_kernel<12> then transforms in sub-frame mode (four-step FFT, scratch kept
-// L2-resident by chunking the frames).
+// L2-resident by chunking the frames).  twT is the [R-1][4096] table of render_big_kernel's
+// pre-pass: twT[(k-1)*4096 + b] = W_n^{b*k}.
 // ---------------------------------------------------------------------------------------------
 template <int R, int FMT>
-__global__ void __launch_bounds__(256) prepass_kernel(const Params p, float2 *__restrict__ out, const float2 *__restrict__ tw_full)
+__global__ void __launch_bounds__(256) prepass_kernel(const Params p, float2 *__restrict__ out, const float2 *__restrict__ twT)
 {
     constexpr int NS = 4096;
     const long long gid = (long long)blockIdx.x * 256 + threadIdx.x;
@@ -555,28 +638,17 @@ __global__ void __launch_bounds__(256) prepass_kernel(const Params p, float2 *__
     const int b = (int)(gid % NS);
     if (xr >= p.chunk_frames) return;
     const long long xl = p.chunk_first + xr;
-    const long long xgl = p.frame_first + xl;
-    const long long p0 = (long long)__dadd_rn(0.5, __dmul_rn(p.stride, (double)xgl)) - p.sample_base;
-    const bool inside = p0 >= 0 &&
-        (unsigned long long)(p0 + (long long)R * NS) * (unsigned)sample_width(FMT == FMT_RUNTIME ? p.format : FMT) <= p.valid_bytes;
+    const long long p0 = frame_start(p, xr);
+    const bool inside = samples_inside(p0, (long long)R * NS, sample_width(FMT == FMT_RUNTIME ? p.format : FMT), p.valid_bytes);
     cf v[R];
-    if (inside) {
 #pragma unroll
-        for (int a = 0; a < R; a++) v[a] = cpk(decode_raw<FMT>(p.buf, p0 + NS * a + b, p.format));
-    } else {
-        const float inv = 1.0f / raw_scale<FMT>();
-#pragma unroll
-        for (int a = 0; a < R; a++) {
-            const float2 d = decode_checked(p.buf, p0 + NS * a + b, p.format, p.valid_bytes);
-            v[a] = cpk(d.x * inv, d.y * inv);
-        }
-    }
-    if (b == 0) p.fmid[xl] = make_float2(cre(v[R / 2]) * raw_scale<FMT>(), cim(v[R / 2]) * raw_scale<FMT>());   // sample p0 + n/2
+    for (int a = 0; a < R; a++) v[a] = decode_point<FMT>(p, p0 + NS * a + b, inside);
+    if (b == 0) p.fmid[xl] = raw_mid<FMT>(v[R / 2]);
 #pragma unroll
     for (int a = 0; a < R; a++) v[a] = cscale(v[a], p.window[NS * a + b]);
     dft<R>(v);
 #pragma unroll
-    for (int k = 1; k < R; k++) v[k] = cmul(v[k], tw_full[b * k]);
+    for (int k = 1; k < R; k++) v[k] = cmul(v[k], twT[(k - 1) * NS + b]);
     float2 *dst = out + (size_t)xr * R * NS + b;
 #pragma unroll
     for (int k = 0; k < R; k++) cst(dst + (size_t)k * NS, v[k]);
@@ -587,7 +659,9 @@ __global__ void __launch_bounds__(256) prepass_kernel(const Params p, float2 *__
 // split-real (lib/fft_nayuki.js:103-119), then dB, histograms, colour, pixel, per-frame min / max
 // exactly as render_kernel does them (lib/worker.js:85-125).  Used where the post-process needs
 // bins of different sub-sequences of the four-step FFT together: channelMode with n > 4096.
-// p.fmin / p.fmax hold order-preserving uints (init_minmax_kernel), as in sub-frame mode.
+// p.fmin / p.fmax hold order-preserving uints (init_minmax_kernel), as in sub-frame mode.  Its histograms keep their own
+// layout and flush: in render_kernel's {RGBA, count} layout with flush_hist (and a shared bin-mapping struct) this kernel
+// was 14 % slower in channel mode at n = 32768 on B200.
 // ---------------------------------------------------------------------------------------------
 static __global__ void __launch_bounds__(256) spectrum_epilogue_kernel(const Params p, const float2 *__restrict__ spec)
 {
@@ -606,13 +680,7 @@ static __global__ void __launch_bounds__(256) spectrum_epilogue_kernel(const Par
         const int bin = (int)(tile % per_frame) * 256 + threadIdx.x;
         const float2 *X = spec + (size_t)xr * n;
         float2 r = X[bin];
-        if (p.channel_mode) {
-            const float2 a = r, b = X[(n - bin) & (n - 1)];
-            if (bin == 0) r = make_float2(fmaf(0.0f, a.y, a.x), 0.f); // a NaN in imag[0] reaches real[0] in the reference (its butterflies multiply by every twiddle, NaN * 0 = NaN): keep that
-            else if (bin == n / 2) r = make_float2(0.f, 0.f);
-            else if (bin < n / 2) r = make_float2(0.5f * (a.x + b.x), 0.5f * (a.y - b.y));
-            else r = make_float2(0.5f * (b.y + a.y), 0.5f * (-b.x + a.x));
-        }
+        if (p.channel_mode) r = cun(split_bin(cpk(r), cld(X + ((n - bin) & (n - 1))), bin, n));
         const float abs2 = fmaf(r.x, r.x, r.y * r.y);
         const float l2 = fast_log2(abs2);
         const float d0 = fmaf(l2, p.c1, p.c0);
@@ -624,7 +692,7 @@ static __global__ void __launch_bounds__(256) spectrum_epilogue_kernel(const Par
         atomicAdd(&s_cnt[g], 1u);
         if (p.db_out) p.db_out[(size_t)xl * n + bin] = d0;
         if (p.image) {
-            const int y = (n / 2 - bin) & (n - 1);                                // lib/worker.js:90
+            const int y = image_row(bin, n);
             const size_t px = p.waterfall ? (size_t)n * (size_t)(p.nframes - 1 - xl) + (size_t)(n - 1 - y)   // :116
                                           : (size_t)xl + (size_t)p.nframes * (size_t)y;                      // :117
             reinterpret_cast<uint32_t *>(p.image)[px] = p.lut[g];

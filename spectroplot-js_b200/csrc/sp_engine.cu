@@ -727,7 +727,7 @@ static int prepare(sp_engine *e, const sp_request *rq, sp_reply *rp, Job &j, boo
     {   // joint-histogram constants (sp_kernels.cuh, jh_eval): in double, rounded once
         const double c1 = 5.0 * log10(2.0), cmaxd = (double)(rq->cmap_len - 1);
         p.jA = (float)(-10.0 * c1 / sp::JH_RCAP);
-        p.jB = (float)((2.0 - 10.0 * block_norm_db) / sp::JH_RCAP);
+        p.jB = (float)((2.5 - 10.0 * block_norm_db) / sp::JH_RCAP);
         p.jC = (float)(-color_norm * c1 / cmaxd);
         p.jD = (float)((cmaxd - (block_norm_db + rq->gain) * color_norm) / cmaxd);
     }

@@ -198,12 +198,15 @@ __host__ __device__ inline size_t main_smem_bytes(int smem_x_float2, int cmap_le
 
 // ---------------------------------------------------------------------------------------------
 // Joint histogram (render_r64_kernel).  Per pixel, with l2 = log2|X|^2 and d0 = c1*l2 + c0 (= dBfs - gain):
-//   r  = RN(sat(jA*l2 + jB) * RCAP),  jA*l2 + jB = (2.0 - 10*d0) / RCAP   : RN(x - 0.5) == trunc(x) for the
-//        x = 2.5 - 10*d0 of the table above (off quantisation ties), saturating at 0 and RCAP = 1003
+//   r  = RD(sat(jA*l2 + jB) * RCAP),  jA*l2 + jB = (2.5 - 10*d0) / RCAP   : floor(x) == trunc(x) for the
+//        x = 2.5 - 10*d0 of the table above, saturating at 0 and RCAP = 1003
 //   g' = RN(sat(jC*l2 + jD) * cmax) subtracted from cmax (as is when range < 0), jC*l2 + jD = (cmax - (d0 + gain)*color_norm) / cmax
 //        (lib/worker.js:111-112: the colour index g = cmax - g', clamped by the saturation)
 // Both roundings are done by adding 2^23 inside an FFMA, so S = 2^23 + r + g' and Y = 2^23 + g' come out of
-// four FMA-pipe instructions with no F2I and no integer clamp.  r falls and g rises with l2, so j = r + g'
+// four FMA-pipe instructions with no F2I and no integer clamp.  r is rounded down, not to nearest: as Y is an integer,
+// RD(kx*RCAP + Y) - Y = floor(kx*RCAP) whatever Y is, where round-to-nearest-even would make the pixels with
+// kx*RCAP = m + 0.5 (kx == 0.5, d0 at -49.95) fall in dB bin 499 or 500 by the parity of their colour index - a dB
+// histogram that changed with gain and range.  r falls and g rises with l2, so j = r + g'
 // is monotone and (r, g') is a function of j: ONE shared-memory atomic per pixel.  jh_decode() inverts j
 // by bisection over the ordered floats with the SAME jh_eval().  Non-finite pixels (|X|^2 flushed to 0,
 // +inf, NaN) take the ordinary path and are corrected per frame through two extra counters:
@@ -236,7 +239,7 @@ __device__ __forceinline__ float jh_eval(float l2, const JhConst &c, float &Y)
     const float kx = __saturatef(fmaf(l2, c.A, c.B));
     const float ky = __saturatef(fmaf(l2, c.C, c.D));
     Y = fmaf(ky, c.ncmax, c.ymagic);
-    return fmaf(kx, c.rcap, Y);
+    return __fmaf_rd(kx, c.rcap, Y);
 }
 
 __device__ __forceinline__ int cb_bin_of_raw(int r)
